@@ -2,7 +2,7 @@
 """bench.py -- Opt fit (orthant NNLS enumeration) throughput on B200, one process per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload NAME]
-                  [--no-cpu-baseline] [--no-extras]
+                  [--no-cpu-baseline] [--no-extras] [--dump-outputs DIR]
 
 BASELINE.json's metric is "Opt fit time-to-solution and orthant NNLS solves/sec at K=20, 1/2/4/8 B200":
 every N runs the SAME problem -- `k20_m200`: synthetic N=100 000, M=200, K=20, eta=1e-3 -- so the series
@@ -27,6 +27,11 @@ BASELINE configs[2] in full (N=1M, M=512, K=24) on that path.
 scaling + data-space Lawson-Hanson + residual norm, i.e. Opt.jl:85-94) on all host threads, on a bounded
 sample of the same workload's orthants, in the same unit (it spends two of its NNLS solves per sign pattern).
 Julia is not in this image, so this is the C restatement ("port"); it never loads the product library.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned as DIR/<name>.npy
+(float64), so that two builds can be compared output for output on the same seeded inputs.  Native arm: the
+fit's winner `b_best`, its objective `opt` and its raw weights `alpha_raw` (M+1).  Reference arm: the sampled
+orthants `b_list` and their objectives `objs`.
 """
 from __future__ import annotations
 
@@ -157,20 +162,26 @@ def make_workload(name, synth):
 
 def cpu_reference_sample(oc, X, y, P, eta, n_orthants, nthreads, seed=0):
     """Times the C restatement of the reference loop on `n_orthants` seeded random orthants (of the reference's
-    2^(K+1)) at full N, M.  Returns (orthant solves per second, seconds)."""
+    2^(K+1)) at full N, M.  Returns (orthant solves per second, seconds, {b_list, objs})."""
     rng = np.random.default_rng(seed)
     bl = rng.integers(0, 1 << (P.shape[1] + 1), size=n_orthants).astype(np.int64)
     t0 = time.perf_counter()
-    oc.opt_fit(X, y, P, eta, b_list=bl, nthreads=nthreads, want_alpha=False)
+    r = oc.opt_fit(X, y, P, eta, b_list=bl, nthreads=nthreads, want_alpha=False)
     dt = time.perf_counter() - t0
-    return n_orthants / dt, dt
+    return n_orthants / dt, dt, {"b_list": bl, "objs": r["objs"]}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of `arrays` as out_dir/<name>.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    _, oc = entry.load_oracle()
-    oc.build()
+    _, oc = entry.load_oracle()           # the library build() made: the tree may be read-only, so no rebuild here
     synth = load_synth()
     X, y, P, eta, wl = make_workload(args.workload or DEFAULT_WORKLOAD, synth)
     cores = oc.num_threads()
@@ -179,9 +190,11 @@ def run_reference(args, rank, world):
         cpu_reference_sample(oc, X, y, P, eta, max(1, per_step // 4), cores, seed=100 + i)
     t_tot, n_tot = 0.0, 0
     for i in range(args.steps):
-        _, dt = cpu_reference_sample(oc, X, y, P, eta, per_step, cores, seed=i)
+        _, dt, last = cpu_reference_sample(oc, X, y, P, eta, per_step, cores, seed=i)
         t_tot += dt
         n_tot += per_step
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     orth = n_tot / t_tot
     val = orth / 2.0                      # the reference spends two NNLS solves (intercept sign -, +) per sign pattern
     sample = (f"{per_step} seeded random orthants per step at full N, M (of the reference's {1 << (P.shape[1] + 1)}); C restatement of "
@@ -302,6 +315,8 @@ def run_native(args, rank, world, local_rank):
     N, M = X.shape
     K = P.shape[1]
     bb, obj, alpha, st = m["last"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"b_best": bb, "opt": obj, "alpha_raw": alpha})
     extra = {}
 
     # ---- extras: never inside the timed region of the headline numbers ------------------------------------
@@ -378,9 +393,8 @@ def run_native(args, rank, world, local_rank):
     }
     if world == 1 and not args.no_cpu_baseline:
         _, oc = entry.load_oracle()
-        oc.build()
         n_s = 4
-        v, dt = cpu_reference_sample(oc, X, y, P, eta, n_s, 1, seed=0)
+        v, dt, _ = cpu_reference_sample(oc, X, y, P, eta, n_s, 1, seed=0)
         line["cpu_baseline"] = {"value": v / 2.0, "unit": UNIT, "cores": 1, "kind": "port",
                                 "sample": f"{n_s} seeded random orthants at full N, M, single thread (the reference loop is serial), {dt:.1f} s: "
                                           f"{v:.4g} orthant solves/s = {v / 2:.4g} sign patterns/s; C restatement of Opt.jl:85-94"}
@@ -450,7 +464,11 @@ def main():
     ap.add_argument("--workload", default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     # keep stdout clean for the one JSON line: libraries (NCCL banner, torchrun) write to fd 1 too
     json_fd = os.dup(1)
     os.dup2(2, 1)

@@ -6,11 +6,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_reference_arm_prints_the_contract_line():
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
+def test_reference_arm_prints_the_contract_line(tmp_path):
+    dump = tmp_path / "outputs"
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                          "--dump-outputs", str(dump)],
                          capture_output=True, text=True, timeout=600, cwd=ROOT, env=dict(os.environ, LD_DEBUG="libs"))        # the dynamic loader lists every library it maps on stderr
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
@@ -26,3 +30,8 @@ def test_reference_arm_prints_the_contract_line():
     assert j["gpu_launches"] == 0
     # the arm is the oracle only: the product library is never mapped into that process
     assert "libpls_oracle" in out.stderr and "libpls_cuda" not in out.stderr
+    # --dump-outputs: the last timed step's sampled orthants and their objectives, float64
+    bl, objs = np.load(dump / "b_list.npy"), np.load(dump / "objs.npy")
+    assert sorted(os.listdir(dump)) == ["b_list.npy", "objs.npy"]
+    assert bl.dtype == objs.dtype == np.float64 and bl.shape == objs.shape == (cb["cores"],)
+    assert np.all(bl == np.round(bl)) and np.all((0 <= bl) & (bl < 2 ** 21)) and np.all(objs > 0)
