@@ -364,8 +364,7 @@ int k6_alt_run(const Problem &pb, SolveWs &ws, const std::vector<uint64_t> &h_gm
       ws.hspill_bytes = hneed;
     }
   }
-  if (!ws.counters) ALT_TRY(cudaMalloc(&ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24)));
-  ALT_TRY(cudaMemsetAsync(ws.counters, 0, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), st));
+  ALT_TRY(ensure_counters(ws, true, st));
   if (ws.alt_win_len < len + 2) {
     cudaFree(ws.alt_win); ws.alt_win = nullptr; ws.alt_win_len = 0;
     ALT_TRY(cudaMalloc(&ws.alt_win, sizeof(double) * (len + 2)));

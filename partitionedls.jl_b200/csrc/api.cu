@@ -111,14 +111,14 @@ void read_counters(pls_ctx *c, const unsigned long long *h) {
   if (getenv("PLS_K2_PHASES")) {
     static const char *nm[] = {"start", "plan", "remove", "add", "grad", "refine", "out", "n_remove_blocks", "n_add_blocks",
                                "r_gather", "r_panel", "r_rank", "r_zero", "a_gather", "a_hmul", "a_spart", "a_inv", "a_panel", "a_rank", "a_rows", "n_tab_sweep_in", "n_tab_unsweep", "tab_ops"};
-    for (int i = 0; i < 23; ++i) fprintf(stderr, "k2 phase %-16s %llu\n", nm[i], h[CNT_NUM + 1 + i]);
+    for (int i = 0; i < 23; ++i) fprintf(stderr, "k2 phase %-16s %llu\n", nm[i], h[CNT_PHASE0 + i]);
   }
-  if (getenv("PLS_K4_DRIFT")) { double d; memcpy(&d, &h[CNT_NUM + 24], sizeof(d)); fprintf(stderr, "k2v4 max KKT violation vs the original system / max|c| = %.3e, cold restarts %llu\n", d, h[CNT_SPILLS]); }
+  if (getenv("PLS_K4_DRIFT")) fprintf(stderr, "k2v4 max KKT violation vs the original system / max|c| = %.3e, cold restarts %llu\n", counter_drift(h), h[CNT_SPILLS]);
   s.pivots = (int64_t)h[CNT_PIVOTS]; s.grad_evals = (int64_t)h[CNT_GRAD];
   s.sum_p = (int64_t)h[CNT_SUMP]; s.sum_p2 = (int64_t)h[CNT_SUMP2];
   s.bpp_iters = (int64_t)h[CNT_ITERS]; s.spills = (int64_t)h[CNT_SPILLS];
   s.rebuilds = (int64_t)h[CNT_REBUILDS]; s.blocked = (int64_t)h[CNT_BLOCKED];
-  { double d; memcpy(&d, &h[CNT_NUM + 24], sizeof(d)); s.k2_max_drift = d; }
+  s.k2_max_drift = counter_drift(h);
   const double Mp = c->pb.Mp;
   s.nnls_flops = 2.0 * Mp * (double)s.sum_p + 4.0 * (double)s.sum_p2;
   s.nnls_l2_bytes = 8.0 * Mp * (double)s.sum_p;
@@ -127,7 +127,7 @@ void read_counters(pls_ctx *c, const unsigned long long *h) {
 // K2 + K3 over a range, winner record left in ws.win.  Caller holds the device.
 // pairs: [b_begin, b_begin + b_count) are sign patterns of the K user groups; the intercept sign is left free, so
 // every solve resolves the two reference orthants b and b + 2^K (the winner record carries the full b).
-int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs, int force_variant) {
+int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs, K2Force force_variant) {
   Problem &pb = c->pb;
   if (!pb.gram_ready) { set_error("Gram matrix not built (call pls_gram_build / pls_gram_finalize)"); return PLS_EINVAL; }
   if (pb.Kp > 40) { set_error("K = %d: 2^(K+1) orthants cannot be enumerated (limit K <= 39); use fit(BnB) or fit(Alt)", pb.K); return PLS_EINVAL; }
@@ -136,40 +136,40 @@ int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj,
   if (b_begin < 0 || b_count <= 0 || b_begin + b_count > total) { set_error("orthant range out of bounds"); return PLS_EINVAL; }
   int rc = ensure_all_buffers(c, b_count, want_obj, want_alpha);
   if (rc) return rc;
-  PLS_CUDA_TRY(ensure_win(c->ws, pb.Mp + 2));
+  PLS_CUDA_TRY(ensure_win(c->ws, record_len(pb.Mp)));
   if (c->ws.counters)
-    PLS_CUDA_TRY(cudaMemsetAsync(c->ws.counters, 0, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), c->stream));
+    PLS_CUDA_TRY(cudaMemsetAsync(c->ws.counters, 0, sizeof(unsigned long long) * CNT_BLOCK_LEN, c->stream));
   rc = k2_solve_range(pb, pb.G, pb.ldg, pb.c, pb.scal, pb.gmask, pb.Mp, pb.Kp, c->ws, b_begin, b_count,
                       want_obj ? c->ws.all_obj : nullptr, want_alpha ? c->ws.all_alpha : nullptr,
                       c->sm_count, c->stream, &c->launches, pairs, force_variant,
                       c->h_gmask.size() == (size_t)pb.Mp ? c->h_gmask.data() : nullptr);
-  if (rc == PLS_OK && force_variant == 0) {      // the main range of a fit (not a polish / fallback re-solve)
+  if (rc == PLS_OK && force_variant == K2_DISPATCH) {      // the main range of a fit (not a polish / fallback re-solve)
     c->stats.k2_variant = c->ws.last_variant; c->stats.k2_threads = c->ws.last_threads;
     c->stats.k2_ctas_per_sm = c->ws.last_occ; c->stats.k2_grid = c->ws.last_grid;
   }
   return rc;
 }
 
-// Precondition: c->h_pin holds the winner record [alpha | obj | b] and, from h_pin + Mp + 4, the K2 counters of the
-// range just solved (stream synchronised).  The two-level kernel reports the largest KKT violation against the
-// ORIGINAL Gram system that any of its periodic checks saw; above 1e-13 max|c| its tableau was losing digits on
-// this (ill-conditioned) problem, and the winner is solved once more -- one orthant / pair, cold, by the one-level
-// kernel, whose every iterate is checked against the original system.  The new record replaces the old one in
-// ws.win and h_pin; the counters of the main run are kept.
+namespace {
+
+// Precondition: c->h_pin holds the winner record and the K2 counters of the range just solved (stream synchronised).
+// The two-level kernel reports the largest KKT violation against the ORIGINAL Gram system that any of its periodic
+// checks saw; above 1e-13 max|c| its tableau was losing digits on this (ill-conditioned) problem, and the winner is
+// solved once more -- one orthant / pair, cold, by the one-level kernel, whose every iterate is checked against the
+// original system.  The new record replaces the old one in ws.win and h_pin; the counters of the main run are kept.
 int polish_if_drifted(pls_ctx *c, bool pairs, bool *did) {
   *did = false;
   const int Mp = c->pb.Mp;
-  unsigned long long *cnt = reinterpret_cast<unsigned long long *>(c->h_pin + Mp + 4);
-  double drift; memcpy(&drift, &cnt[CNT_NUM + 24], sizeof(drift));
-  if (!(drift > 1e-13)) return PLS_OK;
-  long long bb; memcpy(&bb, &c->h_pin[Mp + 1], sizeof(bb));
-  if (bb < 0 || c->h_pin[Mp] != c->h_pin[Mp]) return PLS_OK;
-  std::vector<unsigned long long> keep(cnt, cnt + CNT_NUM + 1 + 24);
+  unsigned long long *cnt = c->pin_counters();
+  if (!(counter_drift(cnt) > 1e-13)) return PLS_OK;
+  const long long bb = c->pin_b();
+  if (bb < 0 || c->pin_obj() != c->pin_obj()) return PLS_OK;
+  std::vector<unsigned long long> keep(cnt, cnt + CNT_BLOCK_LEN);
   const int64_t idx = pairs ? (int64_t)(bb & (((long long)1 << (c->pb.Kp - 1)) - 1)) : (int64_t)bb;
-  int rc = solve_range_dev(c, idx, 1, false, false, pairs, 3);
+  int rc = solve_range_dev(c, idx, 1, false, false, pairs, K2_FORCE_V3);
   if (rc) return rc;
   cudaStream_t st = c->stream;
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
   keep[CNT_REBUILDS] += 1;                      // reported as a rebuild
   memcpy(cnt, keep.data(), sizeof(unsigned long long) * keep.size());
@@ -187,37 +187,111 @@ int polish_if_drifted(pls_ctx *c, bool pairs, bool *did) {
 int fallback_if_stalled(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs, bool *did) {
   *did = false;
   const int Mp = c->pb.Mp;
-  unsigned long long *cnt = reinterpret_cast<unsigned long long *>(c->h_pin + Mp + 4);
+  unsigned long long *cnt = c->pin_counters();
   if (!cnt[CNT_NOCONV]) return PLS_OK;
-  std::vector<unsigned long long> keep(cnt, cnt + CNT_NUM + 1 + 24);
+  std::vector<unsigned long long> keep(cnt, cnt + CNT_BLOCK_LEN);
   cudaStream_t st = c->stream;
   std::vector<double> best;
   const int n_half = pairs ? 2 : 1;
   for (int h = 0; h < n_half; ++h) {
     const int64_t b0 = b_begin + (h ? ((int64_t)1 << (c->pb.Kp - 1)) : 0);
-    int rc = solve_range_dev(c, b0, b_count, want_obj, want_alpha, false, 1);
+    int rc = solve_range_dev(c, b0, b_count, want_obj, want_alpha, false, K2_FORCE_V1);
     if (rc) return rc;
-    PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-    PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
+    PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, st));
+    PLS_CUDA_TRY(cudaMemcpyAsync(cnt, c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
     PLS_CUDA_TRY(cudaStreamSynchronize(st));
     if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves did not converge (block pivoting and the single-pivot fallback)", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
-    long long bb; memcpy(&bb, &c->h_pin[Mp + 1], sizeof(bb));
     bool better = best.empty();
     if (!better) {
-      long long b1; memcpy(&b1, &best[Mp + 1], sizeof(b1));
       double yy = 0.0;
       PLS_CUDA_TRY(cudaMemcpy(&yy, c->pb.scal, sizeof(double), cudaMemcpyDeviceToHost));
-      better = opt_better(c->h_pin[Mp], bb, best[Mp], b1, PLS_TIE_REL * yy);
+      better = opt_better(c->pin_obj(), c->pin_b(), best[Mp], record_b(best.data(), Mp), PLS_TIE_REL * yy);
     }
-    if (better) best.assign(c->h_pin, c->h_pin + Mp + 2);
+    if (better) best.assign(c->h_pin, c->h_pin + record_len(Mp));
   }
-  memcpy(c->h_pin, best.data(), sizeof(double) * (Mp + 2));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->ws.win, c->h_pin, sizeof(double) * (Mp + 2), cudaMemcpyHostToDevice, st));
+  memcpy(c->h_pin, best.data(), sizeof(double) * record_len(Mp));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->ws.win, c->h_pin, sizeof(double) * record_len(Mp), cudaMemcpyHostToDevice, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  keep[CNT_NOCONV] = 0; keep[CNT_REBUILDS] += 1; keep[CNT_NUM + 24] = 0;     // resolved; no polish needed after v1
+  keep[CNT_NOCONV] = 0; keep[CNT_REBUILDS] += 1; keep[CNT_DRIFT] = 0;     // resolved; no polish needed after v1
   memcpy(cnt, keep.data(), sizeof(unsigned long long) * keep.size());
   *did = true;
   return PLS_OK;
+}
+
+int copy_outputs(pls_ctx *c, const K2Range &r) {
+  cudaStream_t st = c->stream;
+  if (r.all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(r.all_obj, c->ws.all_obj, sizeof(double) * (size_t)r.b_count, cudaMemcpyDeviceToHost, st));
+  if (r.all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(r.all_alpha, c->ws.all_alpha, sizeof(double) * (size_t)r.b_count * c->pb.Mp, cudaMemcpyDeviceToHost, st));
+  return PLS_OK;
+}
+
+int launch_total(const pls_ctx *c) {
+  if (c->subs.empty()) return c->launches;
+  int n = 0;
+  for (const pls_ctx *s : c->subs) n += s->launches;
+  return n;
+}
+
+}  // namespace
+
+int k2_range_enqueue(pls_ctx *c, const K2Range &r) {
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[r.ev], c->stream));
+  const int rc = solve_range_dev(c, r.b_begin, r.b_count, r.all_obj != nullptr, r.all_alpha != nullptr, r.pairs);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[r.ev + 1], c->stream));
+  return PLS_OK;
+}
+
+int k2_range_copy(pls_ctx *c, const K2Range &r) {
+  cudaStream_t st = c->stream;
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(c->pb.Mp), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_counters(), c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
+  return copy_outputs(c, r);
+}
+
+int k2_range_settle(pls_ctx *c, K2Range &r) {
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[r.ev], c->ev[r.ev + 1]);
+  c->stats.ms_nnls = ms;
+  int rc = fallback_if_stalled(c, r.b_begin, r.b_count, r.all_obj != nullptr, r.all_alpha != nullptr, r.pairs, &r.fell);
+  if (rc) return rc;
+  if (r.fell && (r.all_obj || r.all_alpha)) {
+    rc = copy_outputs(c, r);
+    if (rc) return rc;
+    PLS_CUDA_TRY(cudaStreamSynchronize(c->stream));
+  }
+  rc = polish_if_drifted(c, r.pairs, &r.polished);
+  if (rc) return rc;
+  const unsigned long long *cnt = c->pin_counters();
+  read_counters(c, cnt);
+  if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves hit the iteration cap", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
+  return PLS_OK;
+}
+
+int k2_range_solve(pls_ctx *c, K2Range &r) {
+  int rc = k2_range_enqueue(c, r);
+  if (rc) return rc;
+  rc = k2_range_copy(c, r);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaStreamSynchronize(c->stream));
+  return k2_range_settle(c, r);
+}
+
+FitMark fit_start(pls_ctx *c) {
+  const FitMark m{now_ms(), launch_total(c)};
+  const double keep_upload = c->stats.ms_upload;
+  memset(&c->stats, 0, sizeof(c->stats));
+  c->stats.ms_upload = keep_upload;
+  return m;
+}
+
+void fit_finish(pls_ctx *c, const FitMark &m, pls_stats *out) {
+  pls_stats &s = c->stats;
+  const double Nd = (double)c->pb.N, Md = (double)c->pb.Mp;
+  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
+  s.kernel_launches = launch_total(c) - m.launches0;
+  s.ms_total = now_ms() - m.t0 + s.ms_upload;
+  if (out) *out = s;
 }
 
 // Paired orthants are used whenever only the winner is asked for, the problem fits the block-pivoting
@@ -264,9 +338,9 @@ int residual_partial_w(pls_ctx *c, const double *w, double *ssq_out) {
   PLS_CUDA_TRY(cudaMemcpyAsync(c->d_w, c->h_pin, sizeof(double) * Mp, cudaMemcpyHostToDevice, st));
   rc = k4_residual(c->pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches);
   if (rc) return rc;
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_ssq(), c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  *ssq_out = c->h_pin[Mp];
+  *ssq_out = *c->pin_ssq();
   return PLS_OK;
 }
 
@@ -443,7 +517,7 @@ int pls_load(pls_ctx *c, const double *X, int64_t N, int64_t ldx, int64_t M, con
     cudaFree(c->d_w); c->d_w = nullptr;
     PLS_CUDA_TRY(cudaMalloc(&c->d_w, sizeof(double) * Mp));
     if (c->h_pin) { cudaFreeHost(c->h_pin); c->h_pin = nullptr; }
-    PLS_CUDA_TRY(cudaMallocHost(&c->h_pin, sizeof(double) * (Mp + 4 + CNT_NUM + 1 + 24)));
+    PLS_CUDA_TRY(cudaMallocHost(&c->h_pin, sizeof(double) * pin_len(Mp)));
   }
   pb.N = N; pb.ldz = ldz; pb.M = (int)M; pb.K = (int)K; pb.Mp = Mp; pb.Kp = (int)K + 1;
   pb.zcols = zc; pb.zcols_pad = zcp; pb.eta = eta;
@@ -513,39 +587,15 @@ int pls_opt_solve_range(pls_ctx *c, int64_t b_begin, int64_t b_count, double *al
   int rc = check_ctx(c);
   if (rc) return rc;
   if (!alpha_raw || !b_best || !obj_best) { set_error("null output pointer"); return PLS_EINVAL; }
-  cudaStream_t st = c->stream;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
-  rc = solve_range_dev(c, b_begin, b_count, all_obj != nullptr, all_alpha != nullptr, false);
-  if (rc) return rc;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
-  const int Mp = c->pb.Mp;
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
-  if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj, c->ws.all_obj, sizeof(double) * (size_t)b_count, cudaMemcpyDeviceToHost, st));
-  if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha, c->ws.all_alpha, sizeof(double) * (size_t)b_count * Mp, cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  float ms = 0.f;
-  cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]);
-  c->stats.ms_nnls = ms;
+  K2Range r;
+  r.b_begin = b_begin; r.b_count = b_count; r.all_obj = all_obj; r.all_alpha = all_alpha;
+  rc = k2_range_solve(c, r);
   c->stats.orthants = b_count; c->stats.nnls_problems = b_count;
-  {
-    bool fell = false, did = false;
-    rc = fallback_if_stalled(c, b_begin, b_count, all_obj != nullptr, all_alpha != nullptr, false, &fell); if (rc) return rc;
-    if (fell) {
-      if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj, c->ws.all_obj, sizeof(double) * (size_t)b_count, cudaMemcpyDeviceToHost, st));
-      if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha, c->ws.all_alpha, sizeof(double) * (size_t)b_count * Mp, cudaMemcpyDeviceToHost, st));
-      PLS_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    rc = polish_if_drifted(c, false, &did); if (rc) return rc;
-  }
-  const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(c->h_pin + Mp + 4);
-  read_counters(c, cnt);
-  memcpy(alpha_raw, c->h_pin, sizeof(double) * Mp);
-  *obj_best = c->h_pin[Mp];
-  long long bb; memcpy(&bb, &c->h_pin[Mp + 1], sizeof(bb));
-  *b_best = bb;
+  if (rc) return rc;
+  memcpy(alpha_raw, c->h_pin, sizeof(double) * c->pb.Mp);
+  *obj_best = c->pin_obj();
+  *b_best = c->pin_b();
   c->stats.kernel_launches = c->launches - c->launch_mark + 3;   // + winner-weights / K4 launches that follow
-  if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves hit the iteration cap", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
   if (*obj_best != *obj_best) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -556,33 +606,16 @@ int pls_opt_solve_pairs(pls_ctx *c, int64_t p_begin, int64_t p_count, double *al
   if (rc) return rc;
   if (!alpha_raw || !b_best || !obj_best) { set_error("null output pointer"); return PLS_EINVAL; }
   if (c->pb.Mp > 1024 || c->pb.Kp < 2) { set_error("paired orthants need M + 1 <= 1024 and K >= 1"); return PLS_EUNSUPPORTED; }
-  cudaStream_t st = c->stream;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
-  rc = solve_range_dev(c, p_begin, p_count, false, false, true);
+  K2Range r;
+  r.b_begin = p_begin; r.b_count = p_count; r.pairs = true;
+  rc = k2_range_solve(c, r);
+  c->stats.orthants = 2 * p_count;
+  c->stats.nnls_problems = r.fell ? 3 * p_count : p_count;     // a fallback solves both halves once more
   if (rc) return rc;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
-  const int Mp = c->pb.Mp;
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  float ms = 0.f;
-  cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]);
-  c->stats.ms_nnls = ms;
-  c->stats.orthants = 2 * p_count; c->stats.nnls_problems = p_count;
-  {
-    bool fell = false, did = false;
-    rc = fallback_if_stalled(c, p_begin, p_count, false, false, true, &fell); if (rc) return rc;
-    if (fell) c->stats.nnls_problems = 3 * p_count;
-    rc = polish_if_drifted(c, true, &did); if (rc) return rc;
-  }
-  const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(c->h_pin + Mp + 4);
-  read_counters(c, cnt);
-  memcpy(alpha_raw, c->h_pin, sizeof(double) * Mp);
-  *obj_best = c->h_pin[Mp];
-  long long bb; memcpy(&bb, &c->h_pin[Mp + 1], sizeof(bb));
-  *b_best = bb;
+  memcpy(alpha_raw, c->h_pin, sizeof(double) * c->pb.Mp);
+  *obj_best = c->pin_obj();
+  *b_best = c->pin_b();
   c->stats.kernel_launches = c->launches - c->launch_mark + 3;
-  if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves hit the iteration cap", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
   if (*obj_best != *obj_best) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -600,9 +633,9 @@ int pls_opt_residual_partial(pls_ctx *c, const double *alpha_raw, int64_t b, dou
   rc = k4_residual(c->pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches);
   if (rc) return rc;
   PLS_CUDA_TRY(cudaEventRecord(c->ev[5], st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_ssq(), c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  *ssq_out = c->h_pin[Mp];
+  *ssq_out = *c->pin_ssq();
   float ms = 0.f;
   if (cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]) == cudaSuccess) c->stats.ms_recompute = ms; else cudaGetLastError();
   return PLS_OK;
@@ -671,11 +704,7 @@ int pls_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_t 
   if (rc) return rc;
   if (!c->pb.loaded) { set_error("no data set loaded"); return PLS_EINVAL; }
   if (!alpha_raw || !b_best || !obj_best) { set_error("null output pointer"); return PLS_EINVAL; }
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
-  const int launches0 = c->launches;
+  const FitMark fm = fit_start(c);
   Problem &pb = c->pb;
   cudaStream_t st = c->stream;
   const int Mp = pb.Mp;
@@ -684,68 +713,45 @@ int pls_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_t 
   PLS_CUDA_TRY(cudaEventRecord(c->ev[0], st));
   rc = k1_gram_build(pb, st, &c->launches); if (rc) return rc;
   rc = k1_gram_finalize(pb, st, &c->launches); if (rc) return rc;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
-  const bool pairs = use_pairs(c, flags, all_obj != nullptr || all_alpha != nullptr);
-  rc = solve_range_dev(c, 0, pairs ? total / 2 : total, all_obj != nullptr, all_alpha != nullptr, pairs); if (rc) return rc;
-  PLS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
+  K2Range r;                                     // K2 timed between ev[1] and ev[2]
+  r.pairs = use_pairs(c, flags, all_obj != nullptr || all_alpha != nullptr);
+  r.b_count = r.pairs ? total / 2 : total; r.all_obj = all_obj; r.all_alpha = all_alpha; r.ev = 1;
+  rc = k2_range_enqueue(c, r); if (rc) return rc;
   const bool recompute = !(flags & PLS_FLAG_NO_RECOMPUTE);
-  if (recompute) {
+  auto winner_ssq = [&]() -> int {               // K4: data-space sum of squares of the winner record in ws.win
     winner_weights<<<1, 256, 0, st>>>(c->ws.win, pb.gmask, Mp, c->d_w);
     PLS_CUDA_TRY(cudaGetLastError());
     ++c->launches;
-    rc = k4_residual(pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches); if (rc) return rc;
-  }
+    return k4_residual(pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches);
+  };
+  if (recompute) { rc = winner_ssq(); if (rc) return rc; }
   PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-  if (recompute) PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 2, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 3, pb.scal + 3, sizeof(double), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
-  if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj, c->ws.all_obj, sizeof(double) * (size_t)total, cudaMemcpyDeviceToHost, st));
-  if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha, c->ws.all_alpha, sizeof(double) * (size_t)total * Mp, cudaMemcpyDeviceToHost, st));
+  rc = k2_range_copy(c, r); if (rc) return rc;
+  if (recompute) PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_ssq(), c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_nonfinite(), pb.scal + 3, sizeof(double), cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
 
-  if (c->h_pin[Mp + 3] != 0.0) { set_error("non-finite values in X or y"); return PLS_ENUMERIC; }
-  float ms = 0.f;
-  cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]);
-  const float ms_nnls_main = ms;
-  bool polished = false, fell = false;
-  rc = fallback_if_stalled(c, 0, pairs ? total / 2 : total, all_obj != nullptr, all_alpha != nullptr, pairs, &fell); if (rc) return rc;
-  if (fell) {
-    if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj, c->ws.all_obj, sizeof(double) * (size_t)total, cudaMemcpyDeviceToHost, st));
-    if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha, c->ws.all_alpha, sizeof(double) * (size_t)total * Mp, cudaMemcpyDeviceToHost, st));
-    PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  }
-  rc = polish_if_drifted(c, pairs, &polished); if (rc) return rc;
-  polished = polished || fell;
-  if (polished && recompute) {                 // data-space objective of the new winner record
-    winner_weights<<<1, 256, 0, st>>>(c->ws.win, pb.gmask, Mp, c->d_w);
-    PLS_CUDA_TRY(cudaGetLastError());
-    ++c->launches;
-    rc = k4_residual(pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches); if (rc) return rc;
-    PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 2, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (*c->pin_nonfinite() != 0.0) { set_error("non-finite values in X or y"); return PLS_ENUMERIC; }
+  rc = k2_range_settle(c, r); if (rc) return rc;
+  if ((r.fell || r.polished) && recompute) {    // data-space objective of the new winner record
+    rc = winner_ssq(); if (rc) return rc;
+    PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_ssq(), c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
     PLS_CUDA_TRY(cudaStreamSynchronize(st));
   }
   memcpy(alpha_raw, c->h_pin, sizeof(double) * Mp);
-  long long bb; memcpy(&bb, &c->h_pin[Mp + 1], sizeof(bb));
+  const long long bb = c->pin_b();
   *b_best = bb;
-  double obj = c->h_pin[Mp];
-  if (recompute && obj == obj) obj = std::sqrt(c->h_pin[Mp + 2] + eta_term(c, alpha_raw, bb));
+  double obj = c->pin_obj();
+  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term(c, alpha_raw, bb));
   *obj_best = obj;
 
   pls_stats &s = c->stats;
+  float ms = 0.f;
   cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); s.ms_gram = ms;
-  s.ms_nnls = ms_nnls_main;
   cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]); s.ms_recompute = ms;
   s.ms_select = 0.0;   // K3 is timed with K2 (same stream, ~microseconds)
-  s.orthants = total; s.nnls_problems = pairs ? total / 2 : total;
-  const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(c->h_pin + Mp + 4);
-  read_counters(c, cnt);
-  const double Nd = (double)pb.N, Md = (double)Mp;
-  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
-  s.kernel_launches = c->launches - launches0;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
-  if (stats) *stats = s;
-  if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves hit the iteration cap", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
+  s.orthants = total; s.nnls_problems = r.b_count;
+  fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -769,11 +775,7 @@ int pls_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, doubl
   if (rc) return rc;
   if (!c->pb.loaded) { set_error("no data set loaded"); return PLS_EINVAL; }
   if (!alpha_signed || !obj_out || !nopen) { set_error("null output pointer"); return PLS_EINVAL; }
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
-  const int launches0 = c->launches;
+  const FitMark fm = fit_start(c);
   Problem &pb = c->pb;
   cudaStream_t st = c->stream;
   const int Mp = pb.Mp;
@@ -783,7 +785,7 @@ int pls_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, doubl
     rc = k1_gram_finalize(pb, st, &c->launches); if (rc) return rc;
   }
   PLS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
-  PLS_CUDA_TRY(ensure_win(c->ws, pb.Mp + 2));
+  PLS_CUDA_TRY(ensure_win(c->ws, record_len(Mp)));
   BnbReport rep;
   rc = k5_bnb_run(pb, c->ws, c->sm_count, st, &c->launches, &rep); if (rc) return rc;
   PLS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
@@ -793,17 +795,16 @@ int pls_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, doubl
     rc = k4_residual(pb, c->ws, c->d_w, c->d_ssq, c->sm_count, st, &c->launches); if (rc) return rc;
   }
   PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-  if (recompute) PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 2, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 3, pb.scal + 3, sizeof(double), cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, st));
+  if (recompute) PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_ssq(), c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_nonfinite(), pb.scal + 3, sizeof(double), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_counters(), c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  if (c->h_pin[Mp + 3] != 0.0) { set_error("non-finite values in X or y"); return PLS_ENUMERIC; }
-  long long seq; memcpy(&seq, &c->h_pin[Mp + 1], sizeof(seq));
-  if (seq < 0) { set_error("bnb: no feasible leaf found"); return PLS_ENUMERIC; }
+  if (*c->pin_nonfinite() != 0.0) { set_error("non-finite values in X or y"); return PLS_ENUMERIC; }
+  if (c->pin_b() < 0) { set_error("bnb: no feasible leaf found"); return PLS_ENUMERIC; }
   memcpy(alpha_signed, c->h_pin, sizeof(double) * Mp);
-  double obj = c->h_pin[Mp];
-  if (recompute && obj == obj) obj = std::sqrt(c->h_pin[Mp + 2] + eta_term_w(c, alpha_signed));
+  double obj = c->pin_obj();
+  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term_w(c, alpha_signed));
   *obj_out = obj;
   *nopen = rep.visited;
   float ms = 0.f;
@@ -811,15 +812,10 @@ int pls_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, doubl
   cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); s.ms_gram = ms;
   cudaEventElapsedTime(&ms, c->ev[1], c->ev[2]); s.ms_nnls = ms;
   cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]); s.ms_recompute = ms;
-  const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(c->h_pin + Mp + 4);
-  read_counters(c, cnt);
+  read_counters(c, c->pin_counters());
   s.spills = 0;
   s.orthants = rep.visited; s.waves = rep.waves; s.max_open = rep.max_open;
-  const double Nd = (double)pb.N, Md = (double)Mp;
-  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
-  s.kernel_launches = c->launches - launches0;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
-  if (stats) *stats = s;
+  fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -845,11 +841,7 @@ int pls_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps,
   if (!c->pb.loaded) { set_error("no data set loaded"); return PLS_EINVAL; }
   if (!beta0 || !alpha || !beta || !obj_out) { set_error("null pointer"); return PLS_EINVAL; }
   if (R < 1 || T < 1 || !(eps > 0.0)) { set_error("alt: need R >= 1, T >= 1, eps > 0"); return PLS_EINVAL; }
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
-  const int launches0 = c->launches;
+  const FitMark fm = fit_start(c);
   Problem &pb = c->pb;
   cudaStream_t st = c->stream;
   const int Mp = pb.Mp, Kp = pb.Kp;
@@ -871,7 +863,7 @@ int pls_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps,
   PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
   const int len = Mp + Kp + 1;
   std::vector<double> h(len + 2 + Mp + 2);
-  std::vector<unsigned long long> cnt(CNT_NUM + 1 + 24);
+  std::vector<unsigned long long> cnt(CNT_BLOCK_LEN);
   PLS_CUDA_TRY(cudaMemcpyAsync(h.data(), d_win, sizeof(double) * (len + 2), cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaMemcpyAsync(h.data() + len + 2, c->d_w, sizeof(double) * Mp, cudaMemcpyDeviceToHost, st));
   if (recompute) PLS_CUDA_TRY(cudaMemcpyAsync(h.data() + len + 2 + Mp, c->d_ssq, sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -896,11 +888,7 @@ int pls_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps,
   read_counters(c, cnt.data());
   s.waves = s.spills; s.spills = 0;          // CNT_SPILLS carries the longest restart's iteration count
   s.orthants = R;
-  const double Nd = (double)pb.N, Md = (double)Mp;
-  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
-  s.kernel_launches = c->launches - launches0;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
-  if (stats) *stats = s;
+  fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -962,7 +950,7 @@ int pls_bnb_lower_bounds(pls_ctx *c, const uint64_t *pos_masks, const uint64_t *
     rc = k1_gram_build(pb, st, &c->launches); if (rc) return rc;
     rc = k1_gram_finalize(pb, st, &c->launches); if (rc) return rc;
   }
-  PLS_CUDA_TRY(ensure_win(c->ws, pb.Mp + 2));
+  PLS_CUDA_TRY(ensure_win(c->ws, record_len(pb.Mp)));
   BnbShard sh;
   sh.probe = true;
   sh.root_pos.assign(pos_masks, pos_masks + n);
@@ -1006,16 +994,16 @@ int pls_nnls_batch(pls_ctx *c, const double *G, const double *cv, double yy, int
   PLS_CUDA_TRY(cudaMemcpy(pb.gmask, gmask, sizeof(uint64_t) * Mp, cudaMemcpyHostToDevice));
   c->h_gmask.assign(gmask, gmask + Mp);
   if (c->h_pin) { cudaFreeHost(c->h_pin); c->h_pin = nullptr; }
-  PLS_CUDA_TRY(cudaMallocHost(&c->h_pin, sizeof(double) * (Mp + 4 + CNT_NUM + 1 + 24)));
+  PLS_CUDA_TRY(cudaMallocHost(&c->h_pin, sizeof(double) * pin_len(Mp)));
   pb.gram_ready = true;
   rc = solve_range_dev(c, b_begin, b_count, obj_out != nullptr, alpha_out != nullptr);
   if (rc) return rc;
   cudaStream_t st = c->stream;
   if (obj_out) PLS_CUDA_TRY(cudaMemcpyAsync(obj_out, c->ws.all_obj, sizeof(double) * (size_t)b_count, cudaMemcpyDeviceToHost, st));
   if (alpha_out) PLS_CUDA_TRY(cudaMemcpyAsync(alpha_out, c->ws.all_alpha, sizeof(double) * (size_t)b_count * Mp, cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin + Mp + 4, c->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(c->pin_counters(), c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(c->h_pin + Mp + 4);
+  const unsigned long long *cnt = c->pin_counters();
   c->stats.orthants = b_count;
   read_counters(c, cnt);
   if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves did not converge", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }

@@ -354,8 +354,7 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
     BNB_TRY(cudaMalloc(&ws.cta_w, sizeof(double) * (size_t)max_grid * Mp));
     ws.max_ctas = max_grid; ws.Mp = Mp;
   }
-  if (!ws.counters) BNB_TRY(cudaMalloc(&ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24)));
-  BNB_TRY(cudaMemsetAsync(ws.counters, 0, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), st));
+  BNB_TRY(ensure_counters(ws, true, st));
   BNB_TRY(ensure_win(ws, Mp + 2));
   BNB_TRY(cudaMemsetAsync(ws.cta_obj, 0, sizeof(double) * max_grid, st));
   BNB_TRY(cudaMemsetAsync(ws.cta_b, 0xff, sizeof(long long) * max_grid, st));     // -1: no leaf yet

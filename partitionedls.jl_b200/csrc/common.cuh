@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <string.h>
 #include <atomic>
 #include <vector>
 #include <nvtx3/nvToolsExt.h>
@@ -53,11 +54,24 @@ static inline bool opt_better(double oa, long long ba, double ob, long long bb, 
 }
 #define PLS_TIE_REL 1e-13
 
-// Solver work counters accumulated by K2 (device side, unsigned long long each).
+// The counter block ws.counters (device side, unsigned long long each): the solver work counters accumulated by K2
+// (and by BnB / Alt), K2's chain scheduler, the per-phase cycle counters, the largest KKT drift.
 enum Counter {
   CNT_PIVOTS = 0, CNT_GRAD, CNT_SUMP, CNT_SUMP2, CNT_ITERS, CNT_SPILLS, CNT_REBUILDS, CNT_BLOCKED,
-  CNT_NOCONV, CNT_NUM
+  CNT_NOCONV, CNT_NUM,
+  CNT_CHAIN = CNT_NUM,                    // dynamic chain scheduler of K2 (zeroed before every launch)
+  CNT_PHASE0,                             // 23 per-phase cycle counters (PLS_K2_PHASES)
+  CNT_V5_FOLDS = CNT_PHASE0 + 20,         // v5: fold passes, reported with the phase counters
+  CNT_DRIFT = CNT_PHASE0 + 23,            // largest KKT violation / max|c| of the two-level kernels, as double bits
+  CNT_BLOCK_LEN
 };
+
+// the drift slot of a counter block copied to the host
+static inline double counter_drift(const unsigned long long *cnt) {
+  double d;
+  memcpy(&d, &cnt[CNT_DRIFT], sizeof(d));
+  return d;
+}
 
 // Device-resident problem (one GPU).
 struct Problem {
@@ -84,7 +98,7 @@ struct SolveWs {
   long long *cta_b = nullptr;     // [max_ctas]
   double *cta_w = nullptr;        // [max_ctas * Mp]
   double *hspill = nullptr;       // [max_ctas * Mp * Mp] (only when the inverse may outgrow smem)
-  unsigned long long *counters = nullptr;  // [CNT_NUM]
+  unsigned long long *counters = nullptr;  // [CNT_BLOCK_LEN]
   double *win = nullptr;          // [Mp + 2]: winner alpha_raw, obj, b (as double bits)
   double *all_obj = nullptr;      // device staging for per-orthant outputs
   double *all_alpha = nullptr;
@@ -114,6 +128,17 @@ static inline cudaError_t ensure_win(SolveWs &ws, int len) {
   const cudaError_t e = cudaMalloc(&ws.win, sizeof(double) * (size_t)len);
   if (e == cudaSuccess) ws.win_len = len;
   return e;
+}
+
+// Allocates the counter block ws.counters on first use, zeroed then; zero_all: zero all of it on this call too.
+static inline cudaError_t ensure_counters(SolveWs &ws, bool zero_all, cudaStream_t st) {
+  const size_t bytes = sizeof(unsigned long long) * CNT_BLOCK_LEN;
+  if (!ws.counters) {
+    const cudaError_t e = cudaMalloc(&ws.counters, bytes);
+    if (e != cudaSuccess) return e;
+    zero_all = true;
+  }
+  return zero_all ? cudaMemsetAsync(ws.counters, 0, bytes, st) : cudaSuccess;
 }
 
 // Arguments of the K2 kernels (both variants).
@@ -149,10 +174,12 @@ struct K2Args {
 // ---- kernel launchers (defined in gram.cu / nnls.cu / resid.cu) -----------------------------
 int k1_gram_build(Problem &pb, cudaStream_t st, int *launches);
 int k1_gram_finalize(Problem &pb, cudaStream_t st, int *launches);
+// force_variant of k2_solve_range: the kernel of a re-solve, in place of the dispatch rules
+enum K2Force { K2_DISPATCH = 0, K2_FORCE_V1 = 1, K2_FORCE_V3 = 3 };
 int k2_solve_range(const Problem &pb, const double *G, int ldg, const double *c, const double *scal,
                    const uint64_t *gmask, int Mp, int Kp, SolveWs &ws, int64_t b_begin,
                    int64_t b_count, double *d_all_obj, double *d_all_alpha, int sm_count,
-                   cudaStream_t st, int *launches, bool free_top = false, int force_variant = 0,
+                   cudaStream_t st, int *launches, bool free_top = false, int force_variant = K2_DISPATCH,
                    const uint64_t *h_gmask = nullptr);
 // K2 variants: v1 = rank-1 updates on a dense inverse with a global-memory spill path (any M').
 // v3 = v2's algorithm with the inverse split between shared memory and an L2-resident global slice,

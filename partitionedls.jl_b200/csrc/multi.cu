@@ -224,12 +224,8 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
   const int G = (int)c->subs.size();
   const int Mp = c->pb.Mp, Kp = c->pb.Kp;
   if (Kp > 40) { set_error("K = %d: 2^(K+1) orthants cannot be enumerated (limit K <= 39); use fit(BnB) or fit(Alt)", c->pb.K); return PLS_EINVAL; }
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
-  int launches0 = 0;
-  for (pls_ctx *s : c->subs) { launches0 += s->launches; memset(&s->stats, 0, sizeof(s->stats)); }
+  const FitMark fm = fit_start(c);
+  for (pls_ctx *s : c->subs) memset(&s->stats, 0, sizeof(s->stats));
   const double tg0 = now_ms();
   int rc = multi_gram(c);
   if (rc) return rc;
@@ -241,40 +237,19 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
   const int64_t total = (int64_t)1 << Ke;
   const int chunk_log2 = Ke < 12 ? (Ke > 3 ? Ke - 3 : 0) : 12;
   const int64_t nchunks = total >> chunk_log2;
-  std::vector<std::vector<double>> rec(G, std::vector<double>(Mp + 2, 0.0));
+  std::vector<std::vector<double>> rec(G, std::vector<double>(record_len(Mp), 0.0));
   std::vector<char> has(G, 0);
   rc = par_for(c, [&](int g, pls_ctx *s) -> int {
     const int64_t b0 = ((nchunks * g) / G) << chunk_log2, b1 = ((nchunks * (g + 1)) / G) << chunk_log2;
     if (b1 <= b0) return PLS_OK;
     int r = check_ctx(s);
     if (r) return r;
-    cudaStream_t st = s->stream;
-    PLS_CUDA_TRY(cudaEventRecord(s->ev[2], st));
-    r = solve_range_dev(s, b0, b1 - b0, all_obj != nullptr, all_alpha != nullptr, pairs);
+    K2Range kr;
+    kr.b_begin = b0; kr.b_count = b1 - b0; kr.pairs = pairs;
+    kr.all_obj = all_obj ? all_obj + b0 : nullptr; kr.all_alpha = all_alpha ? all_alpha + (size_t)b0 * Mp : nullptr;
+    r = k2_range_solve(s, kr);
     if (r) return r;
-    PLS_CUDA_TRY(cudaEventRecord(s->ev[3], st));
-    PLS_CUDA_TRY(cudaMemcpyAsync(s->h_pin, s->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, st));
-    PLS_CUDA_TRY(cudaMemcpyAsync(s->h_pin + Mp + 4, s->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, st));
-    if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj + b0, s->ws.all_obj, sizeof(double) * (size_t)(b1 - b0), cudaMemcpyDeviceToHost, st));
-    if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha + (size_t)b0 * Mp, s->ws.all_alpha, sizeof(double) * (size_t)(b1 - b0) * Mp, cudaMemcpyDeviceToHost, st));
-    PLS_CUDA_TRY(cudaStreamSynchronize(st));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, s->ev[2], s->ev[3]);
-    {
-      bool fell = false, did = false;
-      r = fallback_if_stalled(s, b0, b1 - b0, all_obj != nullptr, all_alpha != nullptr, pairs, &fell); if (r) return r;
-      if (fell) {
-        if (all_obj) PLS_CUDA_TRY(cudaMemcpyAsync(all_obj + b0, s->ws.all_obj, sizeof(double) * (size_t)(b1 - b0), cudaMemcpyDeviceToHost, st));
-        if (all_alpha) PLS_CUDA_TRY(cudaMemcpyAsync(all_alpha + (size_t)b0 * Mp, s->ws.all_alpha, sizeof(double) * (size_t)(b1 - b0) * Mp, cudaMemcpyDeviceToHost, st));
-        PLS_CUDA_TRY(cudaStreamSynchronize(st));
-      }
-      r = polish_if_drifted(s, pairs, &did); if (r) return r;
-    }
-    const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(s->h_pin + Mp + 4);
-    read_counters(s, cnt);
-    s->stats.ms_nnls = ms;
-    if (cnt[CNT_NOCONV]) { set_error("%llu orthant solves hit the iteration cap", cnt[CNT_NOCONV]); return PLS_ENUMERIC; }
-    memcpy(rec[g].data(), s->h_pin, sizeof(double) * (Mp + 2));
+    memcpy(rec[g].data(), s->h_pin, sizeof(double) * record_len(Mp));
     has[g] = 1;
     return PLS_OK;
   });
@@ -290,7 +265,7 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
   int win = -1; double wo = 0.0; long long wb = -1;
   for (int g = 0; g < G; ++g) {
     if (!has[g]) continue;
-    long long bb; memcpy(&bb, &rec[g][Mp + 1], sizeof(bb));
+    const long long bb = record_b(rec[g].data(), Mp);
     if (bb < 0) continue;
     if (win < 0 || opt_better(rec[g][Mp], bb, wo, wb, tau)) { win = g; wo = rec[g][Mp]; wb = bb; }
   }
@@ -314,13 +289,7 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
   s.ms_gram = tg1 - tg0;
   s.ms_recompute = now_ms() - tr0;
   s.orthants = (int64_t)1 << Kp; s.nnls_problems = total;
-  const double Nd = (double)c->pb.N, Md = (double)Mp;
-  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
-  int launches1 = 0;
-  for (pls_ctx *d : c->subs) launches1 += d->launches;
-  s.kernel_launches = launches1 - launches0;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
-  if (stats) *stats = s;
+  fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -330,41 +299,35 @@ int multi_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, dou
   if (!alpha_signed || !obj_out || !nopen) { set_error("null output pointer"); return PLS_EINVAL; }
   const int G = (int)c->subs.size();
   const int Mp = c->pb.Mp;
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
-  int launches0 = 0;
-  for (pls_ctx *s : c->subs) { launches0 += s->launches; memset(&s->stats, 0, sizeof(s->stats)); }
+  const FitMark fm = fit_start(c);
+  for (pls_ctx *s : c->subs) memset(&s->stats, 0, sizeof(s->stats));
   const double tg0 = now_ms();
   int rc = multi_gram(c);
   if (rc) return rc;
   const double tg1 = now_ms();
   std::atomic<unsigned long long> shared_mu(0x7ff0000000000000ull);
-  std::vector<std::vector<double>> rec(G, std::vector<double>(Mp + 2, 0.0));
+  std::vector<std::vector<double>> rec(G, std::vector<double>(record_len(Mp), 0.0));
   std::vector<char> has(G, 0);
   std::vector<long long> visited(G, 0), waves(G, 0), max_open(G, 0);
   // one search (whole tree or a set of subtrees) on one device; keeps the device's best leaf in rec[g]
   auto run_one = [&](int g, pls_ctx *s, BnbShard *sh, bool *complete) -> int {
     int r = check_ctx(s);
     if (r) return r;
-    PLS_CUDA_TRY(ensure_win(s->ws, s->pb.Mp + 2));
+    PLS_CUDA_TRY(ensure_win(s->ws, record_len(s->pb.Mp)));
     BnbReport rep;
     r = k5_bnb_run(s->pb, s->ws, s->sm_count, s->stream, &s->launches, &rep, sh);
     if (r) return r;
     visited[g] += rep.visited; waves[g] += rep.waves; max_open[g] = std::max(max_open[g], rep.max_open);
     if (complete) *complete = rep.complete;
-    PLS_CUDA_TRY(cudaMemcpyAsync(s->h_pin, s->ws.win, sizeof(double) * (Mp + 2), cudaMemcpyDeviceToHost, s->stream));
-    PLS_CUDA_TRY(cudaMemcpyAsync(s->h_pin + Mp + 4, s->ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), cudaMemcpyDeviceToHost, s->stream));
+    PLS_CUDA_TRY(cudaMemcpyAsync(s->h_pin, s->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, s->stream));
+    PLS_CUDA_TRY(cudaMemcpyAsync(s->pin_counters(), s->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, s->stream));
     PLS_CUDA_TRY(cudaStreamSynchronize(s->stream));
-    const unsigned long long *cnt = reinterpret_cast<const unsigned long long *>(s->h_pin + Mp + 4);
     pls_stats keep = s->stats;
-    read_counters(s, cnt);
+    read_counters(s, s->pin_counters());
     s->stats.pivots += keep.pivots; s->stats.grad_evals += keep.grad_evals; s->stats.sum_p += keep.sum_p; s->stats.sum_p2 += keep.sum_p2;
     s->stats.bpp_iters += keep.bpp_iters; s->stats.rebuilds += keep.rebuilds; s->stats.blocked += keep.blocked;
     s->stats.nnls_flops += keep.nnls_flops; s->stats.nnls_l2_bytes += keep.nnls_l2_bytes;
-    long long seq; memcpy(&seq, &s->h_pin[Mp + 1], sizeof(seq));
-    if (seq >= 0 && (!has[g] || s->h_pin[Mp] < rec[g][Mp])) { memcpy(rec[g].data(), s->h_pin, sizeof(double) * (Mp + 2)); has[g] = 1; }
+    if (s->pin_b() >= 0 && (!has[g] || s->pin_obj() < rec[g][Mp])) { memcpy(rec[g].data(), s->h_pin, sizeof(double) * record_len(Mp)); has[g] = 1; }
     return PLS_OK;
   };
   const double ts0 = now_ms();
@@ -417,13 +380,7 @@ int multi_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, dou
   s.orthants = vis;
   s.waves = 0; s.max_open = 0;
   for (int g = 0; g < G; ++g) { s.waves = std::max<int64_t>(s.waves, waves[g]); s.max_open = std::max<int64_t>(s.max_open, max_open[g]); }
-  const double Nd = (double)c->pb.N, Md = (double)Mp;
-  s.gram_flops = Nd * Md * (Md + 1.0) + 2.0 * Nd * Md + 2.0 * Nd;
-  int launches1 = 0;
-  for (pls_ctx *dd : c->subs) launches1 += dd->launches;
-  s.kernel_launches = launches1 - launches0;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
-  if (stats) *stats = s;
+  fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
@@ -436,10 +393,7 @@ int multi_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double ep
   if (R < 1 || T < 1 || !(eps > 0.0)) { set_error("alt: need R >= 1, T >= 1, eps > 0"); return PLS_EINVAL; }
   const int G = (int)c->subs.size();
   const int Mp = c->pb.Mp, Kp = c->pb.Kp;
-  const double t0 = now_ms();
-  const double keep_upload = c->stats.ms_upload;
-  memset(&c->stats, 0, sizeof(c->stats));
-  c->stats.ms_upload = keep_upload;
+  const FitMark fm = fit_start(c);
   const double tg0 = now_ms();
   int rc = multi_gram(c);
   if (rc) return rc;
@@ -484,7 +438,7 @@ int multi_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double ep
   sum_stats(c, s);
   s.ms_gram = tg1 - tg0;
   s.orthants = R;
-  s.ms_total = now_ms() - t0 + s.ms_upload;
+  s.ms_total = now_ms() - fm.t0 + s.ms_upload;   // (gram_flops and kernel_launches are not reported for Alt over several GPUs)
   if (stats) *stats = s;
   return PLS_OK;
 }

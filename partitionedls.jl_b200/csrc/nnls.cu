@@ -482,8 +482,8 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   // least one fast group) and the walks are long enough to amortise a cold start
   const bool force5 = impl && strcmp(impl, "v5") == 0;
   const bool no5 = getenv("PLS_K2_NO_V5") != nullptr;
-  if (force_variant == 3 && Mp <= 1024) variant = 3;
-  if (force_variant == 1 && !free_top) variant = 1;
+  if (force_variant == K2_FORCE_V3 && Mp <= 1024) variant = 3;
+  if (force_variant == K2_FORCE_V1 && !free_top) variant = 1;
   int cap = Mp, occ = 1;
   size_t smem = 0;
   K3Plan plan3;
@@ -508,7 +508,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     else { cap = plan4.cap; occ = plan4.occ; smem = plan4.smem; }
   }
   if (variant == 3) {
-    int rc = k2v3_plan(Mp, &plan3, force_variant == 3);
+    int rc = k2v3_plan(Mp, &plan3, force_variant == K2_FORCE_V3);
     if (rc == PLS_EUNSUPPORTED && free_top) rc = k2v3_plan(Mp, &plan3, true);   // a tuning override asked for a variant that does not exist
     if (rc == PLS_EUNSUPPORTED) variant = 1; else if (rc) return rc;
     else { cap = plan3.cap; occ = plan3.occ; smem = plan3.smem; }
@@ -583,19 +583,16 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     PLS_CUDA_TRY(cudaMalloc(&ws.hspill, hneed));
     ws.hspill_bytes = hneed;
   }
-  if (!ws.counters) {
-    PLS_CUDA_TRY(cudaMalloc(&ws.counters, sizeof(unsigned long long) * (CNT_NUM + 1 + 24)));
-    PLS_CUDA_TRY(cudaMemsetAsync(ws.counters, 0, sizeof(unsigned long long) * (CNT_NUM + 1 + 24), st));
-  }
+  PLS_CUDA_TRY(ensure_counters(ws, false, st));
   PLS_CUDA_TRY(ensure_win(ws, Mp + 2));
-  PLS_CUDA_TRY(cudaMemsetAsync(ws.counters + CNT_NUM, 0, sizeof(unsigned long long), st));
+  PLS_CUDA_TRY(cudaMemsetAsync(ws.counters + CNT_CHAIN, 0, sizeof(unsigned long long), st));
   ws.last_variant = variant; ws.last_occ = occ; ws.last_grid = (int)grid;
   ws.last_threads = variant == 5 ? plan5.T : (variant == 4 ? plan4.T : (variant == 3 ? plan3.T : T2));
 
   K2Args A;
   A.G = G; A.ldg = ldg; A.c = c; A.scal = scal; A.gmask = gmask; A.Mp = Mp; A.Kp = Kp;
   A.b_begin = b_begin; A.chain_log2 = chain_log2; A.n_chains = n_chains;
-  A.chain_counter = ws.counters + CNT_NUM;
+  A.chain_counter = ws.counters + CNT_CHAIN;
   A.cap = cap;
   A.hspill = (variant == 1 && cap < Mp) ? ws.hspill : nullptr;
   A.qs = 0; A.hglob = nullptr; A.hstride = 0;

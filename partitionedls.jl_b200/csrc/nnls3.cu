@@ -127,7 +127,7 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
     atomicAdd(&A.counters[CNT_BLOCKED], (unsigned long long)s.stat[ST_BLOCKED]);
     atomicAdd(&A.counters[CNT_NOCONV], (unsigned long long)s.stat[ST_NOCONV]);
     PH_TICK3(PH_OUT);
-    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_NUM + 1 + i], (unsigned long long)s.prof[i]);
+    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_PHASE0 + i], (unsigned long long)s.prof[i]);
   }
 }
 

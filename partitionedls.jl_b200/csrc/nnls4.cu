@@ -265,9 +265,9 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
     atomicAdd(&A.counters[CNT_BLOCKED], (unsigned long long)s.stat[ST_BLOCKED]);
     atomicAdd(&A.counters[CNT_NOCONV], (unsigned long long)s.stat[ST_NOCONV]);
     atomicAdd(&A.counters[CNT_SPILLS], n_drift);      // reported as pls_stats.spills
-    atomicMax(&A.counters[CNT_NUM + 24], (unsigned long long)__double_as_longlong(max_viol / cmax));   // non-negative doubles order like integers
+    atomicMax(&A.counters[CNT_DRIFT], (unsigned long long)__double_as_longlong(max_viol / cmax));   // non-negative doubles order like integers
     PH_TICK3(PH_OUT);
-    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_NUM + 1 + i], (unsigned long long)s.prof[i]);
+    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_PHASE0 + i], (unsigned long long)s.prof[i]);
   }
 }
 

@@ -1322,8 +1322,8 @@ __global__ void __launch_bounds__(T, MINB) k2v5_orthant_walks(const K2Args A) {
     atomicAdd(&A.counters[CNT_BLOCKED], h.cnt[H_BLK]);
     atomicAdd(&A.counters[CNT_NOCONV], h.cnt[H_NOCONV]);
     atomicAdd(&A.counters[CNT_SPILLS], h.cnt[H_DRIFT]);
-    atomicMax(&A.counters[CNT_NUM + 24], (unsigned long long)__double_as_longlong(h.max_viol / h.cmax));
-    atomicAdd(&A.counters[CNT_NUM + 1 + 20], h.cnt[H_FOLD]);          // reported with the phase counters: fold passes
+    atomicMax(&A.counters[CNT_DRIFT], (unsigned long long)__double_as_longlong(h.max_viol / h.cmax));
+    atomicAdd(&A.counters[CNT_V5_FOLDS], h.cnt[H_FOLD]);
   }
 }
 
