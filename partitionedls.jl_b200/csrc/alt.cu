@@ -322,7 +322,8 @@ int k6_alt_run(const Problem &pb, SolveWs &ws, const std::vector<uint64_t> &h_gm
   PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem));
   if (occ < 1) occ = 1;
   const int max_grid = sm_count * occ;
-  const int grid = (int)std::min<long long>(max_grid, R);
+  int grid = (int)std::min<long long>(max_grid, R);
+  if (const char *eg = getenv("PLS_K6_GRID")) { const int g = atoi(eg); if (g >= 1 && g < grid) grid = g; }   // tests: several restarts per CTA
 
   // group membership lists
   std::vector<int> ptr(Kp + 1, 0), idx;

@@ -309,6 +309,8 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
   PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, TB, smem));
   if (occ < 1) occ = 1;
   const int max_grid = sm_count * occ;
+  int launch_grid = max_grid;                  // per-CTA bests (cta_*) stay sized and scanned by max_grid
+  if (const char *eg = getenv("PLS_BNB_GRID")) { const int g = atoi(eg); if (g >= 1 && g < max_grid) launch_grid = g; }   // tests: several nodes per CTA
 
   // state pool: a bounded share of the free memory
   size_t free_b = 0, total_b = 0;
@@ -318,7 +320,8 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
   if (n_slots > 65536) n_slots = 65536;
   if (shard && shard->stop_open > 0) n_slots = std::min<size_t>(n_slots, std::max<size_t>(2048, 16 * (size_t)shard->stop_open));   // frontier seeding pass: small pool
   if (const char *e = getenv("PLS_BNB_SLOTS")) n_slots = (size_t)atoll(e);
-  if (n_slots < 4) { set_error("bnb: not enough device memory for the state pool"); return PLS_ENOMEM; }
+  // the first wave takes a root only while more than K' + 2 slots are free: a smaller pool would launch an empty wave
+  if (n_slots < (size_t)Kp + 3) { set_error("bnb: state pool of %zu slots is too small (a root needs K + 4 = %d)", n_slots, Kp + 3); return PLS_ENOMEM; }
   const int wave_max = (int)std::min<size_t>((size_t)max_grid * 2, n_slots / 2);
 
   double *pool = nullptr, *mu = nullptr, *d_probe = nullptr;
@@ -394,7 +397,7 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
     }
     BNB_TRY(cudaMemcpyAsync(d_items, items.data(), sizeof(BnbItem) * n, cudaMemcpyHostToDevice, st));
     BNB_TRY(cudaMemsetAsync(d_ctr, 0, sizeof(unsigned long long), st));
-    kern<<<std::min(n, max_grid), TB, smem, st>>>(A);
+    kern<<<std::min(n, launch_grid), TB, smem, st>>>(A);
     BNB_TRY(cudaGetLastError());
     ++*launches; ++waves;
     BNB_TRY(cudaMemcpyAsync(out.data(), d_out, sizeof(BnbChild) * 2 * n, cudaMemcpyDeviceToHost, st));
