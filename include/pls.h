@@ -149,7 +149,9 @@ int pls_alt_fit_resident(pls_ctx *ctx, const double *beta0, int64_t R, double ep
 /* ---- resident data set: upload once, fit many times -------------------------------------------
  * pls_load copies rows [0, N) of X (leading dimension ldx >= N), y and P to the device in the
  * library's augmented layout Z = [X | 1 | y] (zero padded).  In a multi-process run each rank loads
- * its own row shard; n_total is the global row count (only used for reporting). */
+ * its own row shard; n_total is the global row count (only used for reporting).
+ * Widths: M <= 2047 (M' = M + 1 <= 2048), wider problems are refused here with PLS_EUNSUPPORTED.
+ * fit(BnB) and fit(Alt) need M' <= 1024 and return PLS_EUNSUPPORTED above it. */
 int pls_load(pls_ctx *ctx, const double *X, int64_t N, int64_t ldx, int64_t M, const double *y,
              const int64_t *P, int64_t K, double eta);
 int pls_opt_fit_resident(pls_ctx *ctx, uint32_t flags, double *alpha_raw, int64_t *b_best,

@@ -488,7 +488,10 @@ int pls_load(pls_ctx *c, const double *X, int64_t N, int64_t ldx, int64_t M, con
   if (!X || !y || !P) { set_error("null input pointer"); return PLS_EINVAL; }
   if (N < 1 || M < 1 || K < 1 || ldx < N) { set_error("bad shape N=%lld M=%lld K=%lld ldx=%lld", (long long)N, (long long)M, (long long)K, (long long)ldx); return PLS_EINVAL; }
   if (K + 1 > 64) { set_error("K = %lld: at most 63 groups (one bit per group and the intercept)", (long long)K); return PLS_EINVAL; }
-  if (M + 2 > 4096) { set_error("M = %lld exceeds this build's limit (4094)", (long long)M); return PLS_EUNSUPPORTED; }
+  if (M + 1 > MAX_MP) {
+    set_error("M = %lld: M' = M + 1 exceeds this build's limit of %d variables (M <= %d)", (long long)M, MAX_MP, MAX_MP - 1);
+    return PLS_EUNSUPPORTED;
+  }
   if (!(eta >= 0.0) || !std::isfinite(eta)) { set_error("eta must be finite and >= 0"); return PLS_EINVAL; }
   std::vector<uint64_t> gm((size_t)M + 1, 0);
   for (int64_t k = 0; k < K; ++k)

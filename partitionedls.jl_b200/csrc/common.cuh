@@ -25,6 +25,11 @@ void set_error(const char *fmt, ...);
 
 static inline int64_t round_up(int64_t a, int64_t b) { return (a + b - 1) / b * b; }
 
+// The widest problem every stage of an Opt fit supports, in variables M' = M + 1: K4 / K7 gather the winner's non-zero
+// weights in shared memory (resid.cu); above M' = 1024 K2 runs its single-pivot kernel with the inverse in global memory.
+// pls_load refuses wider problems, so that a fit cannot fail after its whole orthant enumeration.
+constexpr int MAX_MP = 2048;
+
 // NVTX range around a stage (header-only NVTX 3: a no-op unless a profiler is attached)
 struct NvtxRange {
   explicit NvtxRange(const char *name) { nvtxRangePushA(name); }

@@ -11,6 +11,7 @@ namespace {
 
 constexpr int T4 = 256;
 constexpr int MAXNZ = 2048;
+static_assert(MAXNZ >= MAX_MP, "K4 / K7 must take every width pls_load accepts");
 
 // One pass over the passive columns of Z for a tile of 64 rows per block: lane = row pair (16-byte loads,
 // a warp reads 512 contiguous bytes of a column), the 8 warps of the block split the non-zero columns
