@@ -64,11 +64,8 @@ __global__ void __launch_bounds__(T, MINB) k6_alt_restarts(const AltArgs A) {
   for (int m = tid; m < cap; m += T) { s.cs[m] = m < Mp ? A.c[m] : 0.0; s.gms[m] = m < Mp ? A.gmask[m] : 0ull; }
   for (int ti = tid; ti < ntc; ti += T)
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
-  if (tid == 0) {
-    for (int i = 0; i < PH_NUM; ++i) s.prof[i] = 0;
+  if (tid == 0)
     for (int i = 0; i < ST_NUM; ++i) s.stat[i] = 0;
-    s.stat[ST_TMARK] = clock64();
-  }
   const double yy = A.scal[0], cmax = A.scal[1];
   double best_obj = 0.0; long long best_r = -1;
   long long max_iters = 0;

@@ -108,12 +108,6 @@ int ensure_all_buffers(pls_ctx *c, int64_t count, bool want_obj, bool want_alpha
 
 void read_counters(pls_ctx *c, const unsigned long long *h) {
   pls_stats &s = c->stats;
-  if (getenv("PLS_K2_PHASES")) {
-    static const char *nm[] = {"start", "plan", "remove", "add", "grad", "refine", "out", "n_remove_blocks", "n_add_blocks",
-                               "r_gather", "r_panel", "r_rank", "r_zero", "a_gather", "a_hmul", "a_spart", "a_inv", "a_panel", "a_rank", "a_rows", "n_tab_sweep_in", "n_tab_unsweep", "tab_ops"};
-    for (int i = 0; i < 23; ++i) fprintf(stderr, "k2 phase %-16s %llu\n", nm[i], h[CNT_PHASE0 + i]);
-  }
-  if (getenv("PLS_K4_DRIFT")) fprintf(stderr, "k2v4 max KKT violation vs the original system / max|c| = %.3e, cold restarts %llu\n", counter_drift(h), h[CNT_SPILLS]);
   s.pivots = (int64_t)h[CNT_PIVOTS]; s.grad_evals = (int64_t)h[CNT_GRAD];
   s.sum_p = (int64_t)h[CNT_SUMP]; s.sum_p2 = (int64_t)h[CNT_SUMP2];
   s.bpp_iters = (int64_t)h[CNT_ITERS]; s.spills = (int64_t)h[CNT_SPILLS];

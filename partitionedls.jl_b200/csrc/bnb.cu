@@ -124,11 +124,8 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
   for (int m = tid; m < cap; m += T) { s.cs[m] = m < Mp ? A.c[m] : 0.0; s.gms[m] = m < Mp ? A.gmask[m] : 0ull; }
   for (int ti = tid; ti < ntc; ti += T)
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
-  if (tid == 0) {
-    for (int i = 0; i < PH_NUM; ++i) s.prof[i] = 0;
+  if (tid == 0)
     for (int i = 0; i < ST_NUM; ++i) s.stat[i] = 0;
-    s.stat[ST_TMARK] = clock64();
-  }
   const double yy = A.scal[0], cmax = A.scal[1];
   double best_obj = A.cta_obj[blockIdx.x];
   long long best_seq = A.cta_b[blockIdx.x];

@@ -60,14 +60,13 @@ static inline bool opt_better(double oa, long long ba, double ob, long long bb, 
 #define PLS_TIE_REL 1e-13
 
 // The counter block ws.counters (device side, unsigned long long each): the solver work counters accumulated by K2
-// (and by BnB / Alt), K2's chain scheduler, the per-phase cycle counters, the largest KKT drift.
+// (and by BnB / Alt), K2's chain scheduler, v5's fold passes, the largest KKT drift.
 enum Counter {
   CNT_PIVOTS = 0, CNT_GRAD, CNT_SUMP, CNT_SUMP2, CNT_ITERS, CNT_SPILLS, CNT_REBUILDS, CNT_BLOCKED,
-  CNT_NOCONV, CNT_NUM,
-  CNT_CHAIN = CNT_NUM,                    // dynamic chain scheduler of K2 (zeroed before every launch)
-  CNT_PHASE0,                             // 23 per-phase cycle counters (PLS_K2_PHASES)
-  CNT_V5_FOLDS = CNT_PHASE0 + 20,         // v5: fold passes, reported with the phase counters
-  CNT_DRIFT = CNT_PHASE0 + 23,            // largest KKT violation / max|c| of the two-level kernels, as double bits
+  CNT_NOCONV,
+  CNT_CHAIN,                              // dynamic chain scheduler of K2 (zeroed before every launch)
+  CNT_V5_FOLDS,                           // v5: fold passes (the kernel counts them; no host code reads the slot)
+  CNT_DRIFT,                              // largest KKT violation / max|c| of the two-level kernels, as double bits
   CNT_BLOCK_LEN
 };
 
@@ -187,8 +186,8 @@ int k2_solve_range(const Problem &pb, const double *G, int ldg, const double *c,
                    cudaStream_t st, int *launches, bool free_top = false, int force_variant = K2_DISPATCH,
                    const uint64_t *h_gmask = nullptr);
 // K2 variants: v1 = rank-1 updates on a dense inverse with a global-memory spill path (any M').
-// v3 = v2's algorithm with the inverse split between shared memory and an L2-resident global slice,
-// any thread count, M' <= 1024 (nnls3.cu)
+// v3 = block pivoting on FP64 tensor cores with the inverse split between shared memory and an L2-resident global
+// slice, any thread count, M' <= 1024 (nnls3.cu)
 struct K3Plan { int cap, qs, T, mode, occ, variant; size_t smem, hstride; };
 int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env = false);   // ignore_env: no PLS_K3_* tuning overrides
 int k2v3_launch(const K2Args &A, const K3Plan &pl, int grid, cudaStream_t st);
@@ -196,9 +195,7 @@ int k2v3_launch(const K2Args &A, const K3Plan &pl, int grid, cudaStream_t st);
 struct K4Plan { int cap, qs, T, mode, occ, variant, low_groups, verify_every; size_t smem, hstride, tabstride; };
 int k2v4_plan(int Mp, int Kp, K4Plan *pl, long long per_sm = 0);   // per_sm: problems per SM of this launch (0 = unknown)
 int k2v4_launch(const K2Args &A, const K4Plan &pl, int grid, cudaStream_t st);
-int k2v4_plan_prof(int Mp, int Kp, K4Plan *pl, long long per_sm = 0);      // nnls4p.cu: same kernels with phase counters
-int k2v4_launch_prof(const K2Args &A, const K4Plan &pl, int grid, cudaStream_t st);
-// v5 = two swept tableaus per Gray walk, one warp per walk (nnls5.cu)
+// v5 = two swept tableaus per Gray walk, one CTA per walk (nnls5.cu)
 struct K5Plan { int variant, T, NR, ld1, occ, low_groups, verify_every, cold_fused; size_t smem, tabstride; };
 int k2v5_plan(int Mp, int n_bits, const uint64_t *h_gmask, K5Plan *pl);
 int k2v5_launch(const K2Args &A, const K5Plan &pl, int grid, cudaStream_t st);

@@ -397,7 +397,7 @@ int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // ~4 waves of CTAs at 3 CTAs per SM (measured: 1 / 2 / 4 waves = 19.2 / 22.5 / 24.5 TFLOP/s at the configs[2] shape), chunks of whole stages
-  const int waves = getenv("PLS_K1_WAVES") ? atoi(getenv("PLS_K1_WAVES")) : 4;
+  const int waves = 4;
   long long want_chunks = ((long long)waves * 3 * sms + n_tiles - 1) / n_tiles;
   long long max_chunks = n_rows_pad / (KB * 8);
   if (max_chunks < 1) max_chunks = 1;
@@ -416,21 +416,13 @@ int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
   const char *impl = getenv("PLS_K1_IMPL");
   CUtensorMap zmap;
   if (!(impl && strcmp(impl, "v1") == 0) && make_zmap(pb, &zmap)) {
-    // pipeline shape (PLS_K1_PIPE = "stages x boxes" overrides).  Measured (profiles/r02_k1_pipe_sweep.txt): deeper rings
-    // do not help -- 2 stages of two 16-row boxes per side (64 KB, 3 CTAs per SM) beat 4 x 1, 6 x 1, 8 x 1 and 3 x 2 at
-    // every shape: the kernel is bound by DMMA issue, not by load latency.  More, shorter row chunks do help (4 waves).
-    int stages = 2, boxes = 2;
-    if (const char *ep = getenv("PLS_K1_PIPE")) sscanf(ep, "%dx%d", &stages, &boxes);
-    typedef void (*K1Fn)(const CUtensorMap, long long, long long, int, int, double *);
-    K1Fn fn = nullptr;
-    if (stages == 3 && boxes == 2) fn = k1_gram_tiles_tma<3, 2>;
-    else if (stages == 6 && boxes == 1) fn = k1_gram_tiles_tma<6, 1>;
-    else if (stages == 8 && boxes == 1) fn = k1_gram_tiles_tma<8, 1>;
-    else if (stages == 4 && boxes == 1) fn = k1_gram_tiles_tma<4, 1>;
-    else { stages = 2; boxes = 2; fn = k1_gram_tiles_tma<2, 2>; }
+    // pipeline shape.  Measured (profiles/r02_k1_pipe_sweep.txt): deeper rings do not help -- 2 stages of two 16-row
+    // boxes per side (64 KB, 3 CTAs per SM) beat 4 x 1, 6 x 1, 8 x 1 and 3 x 2 at every shape: the kernel is bound by
+    // DMMA issue, not by load latency.  More, shorter row chunks do help (4 waves).
+    constexpr int stages = 2, boxes = 2;
     const size_t smem = (size_t)stages * 2 * boxes * BOX_DOUBLES * sizeof(double) + 2 * stages * sizeof(uint64_t);
-    PLS_CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, T1B, smem, st>>>(zmap, rows_per_chunk, n_rows_pad, n_tiles, pb.zcols, pb.part);
+    PLS_CUDA_TRY(cudaFuncSetAttribute(k1_gram_tiles_tma<stages, boxes>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k1_gram_tiles_tma<stages, boxes><<<grid, T1B, smem, st>>>(zmap, rows_per_chunk, n_rows_pad, n_tiles, pb.zcols, pb.part);
   } else {
     k1_gram_tiles<<<grid, T1, 0, st>>>(pb.Z, pb.ldz, rows_per_chunk, n_rows_pad, n_tiles, pb.part);
   }

@@ -463,10 +463,9 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   NvtxRange nvtx("pls:K2 orthant NNLS + K3 argmin");
   if (b_count <= 0) { set_error("k2: empty orthant range"); return PLS_EINVAL; }
   if (free_top && (Mp > 1024 || d_all_obj || d_all_alpha)) { set_error("k2: paired orthants need M' <= 1024 and no per-orthant outputs"); return PLS_EUNSUPPORTED; }
-  // variant (PLS_K2_IMPL = v1 | v2 | v3 overrides):
-  //   v2  block pivoting, DMMA, tile-packed inverse entirely in shared memory   (M' <= 208)
-  //   v3  same algorithm, inverse split between shared memory and L2           (M' <= 1024)
-  //   v1  rank-1 updates on a dense inverse with a global spill path           (any M')
+  // variant (PLS_K2_IMPL = v1 | v3 | v4 | v5 overrides):
+  //   v3  block pivoting, DMMA, tile-packed inverse split between shared memory and L2   (M' <= 1024)
+  //   v1  rank-1 updates on a dense inverse with a global spill path                     (any M')
   const char *impl = getenv("PLS_K2_IMPL");
   int variant = Mp <= 1024 ? 3 : 1;
   if (impl && strcmp(impl, "v1") == 0 && !free_top) variant = 1;
@@ -478,7 +477,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   // per-orthant outputs (returnAllSolutions) stay on the one-level kernel: every orthant is then checked against
   // the original G (accuracy on ill-conditioned data matters more than speed on that path)
   if (variant == 3 && Mp + 1 <= 1024 && pow2 && (force4 || (impl && strcmp(impl, "v5") == 0) || (!impl && !d_all_obj && !d_all_alpha))) variant = 4;
-  // v5 (two swept tableaus, one warp per walk): preferred over v4 wherever its window fits (M' + 1 <= 584 and at
+  // v5 (two swept tableaus, one CTA per walk): preferred over v4 wherever its window fits (M' + 1 <= 640 and at
   // least one fast group) and the walks are long enough to amortise a cold start
   const bool force5 = impl && strcmp(impl, "v5") == 0;
   const bool no5 = getenv("PLS_K2_NO_V5") != nullptr;
@@ -502,7 +501,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   }
   if (variant == 4) {
     const long long per_sm = b_count / (sm_count > 0 ? sm_count : 1);
-    const int rc = getenv("PLS_K2_PHASES") ? k2v4_plan_prof(Mp, Kp, &plan4, per_sm) : k2v4_plan(Mp, Kp, &plan4, per_sm);
+    const int rc = k2v4_plan(Mp, Kp, &plan4, per_sm);
     if (rc == PLS_EUNSUPPORTED) variant = 3; else if (rc) return rc;
     else if (!force4 && b_count < (long long)sm_count * plan4.occ * (Mp <= 256 ? 24 : 96)) variant = 3;   // too short a walk per CTA
     else { cap = plan4.cap; occ = plan4.occ; smem = plan4.smem; }
@@ -542,7 +541,6 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   while (align_log2 < 62 && (((uint64_t)b_begin | (uint64_t)b_count) >> align_log2 & 1ull) == 0) ++align_log2;
   int chain_log2 = 0;
   while (chain_log2 < 8 && (b_count >> (chain_log2 + 1)) >= grid * (variant == 3 ? 4 : 8)) ++chain_log2;
-  if (const char *ec = getenv("PLS_K3_CHAIN")) chain_log2 = atoi(ec);
   if (chain_log2 > align_log2) chain_log2 = align_log2;
   if (chain_log2 > Kp) chain_log2 = Kp;
   long long n_chains = b_count >> chain_log2;
@@ -611,7 +609,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     A.qs = plan4.qs; A.hglob = ws.hspill; A.hstride = plan4.hstride;
     A.tab = ws.tab; A.tabstride = plan4.tabstride;
     A.lowmask = (1ull << plan4.low_groups) - 1ull; A.verify_every = plan4.verify_every;
-    const int rc = getenv("PLS_K2_PHASES") ? k2v4_launch_prof(A, plan4, (int)grid, st) : k2v4_launch(A, plan4, (int)grid, st);
+    const int rc = k2v4_launch(A, plan4, (int)grid, st);
     if (rc) return rc;
   } else if (variant == 3) {
     A.qs = plan3.qs; A.hglob = plan3.hstride ? ws.hspill : nullptr; A.hstride = plan3.hstride;

@@ -2,17 +2,17 @@
 // the inverse of the passive block kept as a tile-packed symmetric matrix that lives PARTLY in
 // shared memory and PARTLY in this CTA's private slice of global memory (L2-resident).
 //
-// Same mathematics and the same reference lines as nnls2.cu (src/PartitionedLSOpt.jl:85-96):
+// One NNLS problem per sign pattern b (src/PartitionedLSOpt.jl:85-96); each block pivot updates the inverse H of
+// the passive block:
 //
 //   remove R:  H <- H - H[:,R] inv(H[R,R]) H[R,:]                      (one rank-8 DMMA update)
 //   add    A:  U = H G[F,A];  S = G[A,A] - G[A,F] U;  T = U inv(S)
 //              H <- [H + T U', -T; -T', inv(S)]                         (one DMMA product + one update)
 //
-// What differs from nnls2.cu:
 //   * tile q of the packed lower triangle is in shared memory when q < qs and in global memory
 //     otherwise (MODE 0: all shared, 1: all global, 2: mixed).  The CTA therefore needs only
 //     ~45 KB (M' = 201) / ~110 KB (M' = 513) of shared memory, several CTAs share an SM and hide
-//     each other's barrier and L2 latencies, and M' is no longer capped by the 227 KB of one SM;
+//     each other's barrier and L2 latencies, and M' is not capped by the 227 KB of one SM;
 //   * every loop is written for any thread count T and any M' <= 1024 (the plan step scans the
 //     <= 32 chunks of 32 variables / 32 slots with one warp-wide prefix sum).
 #include "nnls3_core.cuh"
@@ -35,11 +35,8 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
 
   int hwm = 0, nt_cur = 0;
-  if (tid == 0) {
-    for (int i = 0; i < PH_NUM; ++i) s.prof[i] = 0;
+  if (tid == 0)
     for (int i = 0; i < ST_NUM; ++i) s.stat[i] = 0;
-    s.stat[ST_TMARK] = clock64();
-  }
   const double yy = A.scal[0], cmax = A.scal[1];
   const long long L = 1ll << A.chain_log2;
   double best_obj = 0.0; long long best_b = -1;
@@ -60,7 +57,6 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
     for (int m = tid; m < Mp; m += T) { s.w[m] = 0.0; s.r[m] = s.cs[m]; s.pos[m] = -1; }
     __syncthreads();
     bool r_valid = true;
-    PH_TICK3(PH_START);
 
     for (long long i = 0; i < L; ++i) {
       const long long b = base + (i ^ (i >> 1));
@@ -126,8 +122,6 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
     atomicAdd(&A.counters[CNT_REBUILDS], (unsigned long long)s.stat[ST_REBUILD]);
     atomicAdd(&A.counters[CNT_BLOCKED], (unsigned long long)s.stat[ST_BLOCKED]);
     atomicAdd(&A.counters[CNT_NOCONV], (unsigned long long)s.stat[ST_NOCONV]);
-    PH_TICK3(PH_OUT);
-    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_PHASE0 + i], (unsigned long long)s.prof[i]);
   }
 }
 
@@ -143,15 +137,14 @@ const Variant kVariants[] = {
     {256, 2, 2, k2v3_orthant_chains<256, 2, 2>}, {256, 1, 3, k2v3_orthant_chains<256, 1, 3>},
     {512, 0, 1, k2v3_orthant_chains<512, 0, 1>}, {512, 1, 1, k2v3_orthant_chains<512, 1, 1>},
     {512, 2, 1, k2v3_orthant_chains<512, 2, 1>},
-    {128, 1, 4, k2v3_orthant_chains<128, 1, 4>}, {128, 1, 5, k2v3_orthant_chains<128, 1, 5>},
-    {128, 1, 6, k2v3_orthant_chains<128, 1, 6>}, {128, 2, 4, k2v3_orthant_chains<128, 2, 4>},
-    {256, 1, 4, k2v3_orthant_chains<256, 1, 4>}, {256, 2, 3, k2v3_orthant_chains<256, 2, 3>},
+    {128, 1, 4, k2v3_orthant_chains<128, 1, 4>}, {128, 2, 4, k2v3_orthant_chains<128, 2, 4>},
+    {256, 2, 3, k2v3_orthant_chains<256, 2, 3>},
 };
 
 }  // namespace
 
 // Chooses thread count, storage mode and the number of shared-memory tiles.  Environment overrides
-// for tuning: PLS_K3_T (256|512), PLS_K3_QS (tiles in shared memory, -1 = all), PLS_K3_MINB.
+// for tuning: PLS_K3_T (128|256|512), PLS_K3_QS (tiles in shared memory, -1 = all).
 int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
   if (Mp > CAP3MAX) return PLS_EUNSUPPORTED;
   const int cap = (Mp + 7) & ~7;
@@ -159,8 +152,7 @@ int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
   int dev = 0, max_smem = 0;
   PLS_CUDA_TRY(cudaGetDevice(&dev));
   PLS_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  const char *eT = ignore_env ? nullptr : getenv("PLS_K3_T"), *eQ = ignore_env ? nullptr : getenv("PLS_K3_QS"),
-             *eB = ignore_env ? nullptr : getenv("PLS_K3_MINB");
+  const char *eT = ignore_env ? nullptr : getenv("PLS_K3_T"), *eQ = ignore_env ? nullptr : getenv("PLS_K3_QS");
   int T = eT ? atoi(eT) : (Mp <= 256 ? 128 : 256);   // measured: cfg2 15.3 ms at 4 x 128 threads per SM, M'=513 163 ms at 2 x 256
   if (T != 128 && T != 256 && T != 512) T = 256;
   while (Mp > 4 * T) T *= 2;
@@ -169,7 +161,7 @@ int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
   while (qs > 0 && v3_smem_bytes(cap, qs) > (size_t)max_smem) --qs;
   if (v3_smem_bytes(cap, qs) > (size_t)max_smem) { set_error("k2v3: M' = %d needs more shared memory than one SM has", Mp); return PLS_EUNSUPPORTED; }
   const int mode = qs == 0 ? 1 : (qs == ntiles ? 0 : 2);
-  int minb = eB ? atoi(eB) : (T == 128 ? 4 : (T == 256 ? (Mp <= 256 ? 3 : 2) : 1));
+  const int minb = T == 128 ? 4 : (T == 256 ? (Mp <= 256 ? 3 : 2) : 1);
   const Variant *best = nullptr;
   for (const Variant &v : kVariants)
     if (v.T == T && v.mode == mode && (!best || abs(v.minb - minb) < abs(best->minb - minb))) best = &v;
@@ -179,7 +171,6 @@ int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
   int oc = 1;
   PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&oc, best->fn, T, sm));
   if (oc < 1) oc = 1;
-  if (const char *eO = getenv("PLS_K3_OCC")) { const int o = atoi(eO); if (o >= 1 && o < oc) oc = o; }   // experiments: fewer CTAs per SM
   pl->cap = cap; pl->qs = qs; pl->T = T; pl->mode = mode; pl->occ = oc; pl->smem = sm;
   pl->variant = (int)(best - kVariants);
   pl->hstride = mode == 0 ? 0 : ((size_t)(ntiles - qs) << 6);

@@ -111,31 +111,18 @@ struct Sh3 {
   double *Pa, *Pb, *w, *r, *wF, *cs, *Sinv, *Gaa, *Spart, *rho, *theta, *cA, *red;
   double *yyr;                       // two-level mode: reduced y'y (one double)
   unsigned long long *gms;
-  long long *stat, *prof;
+  long long *stat;
   int *F, *pos, *lst, *asl, *ctl, *pl;
   unsigned short *tmap;
   signed char *sg, *dd, *vflag, *smark, *fl;
   signed char *swp, *ncm;            // two-level mode: variable is swept into the tableau / must not be committed
 };
 
-enum Phase3 { PH_START = 0, PH_PLAN, PH_REMOVE, PH_ADD, PH_GRAD, PH_REFINE, PH_OUT, PH_NREM, PH_NADD,
-              PH_R_GATHER, PH_R_PANEL, PH_R_RANK, PH_R_ZERO, PH_A_GATHER, PH_A_HMUL, PH_A_SPART, PH_A_INV, PH_A_PANEL,
-              PH_A_RANK, PH_A_ROWS, PH_A_INV1, PH_A_INV2, PH_A_INV3, PH_NUM };
-enum Stat3 { ST_P = 0, ST_PIV, ST_GRAD, ST_SUMP, ST_SUMP2, ST_ITER, ST_REBUILD, ST_BLOCKED, ST_NOCONV, ST_TMARK, ST_TSUB, ST_NUM };
-#ifndef PLS_K3_PROF
-#define PLS_K3_PROF 1     // per-phase cycle counters (clock64 by thread 0); nnls4.cu builds without them unless -DPLS_K4_PROF=1
-#endif
-#if PLS_K3_PROF
-#define PROF_ONLY3(x) x
-#define SUBTICK3(which) do { if (threadIdx.x == 0) { const long long now_ = clock64(); s.prof[which] += now_ - s.stat[ST_TSUB]; s.stat[ST_TSUB] = now_; } } while (0)
-#else
-#define PROF_ONLY3(x)
-#define SUBTICK3(which) do { } while (0)
-#endif
+enum Stat3 { ST_P = 0, ST_PIV, ST_GRAD, ST_SUMP, ST_SUMP2, ST_ITER, ST_REBUILD, ST_BLOCKED, ST_NOCONV, ST_NUM };
 #define STAT_ADD3(which, v) do { if (threadIdx.x == 0) s.stat[which] += (long long)(v); } while (0)
 
 __host__ __device__ inline size_t sh3_doubles(int cap) {
-  return 2 * (size_t)cap * 8 + 4 * (size_t)cap + 64 + 64 + 256 + 24 + 32 + (size_t)cap /*gms*/ + ST_NUM + PH_NUM;
+  return 2 * (size_t)cap * 8 + 4 * (size_t)cap + 64 + 64 + 256 + 24 + 32 + (size_t)cap /*gms*/ + ST_NUM;
 }
 __host__ __device__ inline size_t sh3_ints(int cap) {
   const int ntc = cap >> 3;
@@ -167,7 +154,6 @@ __device__ __forceinline__ Sh3 make_sh3(const Cfg3 &cf) {
   if (cf.tab) s.gms = const_cast<unsigned long long *>(cf.gmask_g);       // read-only in every kernel after set-up
   else { s.gms = reinterpret_cast<unsigned long long *>(dp); dp += cap; }
   s.stat = reinterpret_cast<long long *>(dp); dp += ST_NUM;
-  s.prof = reinterpret_cast<long long *>(dp); dp += PH_NUM;
   int *ip = reinterpret_cast<int *>(dp);
   s.F = ip; ip += cap;
   s.pos = ip; ip += cap;
@@ -362,7 +348,6 @@ __device__ __noinline__ void block_remove3(const Cfg3 cf, const int *Rs, int r, 
   constexpr int NW = T / 32;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int nrows = nt * 8;
-  PROF_ONLY3(if (tid == 0) s.stat[ST_TSUB] = clock64());
   if (wid < NW - 1) {                           // B = H[:, R]
     for (int idx = tid; idx < nrows * 8; idx += T - 32) {
       const int row = idx >> 3, q = idx & 7;
@@ -385,13 +370,10 @@ __device__ __noinline__ void block_remove3(const Cfg3 cf, const int *Rs, int r, 
     }
   }
   __syncthreads();
-  SUBTICK3(PH_R_GATHER);
   panel_small3<T>(s, s.Pb, s.Pa, s.theta, -1.0, nrows);   // Pa = -B inv(S);  w -= B phi
   __syncthreads();
-  SUBTICK3(PH_R_PANEL);
   rank_update3<T, MODE>(cf, nt);                          // H -= B inv(S) B'
   __syncthreads();
-  SUBTICK3(PH_R_RANK);
   for (int idx = tid; idx < nrows * 8; idx += T) {        // rows / columns R become exact zeros
     const int row = idx >> 3, q = idx & 7;
     if (q < r) h_set<MODE>(s, Rs[q], row, 0.0);
@@ -401,7 +383,6 @@ __device__ __noinline__ void block_remove3(const Cfg3 cf, const int *Rs, int r, 
     s.w[var] = 0.0; s.pos[var] = -1; s.F[sl] = -1;
   }
   __syncthreads();
-  SUBTICK3(PH_R_ZERO);
   if (tid == 0) { const long long p = s.stat[ST_P]; s.stat[ST_PIV] += r; s.stat[ST_SUMP2] += r * p * p; s.stat[ST_P] = p - r; }
 }
 
@@ -413,7 +394,6 @@ __device__ __noinline__ bool block_add3(const Cfg3 cf, const double *G, int ldg,
   constexpr int NW = T / 32;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int nrows = nt * 8;
-  PROF_ONLY3(if (tid == 0) s.stat[ST_TSUB] = clock64());
   if (wid < NW - 1) {                           // V = G[F, A]  (free slots: zero rows)
     for (int idx = tid; idx < nrows * 8; idx += T - 32) {
       const int row = idx >> 3, q = idx & 7;
@@ -432,10 +412,8 @@ __device__ __noinline__ bool block_add3(const Cfg3 cf, const double *G, int ldg,
     if (cf.gorig && lane >= 8 && lane < 16) { const int q = lane - 8; s.red[16 + q] = q < a ? cf.gorig[(size_t)cf.ldgo * Av[-q] + Av[-q]] : 1.0; }
   }
   __syncthreads();
-  SUBTICK3(PH_A_GATHER);
   hmul3<T, MODE>(cf, s.Pa, s.Pb, nt);           // U = H V
   __syncthreads();
-  SUBTICK3(PH_A_HMUL);
   constexpr int NSP = NW >= 8 ? 4 : (NW >= 4 ? 2 : 1);   // warps on the S partials; the rest on rho
   if (wid < NSP) {                              // S partials = V' U over interleaved k-steps
     const int fr = lane >> 2, fk = lane & 3;
@@ -458,7 +436,6 @@ __device__ __noinline__ bool block_add3(const Cfg3 cf, const double *G, int ldg,
     }
   }
   __syncthreads();
-  SUBTICK3(PH_A_SPART);
   if (wid == 0) {
     const int i = lane >> 2, j0 = (lane & 3) << 1;
     double e0 = s.Gaa[i * 8 + j0], e1 = s.Gaa[i * 8 + j0 + 1];
@@ -484,14 +461,11 @@ __device__ __noinline__ bool block_add3(const Cfg3 cf, const double *G, int ldg,
     if (lane == 0) s.ctl[4] = all_ok ? 1 : 0;
   }
   __syncthreads();
-  SUBTICK3(PH_A_INV);
   if (!s.ctl[4]) { __syncthreads(); return false; }
   panel_small3<T>(s, s.Pb, s.Pa, s.theta, 1.0, nrows);    // T = U inv(S) -> Pa;  w_F -= U theta
   __syncthreads();
-  SUBTICK3(PH_A_PANEL);
   rank_update3<T, MODE>(cf, nt);                          // H += T U'
   __syncthreads();
-  SUBTICK3(PH_A_RANK);
   for (int idx = tid; idx < nrows * 8; idx += T) {        // new rows / columns: -T
     const int row = idx >> 3, q = idx & 7;
     if (q < a && s.F[row] >= 0) h_set<MODE>(s, As[q], row, -s.Pa[pan(row, q)]);
@@ -507,7 +481,6 @@ __device__ __noinline__ bool block_add3(const Cfg3 cf, const double *G, int ldg,
     s.w[var] = s.theta[q]; s.F[sl] = var; s.pos[var] = sl;
   }
   __syncthreads();
-  SUBTICK3(PH_A_ROWS);
   if (tid == 0) { const long long p = s.stat[ST_P]; s.stat[ST_PIV] += a; s.stat[ST_SUMP2] += a * p * p; s.stat[ST_P] = p + a; }
   return true;
 }
@@ -782,10 +755,7 @@ __device__ __noinline__ bool tab_sweep_in3(const Cfg3 cf, const int *Bs, int nb,
   }
   __syncthreads();
   tab_refresh3<T>(cf, s, Mp);
-  if (tid == 0) {
-    s.stat[ST_P] -= nb; s.stat[ST_PIV] += nb; s.stat[ST_SUMP2] += (long long)nb * cap * cap / 2;
-    s.prof[PH_A_INV1]++;
-  }
+  if (tid == 0) { s.stat[ST_P] -= nb; s.stat[ST_PIV] += nb; s.stat[ST_SUMP2] += (long long)nb * cap * cap / 2; }
   __syncthreads();
   return true;
 }
@@ -873,21 +843,11 @@ __device__ __noinline__ void tab_unsweep3(const Cfg3 cf, const int *Bvar, int nb
   }
   __syncthreads();
   tab_refresh3<T>(cf, s, Mp);
-  if (tid == 0) {
-    s.stat[ST_P] += nb; s.stat[ST_PIV] += nb; s.stat[ST_SUMP2] += (long long)nb * cap * cap / 2;
-    s.prof[PH_A_INV2]++;
-  }
+  if (tid == 0) { s.stat[ST_P] += nb; s.stat[ST_PIV] += nb; s.stat[ST_SUMP2] += (long long)nb * cap * cap / 2; }
   st.hwm = hw_new; st.nt_cur = (hw_new + 7) >> 3;
   if (st.nt_cur > st.nt_dirty) st.nt_dirty = st.nt_cur;
   __syncthreads();
 }
-
-
-#if PLS_K3_PROF
-#define PH_TICK3(which) do { if (threadIdx.x == 0) { const long long now_ = clock64(); s.prof[which] += now_ - s.stat[ST_TMARK]; s.stat[ST_TMARK] = now_; } } while (0)
-#else
-#define PH_TICK3(which) do { } while (0)
-#endif
 
 // Block principal pivoting from the current passive set to the KKT point of
 //     min w'Gw - 2c'w   s.t.  sg_m w_m >= 0  (sg_m = +-1),  w_m = 0 (sg_m = 0),  w_m free (SG_FREE)
@@ -909,12 +869,9 @@ __device__ __forceinline__ bool bpp_solve3(const Cfg3 cf, const Sh3 &s, const do
     if (!st.r_valid) {
       int rep = 0;
       for (;;) {
-        PH_TICK3(PH_OUT);
         const double rf = grad_eval3<T, 4, TL && PLS_K4_KEEP>(cf, G, ldg, Mp, st.hwm);      // 4 row pairs per thread: M' <= 8 T
-        PH_TICK3(PH_GRAD);
         if (rf <= 1e-12 * cmax) break;          // carried solution already exact to working accuracy
         refine3<T, MODE>(cf, st.nt_cur);
-        PH_TICK3(PH_REFINE);
         if (rf <= 1e-9 * cmax) break;
         if (++rep >= 4) {                       // inverse degraded: rebuild by re-adding the passive set
           if (tid == 0) {
@@ -976,7 +933,6 @@ __device__ __forceinline__ bool bpp_solve3(const Cfg3 cf, const Sh3 &s, const do
         const int n3 = s.ctl[5];
         for (int q0 = 0; q0 < n3; q0 += 8) tab_unsweep3<T, MODE>(cf, s.lst + q0, min(8, n3 - q0), Mp, st);
         st.r_valid = true;                        // same point, same gradient: plan again
-        PH_TICK3(PH_A_INV3);
         continue;
       }
     } else {
@@ -988,7 +944,7 @@ __device__ __forceinline__ bool bpp_solve3(const Cfg3 cf, const Sh3 &s, const do
     int nr = tot & 0xffff, na = tot >> 16;
     const int mxi = warp_max_i(lane < nvch ? s.pl[32 + lane] : -1);
     const int nv = nr + na;
-    if (nv == 0) { st.r_valid = true; PH_TICK3(PH_PLAN); break; }   // KKT point; r stays valid for the next orthant
+    if (nv == 0) { st.r_valid = true; break; }   // KKT point; r stays valid for the next orthant
     // Murty's rule: only the highest index moves.  `safe`: from the first step on (the fallback of BnB nodes / Alt
     // restarts whose block-pivoting solve passed through a nearly singular intermediate passive set: one variable per
     // step behind the pivot test, as Lawson-Hanson, never forms such sets)
@@ -1043,11 +999,8 @@ __device__ __forceinline__ bool bpp_solve3(const Cfg3 cf, const Sh3 &s, const do
       __syncthreads();
     }
     st.nt_dirty = max(st.nt_dirty, nt_op);
-    PH_TICK3(PH_PLAN);
-    for (int q0 = 0; q0 < nr; q0 += 8) { block_remove3<T, MODE>(cf, s.lst + q0, min(8, nr - q0), nt_op); PROF_ONLY3(if (tid == 0) s.prof[PH_NREM]++); }
-    PH_TICK3(PH_REMOVE);
+    for (int q0 = 0; q0 < nr; q0 += 8) block_remove3<T, MODE>(cf, s.lst + q0, min(8, nr - q0), nt_op);
     for (int q0 = 0; q0 < na; q0 += 8) {
-      PROF_ONLY3(if (tid == 0) s.prof[PH_NADD]++);
       const int a = min(8, na - q0);
       if (!block_add3<T, MODE>(cf, G, ldg, s.lst + (cap - 1 - q0), s.asl + q0, a, nt_op)) {
         // numerically dependent column in the block: retry one variable at a time
@@ -1060,7 +1013,6 @@ __device__ __forceinline__ bool bpp_solve3(const Cfg3 cf, const Sh3 &s, const do
         }
       }
     }
-    PH_TICK3(PH_ADD);
     st.hwm = hw_after; st.nt_cur = (hw_after + 7) >> 3;
     STAT_ADD3(ST_ITER, 1);
     if (++iters > (safe ? 200 + 40 * Mp : 60 + 6 * Mp)) { ok = false; break; }

@@ -19,11 +19,6 @@
 //
 // Each CTA walks one contiguous piece of the Gray sequence of the whole range (static partition), so
 // the cold start (full solve + commit of ~3/4 of the passive set) is paid once per CTA.
-#ifndef PLS_K4_PROF
-#define PLS_K4_PROF 0          // nnls4p.cu compiles this file a second time with the per-phase cycle counters on
-#define K4_NAME(x) x
-#endif
-#define PLS_K3_PROF PLS_K4_PROF
 #include "nnls3_core.cuh"
 
 namespace pls {
@@ -83,11 +78,8 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
   const Sh3 s = make_sh3(cf);
   for (int ti = tid; ti < ntc; ti += T)
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
-  if (tid == 0) {
-    for (int i = 0; i < PH_NUM; ++i) s.prof[i] = 0;
+  if (tid == 0)
     for (int i = 0; i < ST_NUM; ++i) s.stat[i] = 0;
-    s.stat[ST_TMARK] = clock64();
-  }
   const double yy = A.scal[0], cmax = A.scal[1];
   double best_obj = 0.0; long long best_b = -1;
   int low_bits = 0;
@@ -128,7 +120,6 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
       if (tid == 0) *s.yyr = yy;
       __syncthreads();
       r_valid = true; cold = false; just_cold = true; since_check = 0;
-      PH_TICK3(PH_START);
     }
     const long long b = A.b_begin + (i ^ (i >> 1));
     const int fb = i > 0 ? __ffsll(i) - 1 : 63;                      // the group whose sign changed
@@ -143,7 +134,6 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
       if (forget) s.ncm[m] = 0;
     }
     __syncthreads();
-    PH_TICK3(PH_OUT);
 
     Bpp3 st; st.grow_zero = false; st.hwm = hwm; st.nt_cur = nt_cur; st.nt_dirty = nt_dirty; st.r_valid = r_valid;
     const bool ok = bpp_solve3<T, MODE, true>(cf, s, cf.tab, cf.ldt, Mp, cmax, st);
@@ -167,7 +157,6 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
     if (ok && (since_check >= check_every || i + 1 == i1)) {
       since_check = 0;
       const double viol = verify_true3<T>(cf, A.G, A.ldg, A.c, Mp);
-      PH_TICK3(PH_REFINE);
       if (!just_cold) max_viol = fmax(max_viol, viol);
       if (viol > 1e-13 * cmax && check_every > 8) check_every = 8;
       if (viol > 1e-12 * cmax && !just_cold) {       // tableau drifted: restart cold at this orthant
@@ -250,7 +239,6 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
         hwm = pn; nt_cur = ntr; nt_dirty = ntr;
         r_valid = false;
       }
-      PH_TICK3(PH_A_INV3);
     }
   }
   if (tid == 0) {
@@ -266,8 +254,6 @@ __global__ void __launch_bounds__(T, MINB) k2v4_orthant_ranges(const K2Args A) {
     atomicAdd(&A.counters[CNT_NOCONV], (unsigned long long)s.stat[ST_NOCONV]);
     atomicAdd(&A.counters[CNT_SPILLS], n_drift);      // reported as pls_stats.spills
     atomicMax(&A.counters[CNT_DRIFT], (unsigned long long)__double_as_longlong(max_viol / cmax));   // non-negative doubles order like integers
-    PH_TICK3(PH_OUT);
-    for (int i = 0; i < PH_NUM; ++i) atomicAdd(&A.counters[CNT_PHASE0 + i], (unsigned long long)s.prof[i]);
   }
 }
 
@@ -280,9 +266,8 @@ size_t v4_smem_bytes(int cap, int qs) {
 typedef void (*K4Fn)(const K2Args);
 struct Variant4 { int T, mode, minb; K4Fn fn; };
 const Variant4 kVariants4[] = {
-    {64, 1, 5, k2v4_orthant_ranges<64, 1, 5>}, {64, 1, 4, k2v4_orthant_ranges<64, 1, 4>}, {64, 1, 3, k2v4_orthant_ranges<64, 1, 3>},
-    {128, 1, 4, k2v4_orthant_ranges<128, 1, 4>}, {128, 1, 5, k2v4_orthant_ranges<128, 1, 5>},
-    {128, 2, 4, k2v4_orthant_ranges<128, 2, 4>}, {128, 1, 3, k2v4_orthant_ranges<128, 1, 3>},
+    {64, 1, 5, k2v4_orthant_ranges<64, 1, 5>},
+    {128, 1, 4, k2v4_orthant_ranges<128, 1, 4>}, {128, 2, 4, k2v4_orthant_ranges<128, 2, 4>},
     {256, 1, 2, k2v4_orthant_ranges<256, 1, 2>}, {256, 1, 3, k2v4_orthant_ranges<256, 1, 3>},
     {256, 2, 2, k2v4_orthant_ranges<256, 2, 2>}, {512, 1, 1, k2v4_orthant_ranges<512, 1, 1>},
 };
@@ -290,16 +275,15 @@ const Variant4 kVariants4[] = {
 }  // namespace
 
 // Environment overrides for tuning: PLS_K4_T, PLS_K4_QS (tiles of the small inverse in shared memory),
-// PLS_K4_MINB, PLS_K4_L (number of fast groups that are never committed), PLS_K4_VERIFY.
-int K4_NAME(k2v4_plan)(int Mp, int Kp, K4Plan *pl, long long per_sm) {
+// PLS_K4_L (number of fast groups that are never committed), PLS_K4_VERIFY.
+int k2v4_plan(int Mp, int Kp, K4Plan *pl, long long per_sm) {
   if (Mp + 1 > CAP3MAX) return PLS_EUNSUPPORTED;
   const int cap = (Mp + 1 + 7) & ~7;
   const int ntc = cap >> 3, ntiles = ntc * (ntc + 1) / 2;
   int dev = 0, max_smem = 0;
   PLS_CUDA_TRY(cudaGetDevice(&dev));
   PLS_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  const char *eT = getenv("PLS_K4_T"), *eQ = getenv("PLS_K4_QS"), *eB = getenv("PLS_K4_MINB"), *eL = getenv("PLS_K4_L"),
-             *eV = getenv("PLS_K4_VERIFY");
+  const char *eT = getenv("PLS_K4_T"), *eQ = getenv("PLS_K4_QS"), *eL = getenv("PLS_K4_L"), *eV = getenv("PLS_K4_VERIFY");
   // Short walks (few problems per SM: every CTA pays a cold start for little steady-state work) run better on fewer,
   // fatter CTAs: 3 x 256 threads per SM instead of 4 x 128 (cfg 2 with paired orthants, 443 problems per SM: 6.85 vs 7.09 ms;
   // at K = 20, 7 000 per SM, 4 x 128 is 10 % faster).
@@ -312,7 +296,7 @@ int K4_NAME(k2v4_plan)(int Mp, int Kp, K4Plan *pl, long long per_sm) {
   while (qs > 0 && v4_smem_bytes(cap, qs) > (size_t)max_smem) --qs;
   if (v4_smem_bytes(cap, qs) > (size_t)max_smem) { set_error("k2v4: M' = %d needs more shared memory than one SM has", Mp); return PLS_EUNSUPPORTED; }
   const int mode = qs == 0 ? 1 : 2;
-  const int minb = eB ? atoi(eB) : (T == 64 ? 5 : (T == 128 ? 4 : (T == 256 ? (short_walk ? 3 : 2) : 1)));
+  const int minb = T == 64 ? 5 : (T == 128 ? 4 : (T == 256 ? (short_walk ? 3 : 2) : 1));
   const Variant4 *best = nullptr;
   for (const Variant4 &v : kVariants4)
     if (v.T == T && v.mode == mode && (!best || abs(v.minb - minb) < abs(best->minb - minb))) best = &v;
@@ -322,7 +306,6 @@ int K4_NAME(k2v4_plan)(int Mp, int Kp, K4Plan *pl, long long per_sm) {
   int oc = 1;
   PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&oc, best->fn, T, sm));
   if (oc < 1) oc = 1;
-  if (const char *eO = getenv("PLS_K4_OCC")) { const int o = atoi(eO); if (o >= 1 && o < oc) oc = o; }
   // fast groups (never committed).  Measured optimum: l = 5 at M' = 201 (groups of 12), l = 6 at M' = 513
   // (groups of 30): a larger l makes the full-tableau updates rarer (every 2^l orthants) and the small
   // inverse / gradient columns larger; both terms grow with M', so l moves little.
@@ -341,7 +324,7 @@ int K4_NAME(k2v4_plan)(int Mp, int Kp, K4Plan *pl, long long per_sm) {
   return PLS_OK;
 }
 
-int K4_NAME(k2v4_launch)(const K2Args &A, const K4Plan &pl, int grid, cudaStream_t st) {
+int k2v4_launch(const K2Args &A, const K4Plan &pl, int grid, cudaStream_t st) {
   kVariants4[pl.variant].fn<<<grid, pl.T, pl.smem, st>>>(A);
   PLS_CUDA_TRY(cudaGetLastError());
   return PLS_OK;

@@ -29,7 +29,7 @@ K2_VARIANTS = {
     "v5": {"PLS_K2_IMPL": "v5", "PLS_K5_GRID": "3", "PLS_K5_L": "2", "PLS_K5_VERIFY": "5"},
     "v5w": {"PLS_K2_IMPL": "v5", "PLS_K5_GRID": "2", "PLS_K5_L": "1", "PLS_K5_T": "64", "PLS_K5_NR": "64"},
 }
-_K2_KEYS = ("PLS_K2_IMPL", "PLS_K3_QS", "PLS_K3_T", "PLS_K3_MINB", "PLS_K4_GRID", "PLS_K4_L", "PLS_K4_VERIFY", "PLS_K4_QS", "PLS_K4_T",
+_K2_KEYS = ("PLS_K2_IMPL", "PLS_K3_QS", "PLS_K3_T", "PLS_K4_GRID", "PLS_K4_L", "PLS_K4_VERIFY", "PLS_K4_QS", "PLS_K4_T",
             "PLS_K5_GRID", "PLS_K5_L", "PLS_K5_VERIFY", "PLS_K5_T", "PLS_K5_NR", "PLS_K5_MARGIN", "PLS_K2_NO_V5")
 # the kernel a winner-only fit of a long aligned range runs (pls_stats.k2_variant)
 DEFAULT_TWOLEVEL = 5

@@ -21,9 +21,8 @@ import pytest
 pytestmark = pytest.mark.gpu
 RTOL = 1e-9
 ETA = 1e-3
-K2_KEYS = ("PLS_K2_IMPL", "PLS_K2_NO_V5", "PLS_K2_PHASES", "PLS_K3_QS", "PLS_K3_T", "PLS_K3_MINB", "PLS_K3_OCC",
-           "PLS_K3_CHAIN", "PLS_K4_GRID", "PLS_K4_L", "PLS_K4_VERIFY", "PLS_K4_QS", "PLS_K4_T", "PLS_K4_MINB", "PLS_K4_OCC",
-           "PLS_K5_GRID", "PLS_K5_L", "PLS_K5_VERIFY", "PLS_K5_T", "PLS_K5_NR", "PLS_K5_MARGIN", "PLS_K5_FUSED",
+K2_KEYS = ("PLS_K2_IMPL", "PLS_K2_NO_V5", "PLS_K3_QS", "PLS_K3_T", "PLS_K4_GRID", "PLS_K4_L", "PLS_K4_VERIFY",
+           "PLS_K4_QS", "PLS_K4_T", "PLS_K5_GRID", "PLS_K5_L", "PLS_K5_VERIFY", "PLS_K5_T", "PLS_K5_NR", "PLS_K5_MARGIN", "PLS_K5_FUSED",
            "PLS_K5_OCC")
 
 

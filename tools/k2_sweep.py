@@ -21,7 +21,7 @@ ctx.gram_build(); ctx.gram_finalize()
 total = 1 << (K + 1)
 if os.environ.get("SWEEP_COUNT_LOG2"):
     total = min(total, 1 << int(os.environ["SWEEP_COUNT_LOG2"]))   # an aligned sub-range of the enumeration
-KEYS = ("PLS_K4_DIRECT", "PLS_K4_L", "PLS_K4_T", "PLS_K4_QS", "PLS_K4_MINB", "PLS_K4_VERIFY", "PLS_K4_GRID", "PLS_K4_OCC", "PLS_K2_IMPL", "PLS_K3_QS", "PLS_K3_T", "PLS_K3_MINB", "PLS_K3_CHAIN", "PLS_K2_PHASES", "PLS_K3_OCC")
+KEYS = ("PLS_K4_DIRECT", "PLS_K4_L", "PLS_K4_T", "PLS_K4_QS", "PLS_K4_VERIFY", "PLS_K4_GRID", "PLS_K2_IMPL", "PLS_K3_QS", "PLS_K3_T")
 ref = None
 for setting in sys.argv[2:]:
     for k in KEYS:
