@@ -22,7 +22,7 @@
 // which yields the implied weight of every committed variable, the gradient of every active one, the
 // objective (v[rhs] = y'y - c_P' w_P) and -- on the rows of S themselves -- the residual of the S-system, an
 // independent accuracy check of T2.  A variable outside the window that violates its condition JOINS the window
-// (one |S| x |R| product; T1 is not touched) and is toggled like any other.  After a slow Gray group has moved,
+// (up to 8 at a time: one 8 x |S| x |R| DMMA product; T1 is not touched) and is toggled like any other.  After a slow Gray group has moved,
 // or when the window fills up, the toggled SLOW variables are folded into T1 (mixed forward / reverse block
 // sweep: T1 -= P inv(D) P', one DMMA pass per <= 8 variables) and the untoggled slow ones leave the window.
 //
@@ -61,11 +61,6 @@ __device__ __forceinline__ double rcp5(double x) {
   e = fma(-x, r, 1.0);
   return fma(r, e, r);
 }
-__device__ __forceinline__ double wsum5(double v) {
-#pragma unroll
-  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 __device__ __forceinline__ double wmax5(double v) {
 #pragma unroll
   for (int o = 16; o; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
@@ -92,8 +87,8 @@ __device__ __forceinline__ int pan5(int row, int col) { return (row << 3) + (col
 struct Sh5 {
   double *T2;      // [t2_doubles(NR)]  (aliased by the fold's W panel: ld1 x 8)
   double *v;       // [ld1]   streaming result
-  double *Pp, *Wp; // [NR x 8] block pivot: P = T2[:, B], W = P inv(D)   (Wp doubles as the join's scratch)
-  double *yv;      // [NR]    y_s of the S list (stream), coefficients (join)
+  double *Pp, *Wp; // [NR x 8] block pivot: P = T2[:, B], W = P inv(D)   (join: U' and the new rows)
+  double *yv;      // [NR]    y_s of the S list (stream), e_k (fused fold)
   double *D;       // [64]    8 x 8 pivot block, then its inverse
   double *gd;      // [8]     pivot references of the entering variables of a block
   double *red;     // [32]    block reductions
@@ -102,7 +97,7 @@ struct Sh5 {
   short *slot;     // [ld1]   window slot of variable m, -1 outside
   short *rvar;     // [NR]    variable of window slot k (slot 0 = the right-hand side, variable index Mp)
   short *lst;      // [ld1]   list scratch (leaving list / S list / join list)
-  short *lstE;     // [NR]    entering list / fold list
+  short *lstE;     // [NR]    entering list / fold list / the join's toggled slots
   short *lstB;     // [8]     slots of the current block
   unsigned short *tmap; // [NR/8 (NR/8 + 1) / 2] tile coordinates (ti << 8 | tj) of the packed tile sequence
   signed char *sg; // [ld1]
@@ -553,26 +548,68 @@ __device__ __noinline__ void stream5(int n) {
   if (tid == 0) { hdr5().cnt[H_STREAM]++; hdr5().cnt[H_SUMS] += ns; }
 }
 
-// ---- a variable outside the window joins it (not toggled): new last row of T2 ------------------------------------
-//   row[j] = [slot j not toggled] T1[m, var_j] - sum_{s toggled} e_s T1[m, s] T2[s, j],   diag = T1[m, m] - sum_s e_s T1[m, s] row[s]
+// ---- up to 8 variables outside the window join it (not toggled): new rows n .. n + nk - 1 of T2 ---------------------
+// J = the entries of Jl[0 .. nj) that are still outside the window (nk <= 8 of them, in list order), S = the toggled
+// slots, E = diag(e_s), U = T1[J, S] E (gathered once, row s of Pp holds column s of U):
+//     T2[J, Rb] = [col not in S] T1[J, Rb] - U T2[S, Rb]     one DMMA product (K = |S|), stored column-wise in Wp
+//     T2[J, J]  = T1[J, J] - U T2[J, S]'                     (a joiner counts as an untoggled slot for the later ones)
+// -- the algebra of one join after another, with the |S|-long FMA chains of each replaced by DMMA steps of 4.  With
+// S empty (the first round of a cold solve) it is a gather.  Returns nk.
 template <int T, int NR>
-__device__ __noinline__ void join5(int n, int m) {
+__device__ __noinline__ int join_block5(int n, const short *Jl, int nj) {
   const H5 &h = hdr5();
   const Sh5 s = make_sh5(NR, h.ld1);
-  const int tid = threadIdx.x;
-  const double *row1 = h.T1r + (size_t)h.ld1 * m;
-  double *rowv = s.Wp, *tog = s.Wp + NR;              // scratch: the new row, toggled marks
-  // toggled slots -> lstE, coefficients e_s T1[m, s] -> yv, in slot order (all threads; per-warp counts through shared memory)
+  constexpr int NW = T / 32, TPW = (NR / 8 + NW - 1) / NW;   // column tiles of the window per warp
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int fr = lane >> 2, fk = lane & 3;
+  const size_t ld1 = h.ld1;
+  const double *T1r = h.T1r;
+  // every thread lists the joiners itself (slot[] changes only at the end of this call): nk, and the variables of
+  // joiners fr, 2 fk, 2 fk + 1 (its DMMA fragments) and tid (the bookkeeping); -1: none
+  int nk = 0, m_r = -1, m_c0 = -1, m_c1 = -1, m_t = -1;
+  #pragma unroll 1
+  for (int q = 0; q < nj; ++q) {
+    const int m = Jl[q];
+    if (s.slot[m] >= 0) continue;
+    if (nk == tid) m_t = m;
+    if (nk == fr) m_r = m;
+    if (nk == 2 * fk) m_c0 = m;
+    if (nk == 2 * fk + 1) m_c1 = m;
+    ++nk;
+  }
+  // the block T1[J, J] (last warp) and the rows T1[J, Rb] of the untoggled slots are read before anything else: their
+  // L2 round trips overlap the gather of U
+  const auto untoggled = [&](int j) {
+    if (j <= 0 || j >= n) return j == 0;
+    const unsigned char f = s.st[s.rvar[j]];
+    return ((f & ST_PAS) != 0) == ((f & ST_INO) != 0);
+  };
+  double2 acc[TPW];
+#pragma unroll
+  for (int u = 0; u < TPW; ++u) {
+    const int j = (wid + u * NW) * 8 + fr;
+    double x0 = 0.0, x1 = 0.0;
+    if (untoggled(j)) {
+      const int vj = s.rvar[j];
+      if (m_c0 >= 0) x0 = __ldcg(T1r + ld1 * m_c0 + vj);
+      if (m_c1 >= 0) x1 = __ldcg(T1r + ld1 * m_c1 + vj);
+    }
+    acc[u] = make_double2(x0, x1);
+  }
+  double2 blk = make_double2(0.0, 0.0);
+  if (wid == NW - 1 && m_r >= 0) {
+    if (m_c0 >= 0) blk.x = __ldcg(T1r + ld1 * m_r + m_c0);
+    if (m_c1 >= 0) blk.y = __ldcg(T1r + ld1 * m_r + m_c1);
+  }
+  // toggled slots -> lstE, U -> Pp (row p: e_s T1[J, var_s], zero past nk), in slot order (all threads; per-warp
+  // counts through shared memory)
   int ns = 0;
   {
-    constexpr int NW = T / 32;
-    const int lane = tid & 31, wid = tid >> 5;
     int *ri = reinterpret_cast<int *>(s.red);
     #pragma unroll 1
     for (int k0 = 1; k0 < n; k0 += T) {
       const int k = k0 + tid;
-      bool tg = false, pas = false; int var = 0;
-      if (k < n) { var = s.rvar[k]; const unsigned char f = s.st[var]; pas = f & ST_PAS; tg = pas != ((f & ST_INO) != 0); }
+      const bool tg = k < n && !untoggled(k);
       const unsigned bal = __ballot_sync(0xffffffffu, tg);
       if (k0 > 1) SYNC5();
       if (lane == 0) ri[wid] = __popc(bal);
@@ -580,31 +617,73 @@ __device__ __noinline__ void join5(int n, int m) {
       int off = ns;
 #pragma unroll
       for (int w2 = 0; w2 < NW; ++w2) { const int c = ri[w2]; if (w2 < wid) off += c; ns += c; }
-      if (tg) { const int p = off + __popc(bal & ((1u << lane) - 1)); s.lstE[p] = (short)k; const double a = __ldcg(row1 + var); s.yv[p] = pas ? a : -a; }
-      if (k < n) tog[k] = tg ? 1.0 : 0.0;
+      if (tg) {
+        const int p = off + __popc(bal & ((1u << lane) - 1)), var = s.rvar[k];
+        const double e = (s.st[var] & ST_PAS) ? 1.0 : -1.0;
+        s.lstE[p] = (short)k;
+        int a = 0;
+        #pragma unroll 1
+        for (int q = 0; q < nj; ++q) {
+          const int m = Jl[q];
+          if (s.slot[m] < 0) s.Pp[pan5(p, a++)] = e * __ldcg(T1r + ld1 * m + var);
+        }
+        #pragma unroll 1
+        for (; a < 8; ++a) s.Pp[pan5(p, a)] = 0.0;
+      }
     }
-    if (tid == 0) tog[0] = 0.0;
   }
   SYNC5();
-  #pragma unroll 1
-  for (int j = tid; j < n; j += T) {
-    double a = tog[j] != 0.0 ? 0.0 : __ldcg(row1 + s.rvar[j]);
+  // Wp[j][a] = T2new[a, j]:  C = T2[Rb, S] (-U)'  on top of the untoggled T1 entries; a warp takes column tiles
+  // wid, wid + NW, ... of the window, two accumulators per tile (even / odd steps of 4)
+  {
+    const int ntr = (n + 7) >> 3;
+    double2 acc2[TPW];
+#pragma unroll
+    for (int u = 0; u < TPW; ++u) acc2[u] = make_double2(0.0, 0.0);
     #pragma unroll 1
-    for (int p = 0; p < ns; ++p) a = fma(-s.yv[p], t2_get(s.T2, s.lstE[p], j), a);
-    rowv[j] = a;
+    for (int k0 = 0; k0 < ns; k0 += 8) {
+      const int p0 = k0 + fk, p1 = k0 + 4 + fk;
+      const int s0 = p0 < ns ? s.lstE[p0] : 0, s1 = p1 < ns ? s.lstE[p1] : 0;
+      const double b0 = p0 < ns ? -s.Pp[pan5(p0, fr)] : 0.0, b1 = p1 < ns ? -s.Pp[pan5(p1, fr)] : 0.0;
+#pragma unroll
+      for (int u = 0; u < TPW; ++u) {
+        const int j = (wid + u * NW) * 8 + fr;
+        if (wid + u * NW < ntr) {
+          dmma5(acc[u].x, acc[u].y, t2_get(s.T2, j, s0), b0);
+          dmma5(acc2[u].x, acc2[u].y, t2_get(s.T2, j, s1), b1);
+        }
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < TPW; ++u)
+      if (wid + u * NW < ntr) {
+        const int j = (wid + u * NW) * 8 + fr;
+        *reinterpret_cast<double2 *>(s.Wp + pan5(j, 2 * fk)) = make_double2(acc[u].x + acc2[u].x, acc[u].y + acc2[u].y);
+      }
   }
   SYNC5();
-  #pragma unroll 1
-  for (int j = tid; j < n; j += T) t2_set(s.T2, n, j, rowv[j]);
-  if (tid < 32) {
-    double dg = 0.0;
+  if (wid == NW - 1) {                                 // the block among J: T1[J, J] - U Wp[S, :]
+    double2 blk2 = make_double2(0.0, 0.0);
     #pragma unroll 1
-    for (int p = tid; p < ns; p += 32) dg = fma(s.yv[p], rowv[s.lstE[p]], dg);
-    dg = wsum5(dg);
-    if (tid == 0) { t2_set(s.T2, n, n, __ldcg(row1 + m) - dg); s.rvar[n] = (short)m; s.slot[m] = (short)n; }
+    for (int k0 = 0; k0 < ns; k0 += 8) {
+      const int p0 = k0 + fk, p1 = k0 + 4 + fk;
+      const double a0 = p0 < ns ? -s.Pp[pan5(p0, fr)] : 0.0, a1 = p1 < ns ? -s.Pp[pan5(p1, fr)] : 0.0;
+      const double b0 = p0 < ns ? s.Wp[pan5(s.lstE[p0], fr)] : 0.0, b1 = p1 < ns ? s.Wp[pan5(s.lstE[p1], fr)] : 0.0;
+      dmma5(blk.x, blk.y, a0, b0);
+      dmma5(blk2.x, blk2.y, a1, b1);
+    }
+    if (fr < nk && 2 * fk <= fr) t2_set(s.T2, n + fr, n + 2 * fk, blk.x + blk2.x);
+    if (fr < nk && 2 * fk + 1 <= fr) t2_set(s.T2, n + fr, n + 2 * fk + 1, blk.y + blk2.y);
   }
-  if (tid == 0) hdr5().cnt[H_SUMP2] += (unsigned long long)(ns * n) >> 1;
+  if (tid < nk) { s.rvar[n + tid] = (short)m_t; s.slot[m_t] = (short)(n + tid); }
+  #pragma unroll 1
+  for (int idx = tid; idx < nk * n; idx += T) {        // the new rows
+    const int a = idx / n, j = idx - a * n;
+    t2_set(s.T2, n + a, j, s.Wp[pan5(j, a)]);
+  }
+  if (tid == 0) hdr5().cnt[H_SUMP2] += ((unsigned long long)ns * n * nk) >> 1;
   SYNC5();
+  return nk;
 }
 
 // ---- fold: the toggled slow window variables B (<= 8, swept-back ones first) are swept in T1 ----------------------
@@ -1128,10 +1207,10 @@ __device__ __forceinline__ bool solve5(const Sh5 s, int &n_win, bool cold_mode, 
       if (room > nj) room = nj;
       if (room <= 0) return false;                     // the fast groups alone fill the window (the host sized l to prevent this)
       #pragma unroll 1
-      for (int p = 0; p < room; ++p) { const int m = park[p]; if (s.slot[m] < 0) { join5<T, NR>(n_win, m); ++n_win; } }
+      for (int p = 0; p < room; p += 8) n_win += join_block5<T, NR>(n_win, park + p, min(8, room - p));   // (skips parked fast variables)
     } else {
       #pragma unroll 1
-      for (int p = 0; p < nj; ++p) { join5<T, NR>(n_win, s.lst[p]); ++n_win; }     // join5 uses lstE / yv / tv / uv, not lst
+      for (int p = 0; p < nj; p += 8) n_win += join_block5<T, NR>(n_win, s.lst + p, min(8, nj - p));     // (uses lstE / Pp / Wp, not lst)
     }
     t_best = Mp + 1; pbar = 3;
   }

@@ -7,8 +7,8 @@ The passive set is P = O xor S.  For m in R the last column of T2 holds the weig
 (m active); for m outside R one streaming pass over the rows T1[S, :] gives
       v = T1[:, rhs] - sum_s T1[:, s] * (e_s * T2[s, rhs]),   e_s = +1 (s swept forward) / -1 (swept back)
 = weight (m in O) or gradient (m active), and for m in S the residual of the S-system (accuracy check).
-A variable outside R that violates its condition JOINS R (one |S| x |R| product, no T1 update) and is then
-toggled like any other.  When a slow Gray group has moved / R is full, the toggled SLOW variables are FOLDED
+A variable outside R that violates its condition JOINS R (no T1 update; up to 8 at a time: one 8 x |S| x |R|
+product) and is then toggled like any other.  When a slow Gray group has moved / R is full, the toggled SLOW variables are FOLDED
 into T1 (rank-8 block updates) and the untoggled slow ones leave R.
 
   python tools/proto_v5.py N M K l n_steps [rho] [capR]
@@ -43,7 +43,7 @@ class V5:
         self.R = list(np.flatnonzero(self.fast))          # window (variable indices), rhs handled as index Mp
         self.tog = {}                                      # var -> +1 (forward swept in T2) / -1 (swept back)
         self.rebuild_T2()
-        self.stat = dict(sweeps2=0, streams=0, joins=0, folds=0, fold_vars=0, fold_passes=0, iters=0, maxR=0, sumS=0, sumR=0, n=0, blocked=0)
+        self.stat = dict(sweeps2=0, streams=0, joins=0, join_calls=0, folds=0, fold_vars=0, fold_passes=0, iters=0, maxR=0, sumS=0, sumR=0, n=0, blocked=0)
 
     # -- T2 helpers
     def rebuild_T2(self):
@@ -92,6 +92,33 @@ class V5:
         self.T2 = T
         self.R.append(m)
         self.stat["joins"] += 1
+
+    def join_block(self, J):
+        """up to 8 variables outside the window join it in one step (nnls5.cu: join_block5).  With S the toggled window
+        slots, E = diag(e_s) and U = T1[J, S] E:
+            T2[J, Rb] = [col not in S] T1[J, Rb] - U T2[S, Rb],    T2[J, J] = T1[J, J] - U T2[J, S]'
+        -- join() applied to J[0], J[1], ... in turn, with a joiner an untoggled slot for the later ones."""
+        J = [m for m in J if m not in self.R]
+        if not J:
+            return 0
+        idx = self.R + [self.Mp]
+        ks = [k for k, m in enumerate(self.R) if m in self.tog]
+        U = self.T1[np.ix_(J, [self.R[k] for k in ks])] * np.array([float(self.tog[self.R[k]]) for k in ks])
+        rows = self.T1[np.ix_(J, idx)].copy()
+        rows[:, ks] = 0.0
+        rows -= U @ self.T2[ks, :]
+        blk = self.T1[np.ix_(J, J)] - U @ rows[:, ks].T
+        n, k = len(self.R), len(J)
+        T = np.zeros((n + k + 1, n + k + 1))
+        old = list(range(n)) + [n + k]                    # the rhs stays last
+        T[np.ix_(old, old)] = self.T2
+        T[n:n + k, old] = rows; T[old, n:n + k] = rows.T
+        T[n:n + k, n:n + k] = blk
+        self.T2 = T
+        self.R += J
+        self.stat["joins"] += k
+        self.stat["join_calls"] = self.stat.get("join_calls", 0) + 1
+        return k
 
     def fold(self, all_slow=True):
         """toggled slow variables -> T1 (blocks of <= 8, swept-back ones first); untoggled slow variables leave R"""
@@ -213,8 +240,8 @@ class V5:
                 else:
                     self.fold()
                 room = self.capR - len(self.R)
-            for m in J[:room]:
-                self.join(m)
+            for q in range(0, min(room, len(J)), 8):
+                self.join_block(J[q:min(q + 8, room)])
             t_best, pbar = Mp + 1, 3
 
     def full_weights(self, v):
