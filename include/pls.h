@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PLS_VERSION 100 /* 0.1.0 */
+#define PLS_VERSION 110 /* 0.1.1: pls_opt_fit_path */
 
 enum {
   PLS_OK = 0,
@@ -157,6 +157,21 @@ int pls_load(pls_ctx *ctx, const double *X, int64_t N, int64_t ldx, int64_t M, c
 int pls_opt_fit_resident(pls_ctx *ctx, uint32_t flags, double *alpha_raw, int64_t *b_best,
                          double *obj_best, double *all_obj, double *all_alpha, pls_stats *stats);
 
+/* ---- regularisation path: fit(Opt) for several eta on the resident data set -------------------------
+ * Result l is what pls_load(..., eta = etas[l]) followed by pls_opt_fit_resident(ctx, flags, ...) returns: same b,
+ * alpha, objective.  The raw Gram sums S = Z'Z are built once (not at all when the context's Gram matrix is already
+ * finalised); G_l = S + eta_l Po Po' is formed for every eta in one launch.  Where the fit of one eta would run the
+ * one-level K2 kernel (short ranges), all L ranges are solved in one launch; otherwise one launch per eta.  One K4
+ * pass over X evaluates all L winners.  On a multi-GPU context the eta values are dealt round-robin to the devices.
+ *   etas[L]              1 <= L <= 64, each finite and >= 0, any order, duplicates allowed
+ *   alpha_raw[(M+1) x L] column l = raw alpha of eta_l's winner;  b_best[L], obj_best[L] as in pls_opt_fit
+ *   flags                PLS_FLAG_NO_RECOMPUTE and PLS_FLAG_ENUMERATE_INTERCEPT as for pls_opt_fit_resident
+ *   stats                of the whole call (ms_gram: K1 + the batched finalise, ms_nnls: all K2 + K3, ms_recompute:
+ *                        the K4 pass; orthants = L 2^(K+1), nnls_problems = L times the problems of one fit)
+ * The context's own eta, G and c are not changed.  M + 1 > 1024: PLS_EUNSUPPORTED (fit each eta on its own). */
+int pls_opt_fit_path(pls_ctx *ctx, const double *etas, int64_t L, uint32_t flags, double *alpha_raw, int64_t *b_best,
+                     double *obj_best, pls_stats *stats);
+
 /* ---- stage-wise entry points (one process per GPU; the caller owns the collectives) ----------
  * K1 on the loaded rows.  pls_gram_raw exposes the device buffer of raw sums S = Z'Z
  * ((M+2) x (M+2) doubles, column-major, lower triangle valid) so the caller can all-reduce it in
@@ -207,6 +222,9 @@ int pls_gram(pls_ctx *ctx, const double *X, int64_t N, int64_t M, const double *
  * alpha_signed_out[i * (M+1) ...] = alpha_p - alpha_n.  Each node is solved cold by the K5 kernel. */
 int pls_bnb_lower_bounds(pls_ctx *ctx, const uint64_t *pos_masks, const uint64_t *neg_masks, int64_t n, double *lb_out,
                          double *alpha_signed_out);
+/* pls_residual_partial_multi: the K4 pass of pls_opt_fit_path on the resident rows for L <= 64 signed weight vectors
+ * W[l * (M+1) + m]: ssq_out[l] = sum over the loaded rows of (Xo * w_l - y)^2 (one-GPU context). */
+int pls_residual_partial_multi(pls_ctx *ctx, const double *W, int64_t L, double *ssq_out);
 int pls_nnls_batch(pls_ctx *ctx, const double *G, const double *c, double yy, int64_t Mp,
                    const uint64_t *gmask, int64_t Kp, int64_t b_begin, int64_t b_count,
                    double *obj_out, double *alpha_out);

@@ -25,7 +25,7 @@ import numpy as np
 from . import _abi
 from ._abi import Context, PlsError  # noqa: F401
 
-__all__ = ["fit", "predict", "predict_resident", "PartLSFitResult", "Opt", "Alt", "BnB", "homogeneousCoords",
+__all__ = ["fit", "fit_path", "predict", "predict_resident", "PartLSFitResult", "Opt", "Alt", "BnB", "homogeneousCoords",
            "regularizeProblem", "Context", "PlsError", "default_context", "draw_alt_starts"]
 
 
@@ -171,6 +171,29 @@ def fit(alg, X, y, P, *, η=0.0, eta=None, nnlsalg="nnls", returnAllSolutions=Fa
         return model, None, SimpleNamespace(opt=r["opt"], best_restart=r["best_restart"], iters=r["iters"],
                                             all_obj=r["all_obj"], stats=r["stats"])
     raise TypeError(f"unknown algorithm {alg!r}")
+
+
+def fit_path(alg, X, y, P, etas, *, ctx=None, **flags):
+    """fit(Opt, X, y, P; η=η_l) for every η_l in `etas` (1..64 values, any order, duplicates allowed) on one resident
+    copy of the data: one Gram build, the orthant solves of all η in as few launches as the kernel choice allows, and
+    one pass over X for all winners (pls_opt_fit_path).  Returns a list with one entry per η, each what
+    fit(Opt, X, y, P; η=η_l) returns: (PartLSFitResult, None, report) with report.opt, report.b and the call's shared
+    stats.  Keyword flags: enumerate_intercept, no_recompute (as PLS_FLAG_*)."""
+    if not (alg is Opt or isinstance(alg, Opt)):
+        raise TypeError(f"fit_path supports Opt only, not {alg!r}")
+    unknown = set(flags) - {"enumerate_intercept", "no_recompute"}
+    if unknown:
+        raise TypeError(f"unknown keyword(s) {sorted(unknown)}")
+    fl = (_abi.PLS_FLAG_ENUMERATE_INTERCEPT if flags.get("enumerate_intercept") else 0) | \
+         (_abi.PLS_FLAG_NO_RECOMPUTE if flags.get("no_recompute") else 0)
+    c = ctx or default_context()
+    c.load(X, y, P)
+    res, stats = c.opt_fit_path(etas, flags=fl)
+    out = []
+    for r in res:
+        opt, model = _cleanup_result(r["opt"], r["alpha_raw"], r["b_best"], P)
+        out.append((model, None, SimpleNamespace(opt=opt, b=r["b_best"], stats=stats)))
+    return out
 
 
 def predict_resident(model, ctx, N):

@@ -79,11 +79,14 @@ lib.pls_get_stats.argtypes = [_vp, C.POINTER(PlsStats)]
 lib.pls_gram_scalars.argtypes = [_vp, _dp, _dp]
 lib.pls_bnb_lower_bounds.argtypes = [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int64, _dp, _dp]
 lib.pls_gram.argtypes = [_vp, _dp, C.c_int64, C.c_int64, _dp, _ip, C.c_int64, C.c_double, _dp, _dp, _dp]
+lib.pls_opt_fit_path.argtypes = [_vp, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, C.POINTER(PlsStats)]
+lib.pls_residual_partial_multi.argtypes = [_vp, _dp, C.c_int64, _dp]
 lib.pls_nnls_batch.argtypes = [_vp, _dp, _dp, C.c_double, C.c_int64, C.POINTER(C.c_uint64), C.c_int64,
                                C.c_int64, C.c_int64, _dp, _dp]
 for _n in ("pls_create", "pls_opt_fit", "pls_bnb_fit", "pls_bnb_fit_resident", "pls_alt_fit", "pls_alt_fit_resident", "pls_residual_partial_w", "pls_predict_resident", "pls_objective_finish_w", "pls_load", "pls_opt_fit_resident", "pls_gram_build", "pls_gram_raw",
            "pls_gram_finalize", "pls_opt_solve_range", "pls_opt_solve_pairs", "pls_opt_residual_partial", "pls_opt_objective_finish",
-           "pls_get_stats", "pls_gram_scalars", "pls_bnb_lower_bounds", "pls_gram", "pls_nnls_batch"):
+           "pls_get_stats", "pls_gram_scalars", "pls_bnb_lower_bounds", "pls_gram", "pls_nnls_batch", "pls_opt_fit_path",
+           "pls_residual_partial_multi"):
     getattr(lib, _n).restype = C.c_int
 
 
@@ -213,6 +216,16 @@ class Context:
         return dict(alpha_raw=alpha, b_best=b.value, opt=obj.value, objs=all_obj, alphas=all_alpha,
                     stats=st.as_dict())
 
+    def opt_fit_path(self, etas, flags=0):
+        """pls_opt_fit_path: fit(Opt) for every eta in `etas` (1..64 values) on the resident data set.  Returns one
+        dict per eta (alpha_raw, b_best, opt) and the call's shared stats."""
+        N, M, K = self._shape
+        e = np.ascontiguousarray(np.asarray(etas, dtype=np.float64).reshape(-1))
+        L = len(e)
+        alpha = np.zeros((L, M + 1)); b = np.zeros(L, dtype=np.int64); obj = np.zeros(L); st = PlsStats()
+        _check(lib.pls_opt_fit_path(self._h, _d(e), L, flags, _d(alpha), b.ctypes.data_as(_ip), _d(obj), C.byref(st)))
+        return [dict(alpha_raw=alpha[l], b_best=int(b[l]), opt=float(obj[l])) for l in range(L)], st.as_dict()
+
     def gram_build(self):
         _check(lib.pls_gram_build(self._h))
 
@@ -256,6 +269,12 @@ class Context:
         a = np.ascontiguousarray(w, dtype=np.float64); s = C.c_double()
         _check(lib.pls_residual_partial_w(self._h, _d(a), C.byref(s)))
         return s.value
+
+    def residual_partial_multi(self, W):
+        """pls_residual_partial_multi: the path's K4 pass for the rows of W (L x (M+1) signed weights, L <= 64)."""
+        a = np.ascontiguousarray(W, dtype=np.float64); L = a.shape[0]; out = np.zeros(L)
+        _check(lib.pls_residual_partial_multi(self._h, _d(a), L, _d(out)))
+        return out
 
     def predict_resident(self, w, N):
         """pls_predict_resident: X_resident @ w[:M] + w[M] for the N rows loaded on this context."""

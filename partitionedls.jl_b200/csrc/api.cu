@@ -65,7 +65,8 @@ void free_ws(pls_ctx *c) {
   SolveWs &ws = c->ws;
   cudaFree(ws.cta_obj); cudaFree(ws.cta_b); cudaFree(ws.cta_w); cudaFree(ws.hspill); cudaFree(ws.tab);
   cudaFree(ws.counters); cudaFree(ws.win); cudaFree(ws.all_obj); cudaFree(ws.all_alpha);
-  cudaFree(ws.resid_part); cudaFree(ws.alt_win); cudaFree(ws.yhat);
+  cudaFree(ws.resid_part); cudaFree(ws.resid_mpart); cudaFree(ws.alt_win); cudaFree(ws.yhat);
+  cudaFree(ws.path); cudaFree(ws.path_w);
   ws = SolveWs();
 }
 
@@ -121,9 +122,10 @@ void read_counters(pls_ctx *c, const unsigned long long *h) {
 // K2 + K3 over a range, winner record left in ws.win.  Caller holds the device.
 // pairs: [b_begin, b_begin + b_count) are sign patterns of the K user groups; the intercept sign is left free, so
 // every solve resolves the two reference orthants b and b + 2^K (the winner record carries the full b).
-int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs, K2Force force_variant) {
+int solve_range_dev(pls_ctx *c, const GramSys &g, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs,
+                    K2Force force_variant) {
   Problem &pb = c->pb;
-  if (!pb.gram_ready) { set_error("Gram matrix not built (call pls_gram_build / pls_gram_finalize)"); return PLS_EINVAL; }
+  if (g.G == pb.G && !pb.gram_ready) { set_error("Gram matrix not built (call pls_gram_build / pls_gram_finalize)"); return PLS_EINVAL; }
   if (pb.Kp > 40) { set_error("K = %d: 2^(K+1) orthants cannot be enumerated (limit K <= 39); use fit(BnB) or fit(Alt)", pb.K); return PLS_EINVAL; }
   if (pairs && (want_obj || want_alpha)) { set_error("per-orthant outputs need the full enumeration"); return PLS_EINVAL; }
   const int64_t total = (int64_t)1 << (pairs ? pb.Kp - 1 : pb.Kp);
@@ -133,7 +135,7 @@ int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj,
   PLS_CUDA_TRY(ensure_win(c->ws, record_len(pb.Mp)));
   if (c->ws.counters)
     PLS_CUDA_TRY(cudaMemsetAsync(c->ws.counters, 0, sizeof(unsigned long long) * CNT_BLOCK_LEN, c->stream));
-  rc = k2_solve_range(pb, pb.G, pb.ldg, pb.c, pb.scal, pb.gmask, pb.Mp, pb.Kp, c->ws, b_begin, b_count,
+  rc = k2_solve_range(pb, g.G, pb.ldg, g.c, g.scal, pb.gmask, pb.Mp, pb.Kp, c->ws, b_begin, b_count,
                       want_obj ? c->ws.all_obj : nullptr, want_alpha ? c->ws.all_alpha : nullptr,
                       c->sm_count, c->stream, &c->launches, pairs, force_variant,
                       c->h_gmask.size() == (size_t)pb.Mp ? c->h_gmask.data() : nullptr);
@@ -151,7 +153,7 @@ namespace {
 // checks saw; above 1e-13 max|c| its tableau was losing digits on this (ill-conditioned) problem, and the winner is
 // solved once more -- one orthant / pair, cold, by the one-level kernel, whose every iterate is checked against the
 // original system.  The new record replaces the old one in ws.win and h_pin; the counters of the main run are kept.
-int polish_if_drifted(pls_ctx *c, bool pairs, bool *did) {
+int polish_if_drifted(pls_ctx *c, const GramSys &g, bool pairs, bool *did) {
   *did = false;
   const int Mp = c->pb.Mp;
   unsigned long long *cnt = c->pin_counters();
@@ -160,7 +162,7 @@ int polish_if_drifted(pls_ctx *c, bool pairs, bool *did) {
   if (bb < 0 || c->pin_obj() != c->pin_obj()) return PLS_OK;
   std::vector<unsigned long long> keep(cnt, cnt + CNT_BLOCK_LEN);
   const int64_t idx = pairs ? (int64_t)(bb & (((long long)1 << (c->pb.Kp - 1)) - 1)) : (int64_t)bb;
-  int rc = solve_range_dev(c, idx, 1, false, false, pairs, K2_FORCE_V3);
+  int rc = solve_range_dev(c, g, idx, 1, false, false, pairs, K2_FORCE_V3);
   if (rc) return rc;
   cudaStream_t st = c->stream;
   PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, st));
@@ -178,7 +180,8 @@ int polish_if_drifted(pls_ctx *c, bool pairs, bool *did) {
 // variable per step behind a pivot test, as Lawson-Hanson, which never forms such sets) -- literally enumerated, so
 // a paired range becomes its two halves b and b + 2^K.  Leaves the winner in ws.win / h_pin, per-orthant outputs
 // (literal ranges only) in the device staging buffers, and the first run's counters (+1 rebuild) in h_pin.
-int fallback_if_stalled(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs, bool *did) {
+int fallback_if_stalled(pls_ctx *c, const GramSys &g, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs,
+                        bool *did) {
   *did = false;
   const int Mp = c->pb.Mp;
   unsigned long long *cnt = c->pin_counters();
@@ -189,7 +192,7 @@ int fallback_if_stalled(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_
   const int n_half = pairs ? 2 : 1;
   for (int h = 0; h < n_half; ++h) {
     const int64_t b0 = b_begin + (h ? ((int64_t)1 << (c->pb.Kp - 1)) : 0);
-    int rc = solve_range_dev(c, b0, b_count, want_obj, want_alpha, false, K2_FORCE_V1);
+    int rc = solve_range_dev(c, g, b0, b_count, want_obj, want_alpha, false, K2_FORCE_V1);
     if (rc) return rc;
     PLS_CUDA_TRY(cudaMemcpyAsync(c->h_pin, c->ws.win, sizeof(double) * record_len(Mp), cudaMemcpyDeviceToHost, st));
     PLS_CUDA_TRY(cudaMemcpyAsync(cnt, c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
@@ -198,7 +201,7 @@ int fallback_if_stalled(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_
     bool better = best.empty();
     if (!better) {
       double yy = 0.0;
-      PLS_CUDA_TRY(cudaMemcpy(&yy, c->pb.scal, sizeof(double), cudaMemcpyDeviceToHost));
+      PLS_CUDA_TRY(cudaMemcpy(&yy, g.scal, sizeof(double), cudaMemcpyDeviceToHost));
       better = opt_better(c->pin_obj(), c->pin_b(), best[Mp], record_b(best.data(), Mp), PLS_TIE_REL * yy);
     }
     if (better) best.assign(c->h_pin, c->h_pin + record_len(Mp));
@@ -230,7 +233,8 @@ int launch_total(const pls_ctx *c) {
 
 int k2_range_enqueue(pls_ctx *c, const K2Range &r) {
   PLS_CUDA_TRY(cudaEventRecord(c->ev[r.ev], c->stream));
-  const int rc = solve_range_dev(c, r.b_begin, r.b_count, r.all_obj != nullptr, r.all_alpha != nullptr, r.pairs);
+  const int rc = solve_range_dev(c, r.gram.G ? r.gram : ctx_gram(c), r.b_begin, r.b_count, r.all_obj != nullptr,
+                                 r.all_alpha != nullptr, r.pairs);
   if (rc) return rc;
   PLS_CUDA_TRY(cudaEventRecord(c->ev[r.ev + 1], c->stream));
   return PLS_OK;
@@ -247,14 +251,15 @@ int k2_range_settle(pls_ctx *c, K2Range &r) {
   float ms = 0.f;
   cudaEventElapsedTime(&ms, c->ev[r.ev], c->ev[r.ev + 1]);
   c->stats.ms_nnls = ms;
-  int rc = fallback_if_stalled(c, r.b_begin, r.b_count, r.all_obj != nullptr, r.all_alpha != nullptr, r.pairs, &r.fell);
+  const GramSys g = r.gram.G ? r.gram : ctx_gram(c);
+  int rc = fallback_if_stalled(c, g, r.b_begin, r.b_count, r.all_obj != nullptr, r.all_alpha != nullptr, r.pairs, &r.fell);
   if (rc) return rc;
   if (r.fell && (r.all_obj || r.all_alpha)) {
     rc = copy_outputs(c, r);
     if (rc) return rc;
     PLS_CUDA_TRY(cudaStreamSynchronize(c->stream));
   }
-  rc = polish_if_drifted(c, r.pairs, &r.polished);
+  rc = polish_if_drifted(c, g, r.pairs, &r.polished);
   if (rc) return rc;
   const unsigned long long *cnt = c->pin_counters();
   read_counters(c, cnt);
@@ -294,10 +299,10 @@ bool use_pairs(const pls_ctx *c, uint32_t flags, bool per_orthant_outputs) {
   return !per_orthant_outputs && !(flags & PLS_FLAG_ENUMERATE_INTERCEPT) && c->pb.Mp <= 1024 && c->pb.Kp >= 2;
 }
 
-double eta_term(const pls_ctx *c, const double *alpha_raw, int64_t b) {
+double eta_term(const pls_ctx *c, double eta, const double *alpha_raw, int64_t b) {
   // the eta rows of regularizeProblem (PartitionedLS.jl:115-118): eta * sum_k (sum_{m in k} w_m)^2
   const Problem &pb = c->pb;
-  if (pb.eta == 0.0) return 0.0;
+  if (eta == 0.0) return 0.0;
   double tot = 0.0;
   for (int k = 0; k < pb.Kp; ++k) {
     double s = 0.0;
@@ -305,7 +310,7 @@ double eta_term(const pls_ctx *c, const double *alpha_raw, int64_t b) {
       if (c->h_gmask[m] >> k & 1ull) s += (double)host_d(c->h_gmask, m, b) * alpha_raw[m];
     tot += s * s;
   }
-  return pb.eta * tot;
+  return eta * tot;
 }
 
 // the eta rows for signed weights w (BnB / Alt): eta * sum_k (sum_{m in k} w_m)^2
@@ -336,6 +341,156 @@ int residual_partial_w(pls_ctx *c, const double *w, double *ssq_out) {
   PLS_CUDA_TRY(cudaStreamSynchronize(st));
   *ssq_out = *c->pin_ssq();
   return PLS_OK;
+}
+
+namespace {
+
+// The counters one K2 range left in c->stats, added to a path's totals
+void add_counters(pls_stats &a, const pls_stats &s) {
+  a.pivots += s.pivots; a.grad_evals += s.grad_evals; a.sum_p += s.sum_p; a.sum_p2 += s.sum_p2;
+  a.bpp_iters += s.bpp_iters; a.spills += s.spills; a.rebuilds += s.rebuilds; a.blocked += s.blocked;
+  a.nnls_flops += s.nnls_flops; a.nnls_l2_bytes += s.nnls_l2_bytes;
+  a.k2_max_drift = std::fmax(a.k2_max_drift, s.k2_max_drift);
+}
+
+// Layout of ws.path for L problems: etas [64] | failure counts [64] | c [ldg] | scal_l [4 L] | G_l [L][gstride]
+struct PathWs { double *etas, *c, *scal, *G; unsigned long long *noconv; size_t gstride; };
+
+int path_ws(pls_ctx *c, int L, PathWs *p) {
+  const Problem &pb = c->pb;
+  // + 32 doubles past G_l, as pb.G has: K2's gradient threads may read whole 8/16-row units beyond the last column, and
+  // (as with pb.G, which is never initialised there) what they read there is not used
+  const size_t gstride = (size_t)round_up((int64_t)pb.ldg * pb.Mp + 32, 32);
+  const size_t head = 64 + 64 + (size_t)pb.ldg + 4 * 64;
+  const size_t bytes = sizeof(double) * (head + (size_t)L * gstride);
+  SolveWs &ws = c->ws;
+  if (ws.path_bytes < bytes) {
+    cudaFree(ws.path); ws.path = nullptr; ws.path_bytes = 0;
+    PLS_CUDA_TRY(cudaMalloc(&ws.path, bytes));
+    ws.path_bytes = bytes;
+  }
+  p->etas = ws.path;
+  p->noconv = reinterpret_cast<unsigned long long *>(ws.path + 64);
+  p->c = ws.path + 128;
+  p->scal = p->c + pb.ldg;
+  p->G = p->scal + 4 * 64;
+  p->gstride = gstride;
+  return PLS_OK;
+}
+
+}  // namespace
+
+int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool build_S, double *records) {
+  Problem &pb = c->pb;
+  cudaStream_t st = c->stream;
+  const int Mp = pb.Mp, rl = record_len(Mp);
+  PathWs p;
+  int rc = path_ws(c, L, &p);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaMemcpyAsync(p.etas, etas, sizeof(double) * L, cudaMemcpyHostToDevice, st));
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  if (build_S) { rc = k1_gram_build(pb, st, &c->launches); if (rc) return rc; }
+  rc = k1_gram_finalize_path(pb, p.etas, L, p.G, p.gstride, p.c, p.scal, st, &c->launches);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
+  std::vector<double> scal((size_t)4 * L);
+  PLS_CUDA_TRY(cudaMemcpyAsync(scal.data(), p.scal, sizeof(double) * 4 * L, cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaStreamSynchronize(st));
+  for (int l = 0; l < L; ++l)
+    if (scal[4 * l + 3] != 0.0) { set_error("non-finite values in X or y, or in the Gram matrix of eta = %g", etas[l]); return PLS_ENUMERIC; }
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]);
+  const double t0 = now_ms();
+
+  const bool pairs = use_pairs(c, flags, false);
+  const int64_t count = (int64_t)1 << (pairs ? pb.Kp - 1 : pb.Kp);
+  auto sys = [&](int l) { return GramSys{p.G + (size_t)l * p.gstride, p.c, p.scal + 4 * l}; };
+  pls_stats acc;
+  memset(&acc, 0, sizeof(acc));
+  // one eta alone, exactly as its resident fit solves it: K2 + K3, the single-pivot fallback, the polish
+  auto solve_one = [&](int l) -> int {
+    K2Range r;
+    r.b_count = count; r.pairs = pairs; r.gram = sys(l);
+    const int r2 = k2_range_solve(c, r);
+    if (r2) return r2;
+    memcpy(records + (size_t)l * rl, c->h_pin, sizeof(double) * rl);
+    add_counters(acc, c->stats);
+    return PLS_OK;
+  };
+  K2Choice ch;
+  rc = k2_choose(Mp, pb.Kp, 0, count, false, c->sm_count, pairs, K2_DISPATCH,
+                 c->h_gmask.size() == (size_t)Mp ? c->h_gmask.data() : nullptr, &ch);
+  if (rc) return rc;
+  int variant = ch.variant, threads = 0, occ = 0, grid = 0;
+  if (ch.variant == 3) {
+    // every eta in one launch of the one-level kernel, each on its own G_l; an eta with a failed solve is solved again alone
+    PLS_CUDA_TRY(ensure_counters(c->ws, true, st));
+    PLS_CUDA_TRY(cudaMemsetAsync(p.noconv, 0, sizeof(unsigned long long) * L, st));
+    rc = k2_solve_range(pb, p.G, pb.ldg, p.c, p.scal, pb.gmask, Mp, pb.Kp, c->ws, 0, count, nullptr, nullptr, c->sm_count,
+                        st, &c->launches, pairs, K2_DISPATCH, c->h_gmask.data(), L, p.gstride, p.noconv);
+    if (rc) return rc;
+    threads = c->ws.last_threads; occ = c->ws.last_occ; grid = c->ws.last_grid;
+    std::vector<unsigned long long> nc(L), cnt(CNT_BLOCK_LEN);
+    PLS_CUDA_TRY(cudaMemcpyAsync(records, c->ws.win, sizeof(double) * rl * L, cudaMemcpyDeviceToHost, st));
+    PLS_CUDA_TRY(cudaMemcpyAsync(nc.data(), p.noconv, sizeof(unsigned long long) * L, cudaMemcpyDeviceToHost, st));
+    PLS_CUDA_TRY(cudaMemcpyAsync(cnt.data(), c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
+    PLS_CUDA_TRY(cudaStreamSynchronize(st));
+    read_counters(c, cnt.data());
+    add_counters(acc, c->stats);
+    for (int l = 0; l < L; ++l)
+      if (nc[l]) { rc = solve_one(l); if (rc) return rc; }
+  } else {
+    for (int l = 0; l < L; ++l) {
+      rc = solve_one(l);
+      if (rc) return rc;
+      variant = c->stats.k2_variant; threads = (int)c->stats.k2_threads; occ = (int)c->stats.k2_ctas_per_sm; grid = (int)c->stats.k2_grid;
+    }
+  }
+  pls_stats &s = c->stats;
+  s = acc;                                       // (fit_start cleared the rest; the upload time of a path is 0)
+  s.k2_variant = variant; s.k2_threads = threads; s.k2_ctas_per_sm = occ; s.k2_grid = grid;
+  s.ms_gram = ms;
+  s.ms_nnls = now_ms() - t0;
+  return PLS_OK;
+}
+
+// K4 on this device's rows for L <= 64 signed weight vectors W[l * Mp + m] (host): ssq[l]; the pass is timed into
+// c->stats.ms_recompute
+int residual_partial_multi(pls_ctx *c, const double *W, int L, double *ssq) {
+  int rc = check_ctx(c);
+  if (rc) return rc;
+  const Problem &pb = c->pb;
+  cudaStream_t st = c->stream;
+  SolveWs &ws = c->ws;
+  const size_t bytes = sizeof(double) * (64 * (size_t)pb.Mp + 64);
+  if (ws.path_w_bytes < bytes) {
+    cudaFree(ws.path_w); ws.path_w = nullptr; ws.path_w_bytes = 0;
+    PLS_CUDA_TRY(cudaMalloc(&ws.path_w, bytes));
+    ws.path_w_bytes = bytes;
+  }
+  double *d_ssq = ws.path_w + 64 * (size_t)pb.Mp;
+  PLS_CUDA_TRY(cudaMemcpyAsync(ws.path_w, W, sizeof(double) * (size_t)L * pb.Mp, cudaMemcpyHostToDevice, st));
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[4], st));
+  rc = k4_residual_multi(pb, ws, ws.path_w, L, d_ssq, c->sm_count, st, &c->launches);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[5], st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(ssq, d_ssq, sizeof(double) * L, cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaStreamSynchronize(st));
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]);
+  c->stats.ms_recompute = ms;
+  return PLS_OK;
+}
+
+int path_ssq_dev(pls_ctx *c, const double *records, int L, double *ssq) {
+  const int Mp = c->pb.Mp, rl = record_len(Mp);
+  std::vector<double> W((size_t)L * Mp);
+  for (int l = 0; l < L; ++l) {
+    const double *rec = records + (size_t)l * rl;
+    const long long b = record_b(rec, Mp);
+    for (int m = 0; m < Mp; ++m) W[(size_t)l * Mp + m] = (double)host_d(c->h_gmask, m, b) * rec[m];
+  }
+  return residual_partial_multi(c, W.data(), L, ssq);
 }
 
 }  // namespace pls
@@ -640,7 +795,7 @@ int pls_opt_residual_partial(pls_ctx *c, const double *alpha_raw, int64_t b, dou
 
 int pls_opt_objective_finish(pls_ctx *c, const double *alpha_raw, int64_t b, double ssq_total, double *obj_out) {
   if (!c || !alpha_raw || !obj_out) { set_error("null pointer"); return PLS_EINVAL; }
-  *obj_out = std::sqrt(ssq_total + eta_term(c, alpha_raw, b));
+  *obj_out = std::sqrt(ssq_total + eta_term(c, c->pb.eta, alpha_raw, b));
   return PLS_OK;
 }
 
@@ -648,6 +803,13 @@ int pls_residual_partial_w(pls_ctx *c, const double *w, double *ssq_out) {
   if (c && !c->subs.empty()) { set_error("stage-wise entry points need a one-GPU context"); return PLS_EUNSUPPORTED; }
   if (!c || !c->pb.loaded || !w || !ssq_out) { set_error("no data set loaded or null pointer"); return PLS_EINVAL; }
   return residual_partial_w(c, w, ssq_out);
+}
+
+int pls_residual_partial_multi(pls_ctx *c, const double *W, int64_t L, double *ssq_out) {
+  if (c && !c->subs.empty()) { set_error("test hooks need a one-GPU context"); return PLS_EUNSUPPORTED; }
+  if (!c || !c->pb.loaded || !W || !ssq_out) { set_error("no data set loaded or null pointer"); return PLS_EINVAL; }
+  if (L < 1 || L > 64) { set_error("L = %lld weight vectors (1..64)", (long long)L); return PLS_EINVAL; }
+  return residual_partial_multi(c, W, (int)L, ssq_out);
 }
 
 // K7 on one device: yhat[0..N) of this context's resident rows (host pointer)
@@ -739,7 +901,7 @@ int pls_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_t 
   const long long bb = c->pin_b();
   *b_best = bb;
   double obj = c->pin_obj();
-  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term(c, alpha_raw, bb));
+  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term(c, pb.eta, alpha_raw, bb));
   *obj_best = obj;
 
   pls_stats &s = c->stats;
@@ -750,6 +912,50 @@ int pls_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_t 
   s.orthants = total; s.nnls_problems = r.b_count;
   fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
+  return PLS_OK;
+}
+
+int pls_opt_fit_path(pls_ctx *c, const double *etas, int64_t L, uint32_t flags, double *alpha_raw, int64_t *b_best,
+                     double *obj_best, pls_stats *stats) {
+  if (!c) { set_error("null context"); return PLS_EINVAL; }
+  if (!c->pb.loaded) { set_error("no data set loaded"); return PLS_EINVAL; }
+  if (!etas || !alpha_raw || !b_best || !obj_best) { set_error("null pointer"); return PLS_EINVAL; }
+  if (L < 1 || L > 64) { set_error("L = %lld eta values (1..64)", (long long)L); return PLS_EINVAL; }
+  for (int64_t l = 0; l < L; ++l)
+    if (!(etas[l] >= 0.0) || !std::isfinite(etas[l])) { set_error("eta[%lld] must be finite and >= 0", (long long)l); return PLS_EINVAL; }
+  const int Mp = c->pb.Mp, Kp = c->pb.Kp, rl = record_len(Mp);
+  if (Mp > 1024) { set_error("M' = %d: an eta path needs M' <= 1024 (fit each eta on its own)", Mp); return PLS_EUNSUPPORTED; }
+  if (Kp > 40) { set_error("K = %d: 2^(K+1) orthants cannot be enumerated (limit K <= 39); use fit(BnB) or fit(Alt)", c->pb.K); return PLS_EINVAL; }
+  const bool recompute = !(flags & PLS_FLAG_NO_RECOMPUTE);
+  std::vector<double> rec((size_t)L * rl), ssq((size_t)L, 0.0);
+  const FitMark fm = fit_start(c);
+  int rc;
+  if (!c->subs.empty()) {
+    rc = multi_opt_fit_path(c, etas, (int)L, flags, rec.data(), ssq.data());
+    if (rc) return rc;
+  } else {
+    rc = check_ctx(c);
+    if (rc) return rc;
+    rc = path_solve_dev(c, etas, (int)L, flags, !c->pb.gram_ready, rec.data());
+    if (rc) return rc;
+    if (recompute) { rc = path_ssq_dev(c, rec.data(), (int)L, ssq.data()); if (rc) return rc; }
+  }
+  bool nan = false;
+  for (int64_t l = 0; l < L; ++l) {
+    const double *r = rec.data() + (size_t)l * rl;
+    const long long bb = record_b(r, Mp);
+    memcpy(alpha_raw + (size_t)l * Mp, r, sizeof(double) * Mp);
+    b_best[l] = bb;
+    double obj = r[Mp];
+    if (recompute && obj == obj) obj = std::sqrt(ssq[l] + eta_term(c, etas[l], r, bb));
+    obj_best[l] = obj;
+    nan |= obj != obj;
+  }
+  pls_stats &s = c->stats;
+  const int64_t count = (int64_t)1 << (use_pairs(c, flags, false) ? Kp - 1 : Kp);
+  s.orthants = L << Kp; s.nnls_problems = L * count;
+  fit_finish(c, fm, stats);
+  if (nan) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
   return PLS_OK;
 }
 
@@ -993,7 +1199,7 @@ int pls_nnls_batch(pls_ctx *c, const double *G, const double *cv, double yy, int
   if (c->h_pin) { cudaFreeHost(c->h_pin); c->h_pin = nullptr; }
   PLS_CUDA_TRY(cudaMallocHost(&c->h_pin, sizeof(double) * pin_len(Mp)));
   pb.gram_ready = true;
-  rc = solve_range_dev(c, b_begin, b_count, obj_out != nullptr, alpha_out != nullptr);
+  rc = solve_range_dev(c, ctx_gram(c), b_begin, b_count, obj_out != nullptr, alpha_out != nullptr);
   if (rc) return rc;
   cudaStream_t st = c->stream;
   if (obj_out) PLS_CUDA_TRY(cudaMemcpyAsync(obj_out, c->ws.all_obj, sizeof(double) * (size_t)b_count, cudaMemcpyDeviceToHost, st));

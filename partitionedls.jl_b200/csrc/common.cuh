@@ -117,6 +117,12 @@ struct SolveWs {
   size_t yhat_n = 0;
   double *resid_part = nullptr;   // K4 block partials
   int resid_blocks = 0;
+  double *resid_mpart = nullptr;  // K4 over several weight vectors: [blocks][64] partials
+  int resid_mblocks = 0;
+  double *path = nullptr;         // eta path (api.cu): etas, per-problem failure counts, c, scal_l and G_l of L problems
+  size_t path_bytes = 0;
+  double *path_w = nullptr;       // eta path: the winners' signed weights [64][Mp] and their K4 sums [64]
+  size_t path_w_bytes = 0;
   int win_len = 0;                // doubles allocated at win
   // what the last k2_solve_range launched (reported through pls_stats.k2_*)
   int last_variant = 0, last_threads = 0, last_occ = 0, last_grid = 0;
@@ -173,18 +179,31 @@ struct K2Args {
   double *cta_obj; long long *cta_b; double *cta_w;
   double *all_obj; double *all_alpha;   // nullable, indexed by (b - b_begin)
   unsigned long long *counters;
+  // v3 only: n_prob problems of one shape in one launch (an eta path).  Chain i belongs to problem i / n_chains, which
+  // reads the Gram matrix G + problem * gstride; per-CTA winners are kept per (problem, CTA) at problem * gridDim.x +
+  // blockIdx.x, and failed solves are also counted per problem in noconv[problem] (null with one problem).
+  int n_prob = 1;
+  size_t gstride = 0;
+  unsigned long long *noconv = nullptr;
 };
 
 // ---- kernel launchers (defined in gram.cu / nnls.cu / resid.cu) -----------------------------
 int k1_gram_build(Problem &pb, cudaStream_t st, int *launches);
 int k1_gram_finalize(Problem &pb, cudaStream_t st, int *launches);
+// G_l = S + etas[l] |groups(i) & groups(j)| for l < L (device etas) into G + l * gstride, scal_l into scal + 4 l, and
+// the shared c -- each G_l bitwise what k1_gram_finalize gives for eta = etas[l].  pb's own G, c, scal are untouched.
+int k1_gram_finalize_path(const Problem &pb, const double *etas, int L, double *G, size_t gstride, double *c,
+                          double *scal, cudaStream_t st, int *launches);
 // force_variant of k2_solve_range: the kernel of a re-solve, in place of the dispatch rules
 enum K2Force { K2_DISPATCH = 0, K2_FORCE_V1 = 1, K2_FORCE_V3 = 3 };
+// n_prob > 1 (v3 only, k2_choose must pick 3): n_prob ranges of one shape, problem l on G + l * g_stride; winner
+// record l at ws.win + l * (Mp + 2), failed solves of problem l counted in noconv[l].
 int k2_solve_range(const Problem &pb, const double *G, int ldg, const double *c, const double *scal,
                    const uint64_t *gmask, int Mp, int Kp, SolveWs &ws, int64_t b_begin,
                    int64_t b_count, double *d_all_obj, double *d_all_alpha, int sm_count,
                    cudaStream_t st, int *launches, bool free_top = false, int force_variant = K2_DISPATCH,
-                   const uint64_t *h_gmask = nullptr);
+                   const uint64_t *h_gmask = nullptr, int n_prob = 1, size_t g_stride = 0,
+                   unsigned long long *noconv = nullptr);
 // K2 variants: v1 = rank-1 updates on a dense inverse with a global-memory spill path (any M').
 // v3 = block pivoting on FP64 tensor cores with the inverse split between shared memory and an L2-resident global
 // slice, any thread count, M' <= 1024 (nnls3.cu)
@@ -199,6 +218,10 @@ int k2v4_launch(const K2Args &A, const K4Plan &pl, int grid, cudaStream_t st);
 struct K5Plan { int variant, T, NR, ld1, occ, low_groups, verify_every, cold_fused; size_t smem, tabstride; };
 int k2v5_plan(int Mp, int n_bits, const uint64_t *h_gmask, K5Plan *pl);
 int k2v5_launch(const K2Args &A, const K5Plan &pl, int grid, cudaStream_t st);
+// The kernel k2_solve_range runs for a range, and its plan (the dispatch rules of nnls.cu)
+struct K2Choice { int variant = 0, cap = 0, occ = 1; size_t smem = 0; K3Plan p3; K4Plan p4; K5Plan p5; };
+int k2_choose(int Mp, int Kp, int64_t b_begin, int64_t b_count, bool outputs, int sm_count, bool free_top,
+              int force_variant, const uint64_t *h_gmask, K2Choice *ch);
 // K5: branch and bound with batched frontier expansion (bnb.cu); winner left in ws.win
 struct BnbReport { long long visited, waves, max_open, pool_slots; double mu; bool complete, has_leaf; };
 // Multi-GPU sharding of the search (multi.cu).  roots: the subtrees this call searches, each given by the
@@ -223,6 +246,9 @@ int k6_alt_run(const Problem &pb, SolveWs &ws, const std::vector<uint64_t> &h_gm
                double **d_win_out);
 int k4_residual(const Problem &pb, SolveWs &ws, const double *d_w, double *d_ssq, int sm_count,
                 cudaStream_t st, int *launches);
+// K4 for L <= 64 signed weight vectors W[l * Mp + m] in one pass over Z: d_ssq[l] = sum_rows (Z[row,:] . w_l - y)^2
+int k4_residual_multi(const Problem &pb, SolveWs &ws, const double *d_W, int L, double *d_ssq, int sm_count,
+                      cudaStream_t st, int *launches);
 int k7_predict(const Problem &pb, const double *d_w, double *d_yhat, int sm_count, cudaStream_t st, int *launches);
 
 }  // namespace pls

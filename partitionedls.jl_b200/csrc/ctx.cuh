@@ -51,11 +51,15 @@ struct pls_ctx {
 };
 
 namespace pls {
+// A finalised Gram system on one device: G (leading dimension pb.ldg), c and scal = {yy, max|c|, ...}.  A fit solves
+// the context's own (pb.G, pb.c, pb.scal); an eta path solves one per eta from its own workspace.
+struct GramSys { const double *G = nullptr, *c = nullptr, *scal = nullptr; };
+static inline GramSys ctx_gram(const pls_ctx *c) { return GramSys{c->pb.G, c->pb.c, c->pb.scal}; }
 int check_ctx(pls_ctx *c);
 int host_d(const std::vector<uint64_t> &gm, int m, int64_t b);
 void read_counters(pls_ctx *c, const unsigned long long *h);
-int solve_range_dev(pls_ctx *c, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha, bool pairs = false,
-                    K2Force force_variant = K2_DISPATCH);
+int solve_range_dev(pls_ctx *c, const GramSys &g, int64_t b_begin, int64_t b_count, bool want_obj, bool want_alpha,
+                    bool pairs = false, K2Force force_variant = K2_DISPATCH);
 // One K2 range of a fit or a stage-wise call, in three parts so that a caller can put its own work between them:
 //   k2_range_enqueue  K2 + K3 between c->ev[ev] and c->ev[ev + 1];
 //   k2_range_copy     D2H copies of the winner record, the counter block (h_pin) and the per-orthant outputs;
@@ -68,6 +72,7 @@ struct K2Range {
   double *all_obj = nullptr, *all_alpha = nullptr;   // host destinations (literal ranges only), or null
   int ev = 2;
   bool fell = false, polished = false;               // set by k2_range_settle: the fallback ran / the winner was polished
+  GramSys gram;                                      // the system to solve; null G: the context's own
 };
 int k2_range_enqueue(pls_ctx *c, const K2Range &r);
 int k2_range_copy(pls_ctx *c, const K2Range &r);
@@ -79,10 +84,16 @@ struct FitMark { double t0; int launches0; };
 FitMark fit_start(pls_ctx *c);
 void fit_finish(pls_ctx *c, const FitMark &m, pls_stats *out);
 bool use_pairs(const pls_ctx *c, uint32_t flags, bool per_orthant_outputs);
-double eta_term(const pls_ctx *c, const double *alpha_raw, int64_t b);
+double eta_term(const pls_ctx *c, double eta, const double *alpha_raw, int64_t b);
 double eta_term_w(const pls_ctx *c, const double *w);
 int residual_partial_w(pls_ctx *c, const double *w, double *ssq_out);
 double now_ms();
+// The eta path on one device (api.cu): the winner records (record_len(M') doubles each) of etas[0..L) on the S this
+// context holds (built first unless build_S is false), and the counters of the call added into c->stats.
+int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool build_S, double *records);
+// K4 of L winner records on this device's rows: ssq[l] = sum_rows (Z[row,:] . w_l - y)^2, w_l = d(b_l) .* alpha_l
+int path_ssq_dev(pls_ctx *c, const double *records, int L, double *ssq);
+int residual_partial_multi(pls_ctx *c, const double *W, int L, double *ssq);
 // multi.cu
 int multi_create(pls_ctx *c, const int *device_ids, int n_dev);
 int multi_predict(pls_ctx *c, const double *w, double *yhat, int (*predict_dev)(pls_ctx *, const double *, double *));
@@ -91,6 +102,8 @@ int multi_load(pls_ctx *c, const double *X, int64_t N, int64_t ldx, int64_t M, c
                int64_t K, double eta);
 int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_t *b_best, double *obj_best,
                            double *all_obj, double *all_alpha, pls_stats *stats);
+// (c->stats: the counters summed over the devices, the longest stage times)
+int multi_opt_fit_path(pls_ctx *c, const double *etas, int L, uint32_t flags, double *records, double *ssq);
 int multi_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, double *obj_out, int64_t *nopen, pls_stats *stats);
 int multi_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps, int64_t T, uint32_t flags,
                            double *alpha, double *beta, double *obj_out, int64_t *best_restart, int64_t *iters,

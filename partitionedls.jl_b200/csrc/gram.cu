@@ -341,13 +341,12 @@ __global__ void k1_reduce(const double *__restrict__ part, int n_tiles, int n_ch
   S[idx] = s;
 }
 
-// G = S (mirrored) + eta * |groups(i) & groups(j)|;  c = S[y row];
+// G = S (mirrored) + eta * |groups(i) & groups(j)|;  c = S[y row] (when c is not null);
 // scal = {yy, max|c|, max diag, non-finite flag} (scal[1..3] zeroed before launch; max via
 // atomicMax on the bit pattern, valid for non-negative doubles)
-__global__ void k1_finalize(const double *__restrict__ S, int zc, int Mp, double eta,
-                            const uint64_t *__restrict__ gmask, double *__restrict__ G, int ldg,
-                            double *__restrict__ c, double *__restrict__ scal) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+__device__ __forceinline__ void finalize_entry(long long idx, const double *__restrict__ S, int zc, int Mp, double eta,
+                                               const uint64_t *__restrict__ gmask, double *__restrict__ G, int ldg,
+                                               double *__restrict__ c, double *__restrict__ scal) {
   double mc = 0.0, md = 0.0;
   int bad = 0;
   if (idx < (long long)ldg * Mp) {
@@ -362,7 +361,7 @@ __global__ void k1_finalize(const double *__restrict__ S, int zc, int Mp, double
       if (i == j) md = fabs(g);
       if (j == 0) {
         const double ci = S[(size_t)i * zc + Mp];     // row index of y in Z'Z is Mp = M+1
-        c[i] = ci;
+        if (c) c[i] = ci;
         mc = fabs(ci);
         if (!isfinite(ci)) bad = 1;
       }
@@ -384,6 +383,21 @@ __global__ void k1_finalize(const double *__restrict__ S, int zc, int Mp, double
     if (md > 0.0 && isfinite(md)) atomicMax(reinterpret_cast<unsigned long long *>(scal + 2), (unsigned long long)__double_as_longlong(md));
     if (bad) atomicMax(reinterpret_cast<unsigned long long *>(scal + 3), (unsigned long long)__double_as_longlong(1.0));
   }
+}
+
+__global__ void k1_finalize(const double *__restrict__ S, int zc, int Mp, double eta,
+                            const uint64_t *__restrict__ gmask, double *__restrict__ G, int ldg,
+                            double *__restrict__ c, double *__restrict__ scal) {
+  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, S, zc, Mp, eta, gmask, G, ldg, c, scal);
+}
+
+// The eta path: blockIdx.y = l builds G_l and scal_l with etas[l]; c (shared by all l) is written by l = 0.
+__global__ void k1_finalize_path(const double *__restrict__ S, int zc, int Mp, const double *__restrict__ etas,
+                                 const uint64_t *__restrict__ gmask, double *__restrict__ G, size_t gstride, int ldg,
+                                 double *__restrict__ c, double *__restrict__ scal) {
+  const int l = blockIdx.y;
+  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, S, zc, Mp, etas[l], gmask, G + (size_t)l * gstride,
+                 ldg, l == 0 ? c : nullptr, scal + 4 * l);
 }
 
 }  // namespace
@@ -445,6 +459,18 @@ int k1_gram_finalize(Problem &pb, cudaStream_t st, int *launches) {
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   pb.gram_ready = true;
+  return PLS_OK;
+}
+
+int k1_gram_finalize_path(const Problem &pb, const double *etas, int L, double *G, size_t gstride, double *c,
+                          double *scal, cudaStream_t st, int *launches) {
+  NvtxRange nvtx("pls:K1 gram finalize (eta path)");
+  const long long tot = (long long)pb.ldg * pb.Mp;
+  PLS_CUDA_TRY(cudaMemsetAsync(scal, 0, sizeof(double) * 4 * L, st));
+  k1_finalize_path<<<dim3((unsigned)((tot + 255) / 256), (unsigned)L), 256, 0, st>>>(pb.S, pb.zcols, pb.Mp, etas, pb.gmask,
+                                                                                    G, gstride, pb.ldg, c, scal);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
   return PLS_OK;
 }
 

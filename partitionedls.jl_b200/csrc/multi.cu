@@ -281,7 +281,7 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
     if (rc) return rc;
     double tot = 0.0;
     for (int g = 0; g < G; ++g) tot += ssq[g];
-    obj = std::sqrt(tot + eta_term(c, alpha_raw, wb));
+    obj = std::sqrt(tot + eta_term(c, c->pb.eta, alpha_raw, wb));
   }
   *obj_best = obj;
   pls_stats &s = c->stats;
@@ -291,6 +291,49 @@ int multi_opt_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_raw, int64_
   s.orthants = (int64_t)1 << Kp; s.nnls_problems = total;
   fit_finish(c, fm, stats);
   if (obj != obj) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
+  return PLS_OK;
+}
+
+// The eta path over several devices: the raw Gram sums are built and exchanged as for a fit (every device then holds
+// the same S), the eta values are dealt round-robin (eta l to device l % G), and each device finalises, solves and
+// selects the winners of its share.  Every device then evaluates ALL L winners on its own rows in one K4 pass; the
+// partial sums are added in device order.  An eta's winner does not depend on which device solved it.
+int multi_opt_fit_path(pls_ctx *c, const double *etas, int L, uint32_t flags, double *records, double *ssq) {
+  const int G = (int)c->subs.size();
+  const int rl = record_len(c->pb.Mp);
+  for (pls_ctx *s : c->subs) memset(&s->stats, 0, sizeof(s->stats));
+  const double tg0 = now_ms();
+  if (!c->subs[0]->pb.gram_ready) { const int rc = multi_gram(c); if (rc) return rc; }
+  const double tg1 = now_ms();
+  std::vector<std::vector<double>> share_eta(G), share_rec(G);
+  for (int l = 0; l < L; ++l) share_eta[l % G].push_back(etas[l]);
+  int rc = par_for(c, [&](int g, pls_ctx *s) -> int {
+    const int n = (int)share_eta[g].size();
+    if (!n) return PLS_OK;
+    int r = check_ctx(s);
+    if (r) return r;
+    share_rec[g].assign((size_t)n * rl, 0.0);
+    return path_solve_dev(s, share_eta[g].data(), n, flags, false, share_rec[g].data());
+  });
+  if (rc) return rc;
+  for (int l = 0; l < L; ++l)
+    memcpy(records + (size_t)l * rl, share_rec[l % G].data() + (size_t)(l / G) * rl, sizeof(double) * rl);
+  const double tr0 = now_ms();
+  if (!(flags & PLS_FLAG_NO_RECOMPUTE)) {
+    std::vector<double> part((size_t)G * L, 0.0);
+    rc = par_for(c, [&](int g, pls_ctx *s) -> int { return path_ssq_dev(s, records, L, part.data() + (size_t)g * L); });
+    if (rc) return rc;
+    for (int l = 0; l < L; ++l) {
+      double tot = 0.0;
+      for (int g = 0; g < G; ++g) tot += part[(size_t)g * L + l];
+      ssq[l] = tot;
+    }
+  }
+  const double tr1 = now_ms();
+  pls_stats &s = c->stats;
+  sum_stats(c, s);
+  s.ms_gram += tg1 - tg0;                        // the exchange of the sums, then the longest per-device finalise
+  s.ms_recompute = tr1 - tr0;
   return PLS_OK;
 }
 

@@ -423,10 +423,13 @@ __global__ void __launch_bounds__(T2, 1) k2_orthant_chains(const K2Args A) {
 }
 
 // K3: lexicographic (objective, b) minimum over the per-CTA winners; NaN sorts first (Julia
-// argmin semantics, Opt.jl:96).  One block.
+// argmin semantics, Opt.jl:96).  One block per problem: block l reduces the n slots from l * n on and writes winner
+// record l (Mp + 2 doubles).
 __global__ void __launch_bounds__(256) k3_select_winner(const double *cta_obj, const long long *cta_b,
                                                         const double *cta_w, int n, int Mp, double *win, const double *scal) {
   const double tau = PLS_TIE_REL * scal[0];
+  cta_obj += (size_t)blockIdx.x * n; cta_b += (size_t)blockIdx.x * n; cta_w += (size_t)blockIdx.x * n * Mp;
+  win += (size_t)blockIdx.x * (Mp + 2);
   __shared__ double so[256];
   __shared__ long long sb[256];
   __shared__ int si[256];
@@ -456,13 +459,8 @@ size_t k2_smem_bytes(int Mp, int cap) {
 
 }  // namespace
 
-int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, const double *scal,
-                   const uint64_t *gmask, int Mp, int Kp, SolveWs &ws, int64_t b_begin,
-                   int64_t b_count, double *d_all_obj, double *d_all_alpha, int sm_count,
-                   cudaStream_t st, int *launches, bool free_top, int force_variant, const uint64_t *h_gmask) {
-  NvtxRange nvtx("pls:K2 orthant NNLS + K3 argmin");
-  if (b_count <= 0) { set_error("k2: empty orthant range"); return PLS_EINVAL; }
-  if (free_top && (Mp > 1024 || d_all_obj || d_all_alpha)) { set_error("k2: paired orthants need M' <= 1024 and no per-orthant outputs"); return PLS_EUNSUPPORTED; }
+int k2_choose(int Mp, int Kp, int64_t b_begin, int64_t b_count, bool outputs, int sm_count, bool free_top,
+              int force_variant, const uint64_t *h_gmask, K2Choice *ch) {
   // variant (PLS_K2_IMPL = v1 | v3 | v4 | v5 overrides):
   //   v3  block pivoting, DMMA, tile-packed inverse split between shared memory and L2   (M' <= 1024)
   //   v1  rank-1 updates on a dense inverse with a global spill path                     (any M')
@@ -476,7 +474,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   const bool force4 = impl && strcmp(impl, "v4") == 0;
   // per-orthant outputs (returnAllSolutions) stay on the one-level kernel: every orthant is then checked against
   // the original G (accuracy on ill-conditioned data matters more than speed on that path)
-  if (variant == 3 && Mp + 1 <= 1024 && pow2 && (force4 || (impl && strcmp(impl, "v5") == 0) || (!impl && !d_all_obj && !d_all_alpha))) variant = 4;
+  if (variant == 3 && Mp + 1 <= 1024 && pow2 && (force4 || (impl && strcmp(impl, "v5") == 0) || (!impl && !outputs))) variant = 4;
   // v5 (two swept tableaus, one CTA per walk): preferred over v4 wherever its window fits (M' + 1 <= 640 and at
   // least one fast group) and the walks are long enough to amortise a cold start
   const bool force5 = impl && strcmp(impl, "v5") == 0;
@@ -485,9 +483,9 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   if (force_variant == K2_FORCE_V1 && !free_top) variant = 1;
   int cap = Mp, occ = 1;
   size_t smem = 0;
-  K3Plan plan3;
-  K4Plan plan4;
-  K5Plan plan5;
+  K3Plan &plan3 = ch->p3;
+  K4Plan &plan4 = ch->p4;
+  K5Plan &plan5 = ch->p5;
   // (M' + 1 > 328: one 512-thread walk per SM with a large window, worth it on long ranges; beyond M' + 1 = 640 untested -> v4)
   const bool wide5 = Mp + 1 > 328;
   if (variant == 4 && !force4 && !no5 && h_gmask && (force5 || Mp + 1 <= 640)) {
@@ -532,6 +530,27 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_orthant_chains, T2, smem));
     if (occ < 1) occ = 1;
   }
+  ch->variant = variant; ch->cap = cap; ch->occ = occ; ch->smem = smem;
+  return PLS_OK;
+}
+
+int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, const double *scal,
+                   const uint64_t *gmask, int Mp, int Kp, SolveWs &ws, int64_t b_begin,
+                   int64_t b_count, double *d_all_obj, double *d_all_alpha, int sm_count,
+                   cudaStream_t st, int *launches, bool free_top, int force_variant, const uint64_t *h_gmask,
+                   int n_prob, size_t g_stride, unsigned long long *noconv) {
+  NvtxRange nvtx("pls:K2 orthant NNLS + K3 argmin");
+  if (b_count <= 0) { set_error("k2: empty orthant range"); return PLS_EINVAL; }
+  if (free_top && (Mp > 1024 || d_all_obj || d_all_alpha)) { set_error("k2: paired orthants need M' <= 1024 and no per-orthant outputs"); return PLS_EUNSUPPORTED; }
+  K2Choice ch;
+  const int rcc = k2_choose(Mp, Kp, b_begin, b_count, d_all_obj || d_all_alpha, sm_count, free_top, force_variant, h_gmask, &ch);
+  if (rcc) return rcc;
+  const int variant = ch.variant, cap = ch.cap, occ = ch.occ;
+  const size_t smem = ch.smem;
+  const K3Plan &plan3 = ch.p3;
+  const K4Plan &plan4 = ch.p4;
+  const K5Plan &plan5 = ch.p5;
+  if (n_prob > 1 && (variant != 3 || d_all_obj || d_all_alpha || !noconv)) { set_error("k2: several problems in one launch need the one-level kernel (v3), per-problem failure counts and no per-orthant outputs"); return PLS_EUNSUPPORTED; }
   const long long max_grid = (long long)sm_count * occ;
   long long grid = max_grid;
 
@@ -544,23 +563,32 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   if (chain_log2 > align_log2) chain_log2 = align_log2;
   if (chain_log2 > Kp) chain_log2 = Kp;
   long long n_chains = b_count >> chain_log2;
+  // (chain lengths above come from one problem's range and the uncapped grid: every problem of a batched launch runs
+  // the chains its own launch would)
+  // PLS_K3_GRID (tests): caps EVERY v3 launch at g CTAs -- single fits and polish re-solves too, and the batch of an
+  // eta path, where one CTA then runs chains of several problems.  Chain lengths are fixed above, before the cap.
+  if (variant == 3)
+    if (const char *eg = getenv("PLS_K3_GRID")) { const long long g = atoll(eg); if (g >= 1 && g < grid) grid = g; }
   if (variant == 4 || variant == 5) {                            // static partition of the Gray sequence
     n_chains = b_count; chain_log2 = 0;
     if (const char *eg = getenv(variant == 4 ? "PLS_K4_GRID" : "PLS_K5_GRID")) { const long long g = atoll(eg); if (g >= 1 && g < grid) grid = g; }   // tests: long walks on small problems
   }
-  if (grid > n_chains) grid = n_chains;
+  if (grid > n_chains * n_prob) grid = n_chains * n_prob;
 
-  // per-CTA workspaces
-  if (max_grid > ws.max_ctas || Mp != ws.Mp) {
+  // per-CTA workspaces (one slot per problem and CTA)
+  const long long slots = max_grid * n_prob;
+  if (slots > ws.max_ctas || Mp != ws.Mp) {
     if (ws.cta_obj) cudaFree(ws.cta_obj);
     if (ws.cta_b) cudaFree(ws.cta_b);
     if (ws.cta_w) cudaFree(ws.cta_w);
     ws.cta_obj = nullptr; ws.cta_b = nullptr; ws.cta_w = nullptr; ws.max_ctas = 0;
-    PLS_CUDA_TRY(cudaMalloc(&ws.cta_obj, sizeof(double) * max_grid));
-    PLS_CUDA_TRY(cudaMalloc(&ws.cta_b, sizeof(long long) * max_grid));
-    PLS_CUDA_TRY(cudaMalloc(&ws.cta_w, sizeof(double) * max_grid * Mp));
-    ws.max_ctas = (int)max_grid; ws.Mp = Mp;
+    PLS_CUDA_TRY(cudaMalloc(&ws.cta_obj, sizeof(double) * slots));
+    PLS_CUDA_TRY(cudaMalloc(&ws.cta_b, sizeof(long long) * slots));
+    PLS_CUDA_TRY(cudaMalloc(&ws.cta_w, sizeof(double) * slots * Mp));
+    ws.max_ctas = (int)slots; ws.Mp = Mp;
   }
+  // a CTA writes the slot of a problem only if it ran one of its chains: the others must read as "no result"
+  if (n_prob > 1) PLS_CUDA_TRY(cudaMemsetAsync(ws.cta_b, 0xff, sizeof(long long) * grid * n_prob, st));
   size_t hneed = 0;
   if (variant == 1 && cap < Mp) hneed = (size_t)max_grid * Mp * Mp * sizeof(double);
   if (variant == 3) hneed = (size_t)max_grid * plan3.hstride * sizeof(double);
@@ -582,7 +610,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     ws.hspill_bytes = hneed;
   }
   PLS_CUDA_TRY(ensure_counters(ws, false, st));
-  PLS_CUDA_TRY(ensure_win(ws, Mp + 2));
+  PLS_CUDA_TRY(ensure_win(ws, (Mp + 2) * n_prob));
   PLS_CUDA_TRY(cudaMemsetAsync(ws.counters + CNT_CHAIN, 0, sizeof(unsigned long long), st));
   ws.last_variant = variant; ws.last_occ = occ; ws.last_grid = (int)grid;
   ws.last_threads = variant == 5 ? plan5.T : (variant == 4 ? plan4.T : (variant == 3 ? plan3.T : T2));
@@ -597,6 +625,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
   A.free_top = free_top ? 1 : 0;
   A.cta_obj = ws.cta_obj; A.cta_b = ws.cta_b; A.cta_w = ws.cta_w;
   A.all_obj = d_all_obj; A.all_alpha = d_all_alpha; A.counters = ws.counters;
+  A.n_prob = n_prob; A.gstride = g_stride; A.noconv = noconv;
   if (variant == 5) {
     A.tab = ws.tab; A.tabstride = plan5.tabstride;
     A.hglob = ws.tab + (size_t)max_grid * plan5.tabstride;        // T0 = [G c; c' yy], written by the launch's prologue kernel
@@ -620,7 +649,7 @@ int k2_solve_range(const Problem &, const double *G, int ldg, const double *c, c
     PLS_CUDA_TRY(cudaGetLastError());
   }
   ++*launches;
-  k3_select_winner<<<1, 256, 0, st>>>(ws.cta_obj, ws.cta_b, ws.cta_w, (int)grid, Mp, ws.win, scal);
+  k3_select_winner<<<n_prob, 256, 0, st>>>(ws.cta_obj, ws.cta_b, ws.cta_w, (int)grid, Mp, ws.win, scal);
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   return PLS_OK;

@@ -20,7 +20,9 @@
 namespace pls {
 namespace {
 
-template <int T, int MODE, int MINB>
+// BATCH: the launch runs A.n_prob problems (an eta path).  It is a template parameter so that the one-problem
+// instantiations keep the registers and spills of a kernel without the per-problem state.
+template <int T, int MODE, int MINB, bool BATCH>
 __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
   constexpr int NW = T / 32;
   const int tid = threadIdx.x;
@@ -40,15 +42,43 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
   const double yy = A.scal[0], cmax = A.scal[1];
   const long long L = 1ll << A.chain_log2;
   double best_obj = 0.0; long long best_b = -1;
+  // BATCH: s_prob is the problem of the chain this CTA runs, s_G its Gram matrix and s_wrow this CTA's alpha row of its
+  // winner slot s_prob * gridDim.x + blockIdx.x, set by thread 0 between chains.  Failed solves are counted per
+  // problem: s_fail0 is ST_NOCONV when the current problem began on this CTA.
   __shared__ unsigned long long s_chain;
+  __shared__ const double *s_G;
+  __shared__ double *s_wrow;
+  __shared__ long long s_fail0;
+  __shared__ int s_prob, s_new;
+  if (BATCH && tid == 0) { s_prob = 0; s_G = A.G; s_wrow = A.cta_w + (size_t)blockIdx.x * Mp; s_fail0 = 0; }
   int nt_dirty = ntc;                          // tiles that may hold stale data (first chain: all)
 
   for (;;) {   // persistent CTA: fetch chains until the range is exhausted
-    if (tid == 0) s_chain = atomicAdd(A.chain_counter, 1ull);
+    if (!BATCH) {
+      if (tid == 0) s_chain = atomicAdd(A.chain_counter, 1ull);
+    } else if (tid == 0) {
+      const unsigned long long ch = atomicAdd(A.chain_counter, 1ull);
+      // chains arrive in increasing order, so this CTA's winner of a problem is final when the problem changes
+      int p = s_prob;
+      const bool live = ch < (unsigned long long)A.n_chains * A.n_prob;
+      const bool nw = live && ch >= (unsigned long long)(p + 1) * A.n_chains;
+      if (nw) {
+        const size_t slot = (size_t)p * gridDim.x + blockIdx.x;
+        if (best_b >= 0) { A.cta_obj[slot] = best_obj; A.cta_b[slot] = best_b; }
+        if (s.stat[ST_NOCONV] != s_fail0) atomicAdd(&A.noconv[p], (unsigned long long)(s.stat[ST_NOCONV] - s_fail0));
+        while (ch >= (unsigned long long)(p + 1) * A.n_chains) ++p;
+        s_prob = p; s_G = A.G + (size_t)p * A.gstride; s_wrow = A.cta_w + ((size_t)p * gridDim.x + blockIdx.x) * Mp;
+        s_fail0 = s.stat[ST_NOCONV];
+      }
+      s_new = nw;
+      s_chain = live ? ch - (unsigned long long)p * A.n_chains : (unsigned long long)A.n_chains;   // the chain within its problem
+    }
     __syncthreads();
     const unsigned long long chain = s_chain;
+    const bool new_prob = BATCH && s_new;
     __syncthreads();
     if (chain >= (unsigned long long)A.n_chains) break;
+    if (new_prob) { best_obj = 0.0; best_b = -1; }
     const long long base = A.b_begin + (long long)chain * L;
 
     clear_state3<T, MODE>(cf, nt_dirty);
@@ -70,7 +100,7 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
       __syncthreads();
 
       Bpp3 st; st.grow_zero = false; st.hwm = hwm; st.nt_cur = nt_cur; st.nt_dirty = nt_dirty; st.r_valid = r_valid;
-      const bool ok = bpp_solve3<T, MODE>(cf, s, A.G, A.ldg, Mp, cmax, st);
+      const bool ok = bpp_solve3<T, MODE>(cf, s, BATCH ? s_G : A.G, A.ldg, Mp, cmax, st);
       if (!ok) STAT_ADD3(ST_NOCONV, 1);
       hwm = st.hwm; nt_cur = st.nt_cur; nt_dirty = st.nt_dirty; r_valid = st.r_valid;
       if (!ok) {                               // failed solve (counted; the caller re-solves the range): restart the chain state
@@ -105,15 +135,21 @@ __global__ void __launch_bounds__(T, MINB) k2v3_orthant_chains(const K2Args A) {
           const int d = s.dd[m];
           double a = (s.pos[m] >= 0 && d != 0) ? fmax(s.w[m] / (double)d, 0.0) : 0.0;
           if (s.sg[m] == SG_FREE) a = s.pos[m] >= 0 ? fabs(s.w[m]) : 0.0;
-          A.cta_w[(size_t)blockIdx.x * Mp + m] = a;
+          if (BATCH) s_wrow[m] = a; else A.cta_w[(size_t)blockIdx.x * Mp + m] = a;
         }
       }
       __syncthreads();
     }
   }  // chains
   if (tid == 0) {
-    A.cta_obj[blockIdx.x] = best_obj;
-    A.cta_b[blockIdx.x] = best_b;
+    if (!BATCH) {
+      A.cta_obj[blockIdx.x] = best_obj;
+      A.cta_b[blockIdx.x] = best_b;
+    } else {
+      const size_t slot = (size_t)s_prob * gridDim.x + blockIdx.x;
+      if (best_b >= 0) { A.cta_obj[slot] = best_obj; A.cta_b[slot] = best_b; }
+      if (s.stat[ST_NOCONV] != s_fail0) atomicAdd(&A.noconv[s_prob], (unsigned long long)(s.stat[ST_NOCONV] - s_fail0));
+    }
     atomicAdd(&A.counters[CNT_PIVOTS], (unsigned long long)s.stat[ST_PIV]);
     atomicAdd(&A.counters[CNT_GRAD], (unsigned long long)s.stat[ST_GRAD]);
     atomicAdd(&A.counters[CNT_SUMP], (unsigned long long)s.stat[ST_SUMP]);
@@ -131,15 +167,13 @@ size_t v3_smem_bytes(int cap, int qs) {
 }
 
 typedef void (*K3Fn)(const K2Args);
-struct Variant { int T, mode, minb; K3Fn fn; };
+struct Variant { int T, mode, minb; K3Fn fn, fn_batch; };   // fn_batch: the instantiation for several problems
+#define V3(t, m, b) {t, m, b, k2v3_orthant_chains<t, m, b, false>, k2v3_orthant_chains<t, m, b, true>}
 const Variant kVariants[] = {
-    {256, 0, 1, k2v3_orthant_chains<256, 0, 1>}, {256, 1, 2, k2v3_orthant_chains<256, 1, 2>},
-    {256, 2, 2, k2v3_orthant_chains<256, 2, 2>}, {256, 1, 3, k2v3_orthant_chains<256, 1, 3>},
-    {512, 0, 1, k2v3_orthant_chains<512, 0, 1>}, {512, 1, 1, k2v3_orthant_chains<512, 1, 1>},
-    {512, 2, 1, k2v3_orthant_chains<512, 2, 1>},
-    {128, 1, 4, k2v3_orthant_chains<128, 1, 4>}, {128, 2, 4, k2v3_orthant_chains<128, 2, 4>},
-    {256, 2, 3, k2v3_orthant_chains<256, 2, 3>},
+    V3(256, 0, 1), V3(256, 1, 2), V3(256, 2, 2), V3(256, 1, 3), V3(512, 0, 1), V3(512, 1, 1), V3(512, 2, 1),
+    V3(128, 1, 4), V3(128, 2, 4), V3(256, 2, 3),
 };
+#undef V3
 
 }  // namespace
 
@@ -168,6 +202,7 @@ int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
   if (!best) { set_error("k2v3: no kernel variant for T=%d mode=%d", T, mode); return PLS_EUNSUPPORTED; }
   const size_t sm = v3_smem_bytes(cap, qs);
   PLS_CUDA_TRY(cudaFuncSetAttribute(best->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  PLS_CUDA_TRY(cudaFuncSetAttribute(best->fn_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   int oc = 1;
   PLS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&oc, best->fn, T, sm));
   if (oc < 1) oc = 1;
@@ -178,7 +213,8 @@ int k2v3_plan(int Mp, K3Plan *pl, bool ignore_env) {
 }
 
 int k2v3_launch(const K2Args &A, const K3Plan &pl, int grid, cudaStream_t st) {
-  kVariants[pl.variant].fn<<<grid, pl.T, pl.smem, st>>>(A);
+  // (the grid and the chain lengths come from fn's occupancy for a batch too: a batch runs every problem's own chains)
+  (A.n_prob > 1 ? kVariants[pl.variant].fn_batch : kVariants[pl.variant].fn)<<<grid, pl.T, pl.smem, st>>>(A);
   PLS_CUDA_TRY(cudaGetLastError());
   return PLS_OK;
 }

@@ -101,6 +101,90 @@ __global__ void k4_sum_parts(const double *__restrict__ part, int n, double *__r
   if (threadIdx.x == 0) *out = sm[0];
 }
 
+// K4 for several weight vectors (an eta path's winners): every tile of 64 rows x 32 columns of Z is read once and
+// dotted with 16 * LJ vectors, a register-tiled product of the tile with W[32 x 16 LJ] (thread: 4 rows x LJ vectors).
+// out[block * 64 + l] = sum over the block's rows of (Z[row,:] . w_l - y[row])^2, each partial added in a fixed order.
+constexpr int KM_ROWS = 64, KM_COLS = 32, KM_VEC = 64;
+template <int LJ>
+__global__ void __launch_bounds__(T4) k4_rows_multi(const double *__restrict__ Z, long long ldz, long long n_rows, int ycol,
+                                                    const double *__restrict__ W, int Mp, int L, double *__restrict__ out) {
+  __shared__ double zs[KM_COLS][KM_ROWS + 1];
+  __shared__ double wsm[KM_COLS][16 * LJ];
+  __shared__ double red[16][16 * LJ];
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;        // vectors tx + 16 j, rows ty + 16 i
+  double ssq[LJ];
+#pragma unroll
+  for (int j = 0; j < LJ; ++j) ssq[j] = 0.0;
+  const long long n_tiles = (n_rows + KM_ROWS - 1) / KM_ROWS;
+  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const long long r0 = tile * KM_ROWS;
+    double acc[4][LJ];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < LJ; ++j) acc[i][j] = 0.0;
+    for (int c0 = 0; c0 < Mp; c0 += KM_COLS) {
+      for (int e = tid; e < KM_COLS * KM_ROWS; e += T4) {
+        const int cc = e / KM_ROWS, rr = e - cc * KM_ROWS;
+        const long long row = r0 + rr;
+        zs[cc][rr] = (c0 + cc < Mp && row < n_rows) ? Z[(long long)(c0 + cc) * ldz + row] : 0.0;
+      }
+      for (int e = tid; e < KM_COLS * 16 * LJ; e += T4) {
+        const int l = e / KM_COLS, cc = e - l * KM_COLS;
+        wsm[cc][l] = (c0 + cc < Mp && l < L) ? W[(size_t)l * Mp + c0 + cc] : 0.0;
+      }
+      __syncthreads();
+#pragma unroll 8
+      for (int k = 0; k < KM_COLS; ++k) {
+        double a[4], b[LJ];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) a[i] = zs[k][ty + 16 * i];
+#pragma unroll
+        for (int j = 0; j < LJ; ++j) b[j] = wsm[k][tx + 16 * j];
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int j = 0; j < LJ; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const long long row = r0 + ty + 16 * i;
+      if (row < n_rows) {
+        const double yv = Z[(long long)ycol * ldz + row];
+#pragma unroll
+        for (int j = 0; j < LJ; ++j) { const double e = acc[i][j] - yv; ssq[j] = fma(e, e, ssq[j]); }
+      }
+    }
+  }
+  // fixed-order sum of the 16 row groups of each vector
+#pragma unroll
+  for (int j = 0; j < LJ; ++j) red[ty][tx + 16 * j] = ssq[j];
+  __syncthreads();
+  for (int l = tid; l < KM_VEC; l += T4) {
+    double s = 0.0;
+    if (l < 16 * LJ)
+      for (int q = 0; q < 16; ++q) s += red[q][l];
+    out[(size_t)blockIdx.x * KM_VEC + l] = s;
+  }
+}
+
+// out[l] = sum over blocks of part[block * 64 + l], one block per vector, fixed order
+__global__ void k4_sum_parts_multi(const double *__restrict__ part, int n, double *__restrict__ out) {
+  __shared__ double sm[256];
+  const int l = blockIdx.x;
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n; i += 256) s += part[(size_t)i * KM_VEC + l];
+  sm[threadIdx.x] = s;
+  __syncthreads();
+  for (int st = 128; st; st >>= 1) {
+    if (threadIdx.x < st) sm[threadIdx.x] += sm[threadIdx.x + st];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[l] = sm[0];
+}
+
 }  // namespace
 
 static long long rows_grid(long long N, int sm_count) {
@@ -129,6 +213,31 @@ int k4_residual(const Problem &pb, SolveWs &ws, const double *d_w, double *d_ssq
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   k4_sum_parts<<<1, 256, 0, st>>>(ws.resid_part, (int)blocks, d_ssq);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  return PLS_OK;
+}
+
+// d_W: L <= 64 device vectors of signed weights, vector l at d_W + l * Mp; d_ssq: L doubles.
+int k4_residual_multi(const Problem &pb, SolveWs &ws, const double *d_W, int L, double *d_ssq, int sm_count,
+                      cudaStream_t st, int *launches) {
+  NvtxRange nvtx("pls:K4 recompute of several winners");
+  if (L < 1 || L > KM_VEC) { set_error("k4: %d weight vectors (1..%d)", L, KM_VEC); return PLS_EINVAL; }
+  const long long n_tiles = (pb.N + KM_ROWS - 1) / KM_ROWS;
+  const long long cap = (long long)sm_count * 4;
+  const int blocks = (int)(n_tiles < cap ? n_tiles : cap);
+  if (blocks > ws.resid_mblocks) {
+    if (ws.resid_mpart) cudaFree(ws.resid_mpart);
+    ws.resid_mpart = nullptr; ws.resid_mblocks = 0;
+    PLS_CUDA_TRY(cudaMalloc(&ws.resid_mpart, sizeof(double) * KM_VEC * (size_t)cap));
+    ws.resid_mblocks = (int)cap;
+  }
+  if (L <= 16) k4_rows_multi<1><<<blocks, T4, 0, st>>>(pb.Z, pb.ldz, pb.N, pb.M + 1, d_W, pb.Mp, L, ws.resid_mpart);
+  else if (L <= 32) k4_rows_multi<2><<<blocks, T4, 0, st>>>(pb.Z, pb.ldz, pb.N, pb.M + 1, d_W, pb.Mp, L, ws.resid_mpart);
+  else k4_rows_multi<4><<<blocks, T4, 0, st>>>(pb.Z, pb.ldz, pb.N, pb.M + 1, d_W, pb.Mp, L, ws.resid_mpart);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  k4_sum_parts_multi<<<L, 256, 0, st>>>(ws.resid_mpart, blocks, d_ssq);
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   return PLS_OK;

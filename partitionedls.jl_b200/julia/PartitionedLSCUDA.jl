@@ -26,7 +26,7 @@ using PartitionedLS: PartLSFitResult, Opt, Alt, BnB, cleanupResult, homogeneousC
 using Random
 import PartitionedLS: fit
 
-export OptCUDA, AltCUDA, BnBCUDA, predict_resident
+export OptCUDA, AltCUDA, BnBCUDA, predict_resident, fit_path
 
 """Marker types of the GPU solvers: `fit(OptCUDA, X, y, P; η)` is `fit(Opt, X, y, P; η)` on libpls_cuda.so."""
 struct OptCUDA end
@@ -98,6 +98,38 @@ function fit(::Type{OptCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:Ab
         return (model, nothing, (; solutions = sols))
     end
     return (model, nothing, (; opt = opt))
+end
+
+"""
+    fit_path(OptCUDA, X, y, P; η::AbstractVector)
+
+`fit(OptCUDA, X, y, P; η=η[l])` for every value of `η` (1 to 64 values, any order, duplicates allowed) on one upload
+of the data (`pls_load` + `pls_opt_fit_path`): one Gram build, the orthant solves of all η, one pass over X for all
+winners.  Returns a vector with one `(model, nothing, (; opt, b, stats))` per η; entry l is bitwise the model
+`fit(OptCUDA, X, y, P; η=η[l])` returns (objective within 1e-12 relative).  `stats` is the call's, shared by all.
+"""
+function fit_path(::Type{OptCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:AbstractFloat,1}, P::Array{Int,2};
+                  η::AbstractVector)
+    Xd = convert(Matrix{Float64}, X); yd = convert(Vector{Float64}, y); Pd = convert(Matrix{Int64}, P)
+    N, M = size(Xd); K = size(Pd, 2); L = length(η); etas = convert(Vector{Float64}, η)
+    alpha = zeros(Float64, M + 1, L); b = zeros(Int64, L); obj = zeros(Float64, L); stats = Ref{PlsStats}()
+    ctx = context()
+    GC.@preserve Xd yd Pd etas alpha b obj begin
+        _check(ccall((:pls_load, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, Int64, Int64, Ptr{Cdouble}, Ptr{Int64}, Int64, Cdouble),
+            ctx, Xd, N, N, M, yd, Pd, K, 0.0))
+        _check(ccall((:pls_opt_fit_path, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, UInt32, Ptr{Cdouble}, Ptr{Int64}, Ptr{Cdouble}, Ref{PlsStats}),
+            ctx, etas, L, UInt32(0), alpha, b, obj, stats))
+    end
+    beta(bb) = [2 * ((bb >> (k - 1)) & 1) - 1 for k in 1:K+1]          # indextobeta, Opt.jl:4-20
+    out = []
+    for l in 1:L
+        a = alpha[:, l]
+        opt, model = cleanupResult(Opt, (obj[l], a[1:end-1], beta(b[l])[1:end-1], beta(b[l])[end] * a[end], P), P)
+        push!(out, (model, nothing, (; opt = opt, b = b[l], stats = stats[])))
+    end
+    return out
 end
 
 """
