@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PLS_VERSION 110 /* 0.1.1: pls_opt_fit_path */
+#define PLS_VERSION 120 /* 0.1.2: pls_opt_cv_path */
 
 enum {
   PLS_OK = 0,
@@ -172,6 +172,28 @@ int pls_opt_fit_resident(pls_ctx *ctx, uint32_t flags, double *alpha_raw, int64_
 int pls_opt_fit_path(pls_ctx *ctx, const double *etas, int64_t L, uint32_t flags, double *alpha_raw, int64_t *b_best,
                      double *obj_best, pls_stats *stats);
 
+/* ---- K-fold cross-validation of fit(Opt) over a grid of eta on the resident data set (one-GPU context) -------------
+ * One K1 pass over a fold-contiguous copy of the loaded rows gives the raw Gram sums S_f of every fold; the training
+ * system of fold f is sum_{g != f} S_g (ascending g) + eta_l Po Po', solved as pls_opt_fit_path solves its systems, and
+ * one K4 pass over the copy scores every winner on its held-out rows.  X is not uploaded again.
+ *   fold_id[N]          fold of every loaded row, 0 <= fold_id[n] < F, every fold non-empty; 2 <= F <= 32
+ *   etas[L]             as for pls_opt_fit_path (1 <= L <= 64, finite, >= 0, duplicates allowed)
+ *   alpha_raw[(M+1) x F*L], b_best[F*L], obj_train[F*L]
+ *                       column f*L + l = the winner of fit(Opt) on the rows with fold_id != f at eta_l; obj_train is its
+ *                       Gram-space objective (what PLS_FLAG_NO_RECOMPUTE returns, eta rows included)
+ *   ssq_heldout[F*L]    sum over the rows of fold f of (Xo * w - y)^2 for that winner, w = (Po .* alpha) * beta (no eta term)
+ *   cv_err[L]           sum over f of ssq_heldout[f*L + l] / N   (pooled held-out MSE)
+ *   best                argmin over l of cv_err, lowest index on exact ties
+ *   flags               PLS_FLAG_ENUMERATE_INTERCEPT as for pls_opt_fit_resident
+ *   stats               of the whole call (ms_gram: the copy and the per-fold K1, ms_nnls: every fold's finalise, K2 and
+ *                       K3, ms_recompute: the held-out K4 pass; orthants = F L 2^(K+1))
+ * The context's own eta, S, G, c and gram_ready are not changed.  Refused: PLS_EINVAL for a null pointer, no data loaded,
+ * F or L out of range, a fold id out of range, an empty fold, a bad eta or K' > 40; PLS_EUNSUPPORTED for M' > 1024 or a
+ * multi-GPU context.  The copy of X is a scratch buffer of the call (PLS_ENOMEM if it cannot be allocated). */
+int pls_opt_cv_path(pls_ctx *ctx, const int32_t *fold_id, int64_t F, const double *etas, int64_t L, uint32_t flags,
+                    double *alpha_raw, int64_t *b_best, double *obj_train, double *ssq_heldout, double *cv_err,
+                    int64_t *best, pls_stats *stats);
+
 /* ---- stage-wise entry points (one process per GPU; the caller owns the collectives) ----------
  * K1 on the loaded rows.  pls_gram_raw exposes the device buffer of raw sums S = Z'Z
  * ((M+2) x (M+2) doubles, column-major, lower triangle valid) so the caller can all-reduce it in
@@ -225,6 +247,9 @@ int pls_bnb_lower_bounds(pls_ctx *ctx, const uint64_t *pos_masks, const uint64_t
 /* pls_residual_partial_multi: the K4 pass of pls_opt_fit_path on the resident rows for L <= 64 signed weight vectors
  * W[l * (M+1) + m]: ssq_out[l] = sum over the loaded rows of (Xo * w_l - y)^2 (one-GPU context). */
 int pls_residual_partial_multi(pls_ctx *ctx, const double *W, int64_t L, double *ssq_out);
+/* pls_cv_fold_sums: the F raw fold sums S_f = Z_f' Z_f of pls_opt_cv_path ((M+2) x (M+2) each, column-major, lower
+ * triangle valid, as pls_gram_raw), fold f at S_out + f * (M+2)^2 (one-GPU context). */
+int pls_cv_fold_sums(pls_ctx *ctx, const int32_t *fold_id, int64_t F, double *S_out);
 int pls_nnls_batch(pls_ctx *ctx, const double *G, const double *c, double yy, int64_t Mp,
                    const uint64_t *gmask, int64_t Kp, int64_t b_begin, int64_t b_count,
                    double *obj_out, double *alpha_out);

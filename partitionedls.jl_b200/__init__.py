@@ -25,7 +25,7 @@ import numpy as np
 from . import _abi
 from ._abi import Context, PlsError  # noqa: F401
 
-__all__ = ["fit", "fit_path", "predict", "predict_resident", "PartLSFitResult", "Opt", "Alt", "BnB", "homogeneousCoords",
+__all__ = ["fit", "fit_path", "fit_cv", "draw_folds", "predict", "predict_resident", "PartLSFitResult", "Opt", "Alt", "BnB", "homogeneousCoords",
            "regularizeProblem", "Context", "PlsError", "default_context", "draw_alt_starts"]
 
 
@@ -194,6 +194,79 @@ def fit_path(alg, X, y, P, etas, *, ctx=None, **flags):
         opt, model = _cleanup_result(r["opt"], r["alpha_raw"], r["b_best"], P)
         out.append((model, None, SimpleNamespace(opt=opt, b=r["b_best"], stats=stats)))
     return out
+
+
+def draw_folds(N, folds=5, seed=0):
+    """Balanced random folds of N rows: fold_id = permutation(N) % folds with numpy's default_rng(seed), so the fold
+    sizes differ by at most one and the same seed gives the same folds."""
+    return (np.random.default_rng(seed).permutation(int(N)) % int(folds)).astype(np.int32)
+
+
+def _check_cv_args(N, etas, folds, seed, fold_ids):
+    """fit_cv's arguments, checked on the host before any device work: returns (fold ids, F, etas)."""
+    e = np.asarray(etas, dtype=np.float64).reshape(-1)
+    if not 1 <= len(e) <= 64:
+        raise ValueError(f"{len(e)} values of η (1..64)")
+    if not np.all(np.isfinite(e)) or np.any(e < 0):
+        raise ValueError("every η must be finite and >= 0")
+    if fold_ids is None:
+        if int(folds) != folds or not 2 <= folds <= 32:
+            raise ValueError(f"folds = {folds} (2..32)")
+        if N < folds:
+            raise ValueError(f"{N} rows cannot fill {folds} folds")
+        f = draw_folds(N, folds, seed)
+    else:
+        f = np.asarray(fold_ids).reshape(-1)
+        if f.shape[0] != N:
+            raise ValueError(f"{f.shape[0]} fold ids for {N} rows")
+        if not np.issubdtype(f.dtype, np.integer):
+            raise ValueError("fold ids must be integers")
+        if f.min() < 0:
+            raise ValueError("fold ids must be >= 0")
+        folds = int(f.max()) + 1
+        if not 2 <= folds <= 32:
+            raise ValueError(f"{folds} folds (2..32)")
+        if np.any(np.bincount(f, minlength=folds) == 0):
+            raise ValueError("every fold 0..max(fold_ids) must hold a row")
+        f = f.astype(np.int32)
+    return f, int(folds), e
+
+
+def fit_cv(alg, X, y, P, etas, *, folds=5, seed=0, fold_ids=None, refit=True, ctx=None):
+    """K-fold cross-validation of fit(Opt, X, y, P; η) over `etas` (1..64 values) on one resident copy of the data
+    (pls_opt_cv_path): for every fold f and η_l, fit(Opt) on the rows outside fold f and its squared error on fold f.
+    fold_ids (N integers, folds 0..F-1, none empty, 2 <= F <= 32) defaults to draw_folds(N, folds, seed).
+
+    Returns a namespace with
+      cv_err[l]    pooled held-out mean squared error of η_l (sum over folds of the squared errors / N)
+      best, η      index of the lowest cv_err (lowest index on ties) and its η
+      folds[f][l]  (PartLSFitResult, None, report) of fold f's training fit at η_l, cleaned as fit cleans it;
+                   report.opt is its Gram-space training objective, report.b its orthant, report.ssq_heldout its
+                   squared error on fold f
+      fold_ids, stats
+      model, report  with refit: fit(Opt, X, y, P; η=best η) on all rows, from the same upload (None without)."""
+    if not (alg is Opt or isinstance(alg, Opt)):
+        raise TypeError(f"fit_cv supports Opt only, not {alg!r}")
+    Xd, yd, Pd = _abi._as_inputs(X, y, P)
+    f, F, e = _check_cv_args(Xd.shape[0], etas, folds, seed, fold_ids)
+    c = ctx or default_context()
+    c.load(Xd, yd, Pd, prepared=True)
+    r = c.opt_cv_path(f, e, F=F)
+    per_fold = []
+    for g in range(F):
+        row = []
+        for l in range(len(e)):
+            opt, m = _cleanup_result(r["obj_train"][g, l], r["alpha_raw"][g, l], int(r["b_best"][g, l]), P)
+            row.append((m, None, SimpleNamespace(opt=opt, b=int(r["b_best"][g, l]), ssq_heldout=r["ssq_heldout"][g, l])))
+        per_fold.append(row)
+    best = r["best"]
+    model = report = None
+    if refit:
+        res, st = c.opt_fit_path([e[best]])
+        opt, model = _cleanup_result(res[0]["opt"], res[0]["alpha_raw"], res[0]["b_best"], P)
+        report = SimpleNamespace(opt=opt, b=res[0]["b_best"], stats=st)
+    return SimpleNamespace(cv_err=r["cv_err"], best=best, η=float(e[best]), eta=float(e[best]), folds=per_fold,
+                           fold_ids=f, model=model, report=report, stats=r["stats"])
 
 
 def predict_resident(model, ctx, N):

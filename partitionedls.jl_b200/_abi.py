@@ -81,12 +81,16 @@ lib.pls_bnb_lower_bounds.argtypes = [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_u
 lib.pls_gram.argtypes = [_vp, _dp, C.c_int64, C.c_int64, _dp, _ip, C.c_int64, C.c_double, _dp, _dp, _dp]
 lib.pls_opt_fit_path.argtypes = [_vp, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, C.POINTER(PlsStats)]
 lib.pls_residual_partial_multi.argtypes = [_vp, _dp, C.c_int64, _dp]
+_i32p = C.POINTER(C.c_int32)
+lib.pls_opt_cv_path.argtypes = [_vp, _i32p, C.c_int64, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, _dp, _dp, _ip,
+                                C.POINTER(PlsStats)]
+lib.pls_cv_fold_sums.argtypes = [_vp, _i32p, C.c_int64, _dp]
 lib.pls_nnls_batch.argtypes = [_vp, _dp, _dp, C.c_double, C.c_int64, C.POINTER(C.c_uint64), C.c_int64,
                                C.c_int64, C.c_int64, _dp, _dp]
 for _n in ("pls_create", "pls_opt_fit", "pls_bnb_fit", "pls_bnb_fit_resident", "pls_alt_fit", "pls_alt_fit_resident", "pls_residual_partial_w", "pls_predict_resident", "pls_objective_finish_w", "pls_load", "pls_opt_fit_resident", "pls_gram_build", "pls_gram_raw",
            "pls_gram_finalize", "pls_opt_solve_range", "pls_opt_solve_pairs", "pls_opt_residual_partial", "pls_opt_objective_finish",
            "pls_get_stats", "pls_gram_scalars", "pls_bnb_lower_bounds", "pls_gram", "pls_nnls_batch", "pls_opt_fit_path",
-           "pls_residual_partial_multi"):
+           "pls_residual_partial_multi", "pls_opt_cv_path", "pls_cv_fold_sums"):
     getattr(lib, _n).restype = C.c_int
 
 
@@ -225,6 +229,39 @@ class Context:
         alpha = np.zeros((L, M + 1)); b = np.zeros(L, dtype=np.int64); obj = np.zeros(L); st = PlsStats()
         _check(lib.pls_opt_fit_path(self._h, _d(e), L, flags, _d(alpha), b.ctypes.data_as(_ip), _d(obj), C.byref(st)))
         return [dict(alpha_raw=alpha[l], b_best=int(b[l]), opt=float(obj[l])) for l in range(L)], st.as_dict()
+
+    def _fold_ids(self, fold_id):
+        f = np.ascontiguousarray(np.asarray(fold_id).reshape(-1), dtype=np.int32)
+        if len(f) != self._shape[0]:
+            raise ValueError(f"{len(f)} fold ids for {self._shape[0]} loaded rows")
+        return f
+
+    def opt_cv_path(self, fold_id, etas, flags=0, F=None):
+        """pls_opt_cv_path: K-fold cross-validation of fit(Opt) over `etas` on the resident data set.  fold_id[n] is the
+        fold of loaded row n; F defaults to max(fold_id) + 1.  Per (fold f, eta l): the winner on the other folds' rows
+        (alpha_raw[f, l], b_best[f, l], obj_train[f, l], its Gram-space objective) and its sum of squared errors on fold f
+        (ssq_heldout[f, l]); cv_err[l] = sum_f ssq_heldout[f, l] / N, best = argmin (lowest index on ties)."""
+        N, M, K = self._shape
+        f = self._fold_ids(fold_id)
+        F = int(f.max()) + 1 if F is None else int(F)
+        e = np.ascontiguousarray(np.asarray(etas, dtype=np.float64).reshape(-1))
+        L = len(e)
+        FL = max(F, 0) * L
+        alpha = np.zeros((FL, M + 1)); b = np.zeros(FL, dtype=np.int64); obj = np.zeros(FL); ssq = np.zeros(FL)
+        cv = np.zeros(L); best = C.c_int64(); st = PlsStats()
+        _check(lib.pls_opt_cv_path(self._h, f.ctypes.data_as(_i32p), F, _d(e), L, flags, _d(alpha), b.ctypes.data_as(_ip),
+                                   _d(obj), _d(ssq), _d(cv), C.byref(best), C.byref(st)))
+        return dict(alpha_raw=alpha.reshape(F, L, M + 1), b_best=b.reshape(F, L), obj_train=obj.reshape(F, L),
+                    ssq_heldout=ssq.reshape(F, L), cv_err=cv, best=best.value, stats=st.as_dict())
+
+    def cv_fold_sums(self, fold_id, F):
+        """pls_cv_fold_sums: the raw Gram sums S_f = Z_f' Z_f of every fold, (F, M+2, M+2) (S_f[j, i] = column-major
+        entry (i, j); lower triangle valid)."""
+        N, M, K = self._shape
+        f = self._fold_ids(fold_id)
+        out = np.zeros((max(int(F), 0), M + 2, M + 2))
+        _check(lib.pls_cv_fold_sums(self._h, f.ctypes.data_as(_i32p), int(F), _d(out)))
+        return out
 
     def gram_build(self):
         _check(lib.pls_gram_build(self._h))

@@ -353,8 +353,7 @@ void add_counters(pls_stats &a, const pls_stats &s) {
   a.k2_max_drift = std::fmax(a.k2_max_drift, s.k2_max_drift);
 }
 
-// Layout of ws.path for L problems: etas [64] | failure counts [64] | c [ldg] | scal_l [4 L] | G_l [L][gstride]
-struct PathWs { double *etas, *c, *scal, *G; unsigned long long *noconv; size_t gstride; };
+}  // namespace
 
 int path_ws(pls_ctx *c, int L, PathWs *p) {
   const Problem &pb = c->pb;
@@ -378,12 +377,19 @@ int path_ws(pls_ctx *c, int L, PathWs *p) {
   return PLS_OK;
 }
 
-}  // namespace
+int path_check_formed(pls_ctx *c, const PathWs &p, const double *etas, int L) {
+  cudaStream_t st = c->stream;
+  std::vector<double> scal((size_t)4 * L);
+  PLS_CUDA_TRY(cudaMemcpyAsync(scal.data(), p.scal, sizeof(double) * 4 * L, cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaStreamSynchronize(st));
+  for (int l = 0; l < L; ++l)
+    if (scal[4 * l + 3] != 0.0) { set_error("non-finite values in X or y, or in the Gram matrix of eta = %g", etas[l]); return PLS_ENUMERIC; }
+  return PLS_OK;
+}
 
 int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool build_S, double *records) {
   Problem &pb = c->pb;
   cudaStream_t st = c->stream;
-  const int Mp = pb.Mp, rl = record_len(Mp);
   PathWs p;
   int rc = path_ws(c, L, &p);
   if (rc) return rc;
@@ -393,20 +399,31 @@ int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool b
   rc = k1_gram_finalize_path(pb, p.etas, L, p.G, p.gstride, p.c, p.scal, st, &c->launches);
   if (rc) return rc;
   PLS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
-  std::vector<double> scal((size_t)4 * L);
-  PLS_CUDA_TRY(cudaMemcpyAsync(scal.data(), p.scal, sizeof(double) * 4 * L, cudaMemcpyDeviceToHost, st));
-  PLS_CUDA_TRY(cudaStreamSynchronize(st));
-  for (int l = 0; l < L; ++l)
-    if (scal[4 * l + 3] != 0.0) { set_error("non-finite values in X or y, or in the Gram matrix of eta = %g", etas[l]); return PLS_ENUMERIC; }
+  rc = path_check_formed(c, p, etas, L);
+  if (rc) return rc;
   float ms = 0.f;
   cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]);
   const double t0 = now_ms();
+  pls_stats acc;
+  memset(&acc, 0, sizeof(acc));
+  rc = path_solve_formed(c, p, L, flags, records, &acc);
+  if (rc) return rc;
+  pls_stats &s = c->stats;
+  s = acc;                                       // (fit_start cleared the rest; the upload time of a path is 0)
+  s.ms_gram = ms;
+  s.ms_nnls = now_ms() - t0;
+  return PLS_OK;
+}
 
+int path_solve_formed(pls_ctx *c, const PathWs &p, int L, uint32_t flags, double *records, pls_stats *acc_out) {
+  Problem &pb = c->pb;
+  cudaStream_t st = c->stream;
+  const int Mp = pb.Mp, rl = record_len(Mp);
+  int rc;
   const bool pairs = use_pairs(c, flags, false);
   const int64_t count = (int64_t)1 << (pairs ? pb.Kp - 1 : pb.Kp);
   auto sys = [&](int l) { return GramSys{p.G + (size_t)l * p.gstride, p.c, p.scal + 4 * l}; };
-  pls_stats acc;
-  memset(&acc, 0, sizeof(acc));
+  pls_stats &acc = *acc_out;
   // one eta alone, exactly as its resident fit solves it: K2 + K3, the single-pivot fallback, the polish
   auto solve_one = [&](int l) -> int {
     K2Range r;
@@ -446,11 +463,7 @@ int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool b
       variant = c->stats.k2_variant; threads = (int)c->stats.k2_threads; occ = (int)c->stats.k2_ctas_per_sm; grid = (int)c->stats.k2_grid;
     }
   }
-  pls_stats &s = c->stats;
-  s = acc;                                       // (fit_start cleared the rest; the upload time of a path is 0)
-  s.k2_variant = variant; s.k2_threads = threads; s.k2_ctas_per_sm = occ; s.k2_grid = grid;
-  s.ms_gram = ms;
-  s.ms_nnls = now_ms() - t0;
+  acc.k2_variant = variant; acc.k2_threads = threads; acc.k2_ctas_per_sm = occ; acc.k2_grid = grid;
   return PLS_OK;
 }
 

@@ -188,7 +188,19 @@ struct K2Args {
 };
 
 // ---- kernel launchers (defined in gram.cu / nnls.cu / resid.cu) -----------------------------
+// K1's split-K plan for N rows: n_chunks chunks of rows_per_chunk rows (a multiple of 32) over the n_rows_pad = round_up(N,
+// 32) rows, each chunk one CTA per lower-triangle tile of the zcols_pad columns
+struct K1Plan { int n_tiles, n_chunks; long long n_rows_pad, rows_per_chunk; };
+K1Plan k1_plan(int64_t N, int zcols_pad);
 int k1_gram_build(Problem &pb, cudaStream_t st, int *launches);
+// K1 on the fold-contiguous copy Zf of Z (ldf rows per column, zero padded like Z, ldf a multiple of R): every chunk of R
+// rows lies in one fold, fold f in chunks [d_chunk0[f], d_chunk0[f + 1]).  S_folds + f * zcols^2 = S_f, the raw sums of
+// fold f's rows (lower triangle valid, as pb.S).  pb's own S is untouched; pb.part is the scratch of the partial tiles.
+int k1_gram_build_folds(Problem &pb, const double *Zf, int64_t ldf, long long R, const int *d_chunk0, int F,
+                        double *S_folds, cudaStream_t st, int *launches);
+// k1_gram_finalize_path on the training sums of held-out fold f: sum over g != f (ascending) of S_folds + g * zcols^2
+int k1_gram_finalize_folds(const Problem &pb, const double *S_folds, int F, int f, const double *etas, int L, double *G,
+                           size_t gstride, double *c, double *scal, cudaStream_t st, int *launches);
 int k1_gram_finalize(Problem &pb, cudaStream_t st, int *launches);
 // G_l = S + etas[l] |groups(i) & groups(j)| for l < L (device etas) into G + l * gstride, scal_l into scal + 4 l, and
 // the shared c -- each G_l bitwise what k1_gram_finalize gives for eta = etas[l].  pb's own G, c, scal are untouched.
@@ -249,6 +261,13 @@ int k4_residual(const Problem &pb, SolveWs &ws, const double *d_w, double *d_ssq
 // K4 for L <= 64 signed weight vectors W[l * Mp + m] in one pass over Z: d_ssq[l] = sum_rows (Z[row,:] . w_l - y)^2
 int k4_residual_multi(const Problem &pb, SolveWs &ws, const double *d_W, int L, double *d_ssq, int sm_count,
                       cudaStream_t st, int *launches);
+// K4 of cross-validation on the fold-contiguous copy Zf: d_ssq[f * L + l] = sum over fold f's rows (segment f: rows
+// [d_row0[f], d_row0[f] + d_nrows[f])) of (Zf[row,:] . w_{f,l} - y)^2, w_{f,l} = d_W + (f * L + l) * Mp; one pass over the
+// F segments, `blocks` CTAs per fold, partials in d_part (F * blocks * 64 doubles)
+int k4_residual_folds(const Problem &pb, const double *Zf, int64_t ldf, const long long *d_row0, const long long *d_nrows,
+                      int F, const double *d_W, int L, int blocks, double *d_part, double *d_ssq, cudaStream_t st,
+                      int *launches);
+int k4_folds_blocks(int64_t max_rows, int F, int sm_count);
 int k7_predict(const Problem &pb, const double *d_w, double *d_yhat, int sm_count, cudaStream_t st, int *launches);
 
 }  // namespace pls

@@ -88,6 +88,16 @@ double eta_term(const pls_ctx *c, double eta, const double *alpha_raw, int64_t b
 double eta_term_w(const pls_ctx *c, const double *w);
 int residual_partial_w(pls_ctx *c, const double *w, double *ssq_out);
 double now_ms();
+// The eta path's workspace in ws.path for L <= 64 problems: etas [64] | failure counts [64] | c [ldg] | scal_l [4 L] |
+// G_l [L][gstride]
+struct PathWs { double *etas, *c, *scal, *G; unsigned long long *noconv; size_t gstride; };
+int path_ws(pls_ctx *c, int L, PathWs *p);
+// Synchronises the stream; PLS_ENUMERIC if a finalise flagged a non-finite value in scal_l of p
+int path_check_formed(pls_ctx *c, const PathWs &p, const double *etas, int L);
+// K2 + K3 of the L systems already formed in p (G_l, the shared c, scal_l), each exactly as its resident fit solves it:
+// the batched one-level launch or one launch per eta, the single-pivot fallback, the polish.  Winner records as for
+// path_solve_dev; the work counters are added into *acc and the kernel of the main ranges is set in acc->k2_*.
+int path_solve_formed(pls_ctx *c, const PathWs &p, int L, uint32_t flags, double *records, pls_stats *acc);
 // The eta path on one device (api.cu): the winner records (record_len(M') doubles each) of etas[0..L) on the S this
 // context holds (built first unless build_S is false), and the counters of the call added into c->stats.
 int path_solve_dev(pls_ctx *c, const double *etas, int L, uint32_t flags, bool build_S, double *records);

@@ -305,7 +305,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-bool make_zmap(const Problem &pb, CUtensorMap *map) {
+bool make_zmap(const double *Z, int64_t ldz, int zcols_pad, CUtensorMap *map) {
   static EncodeTiledFn fn = nullptr;
   if (!fn) {
     void *p = nullptr;
@@ -317,11 +317,11 @@ bool make_zmap(const Problem &pb, CUtensorMap *map) {
     }
     fn = (EncodeTiledFn)p;
   }
-  const cuuint64_t gdim[2] = {(cuuint64_t)pb.ldz, (cuuint64_t)pb.zcols_pad};
-  const cuuint64_t gstr[1] = {(cuuint64_t)pb.ldz * sizeof(double)};
+  const cuuint64_t gdim[2] = {(cuuint64_t)ldz, (cuuint64_t)zcols_pad};
+  const cuuint64_t gstr[1] = {(cuuint64_t)ldz * sizeof(double)};
   const cuuint32_t box[2] = {KS, BT};
   const cuuint32_t estr[2] = {1, 1};
-  return fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, pb.Z, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  return fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double *>(Z), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -341,10 +341,48 @@ __global__ void k1_reduce(const double *__restrict__ part, int n_tiles, int n_ch
   S[idx] = s;
 }
 
+// K1 over fold-contiguous rows: chunks [chunk0[f], chunk0[f + 1]) hold fold f only.  blockIdx.y = f:
+// S_f[i + j*zc] (i >= j) = sum over fold f's chunks of the partial tiles, fixed order.
+__global__ void k1_reduce_folds(const double *__restrict__ part, int n_tiles, const int *__restrict__ chunk0, int zc,
+                                double *__restrict__ S_folds) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)zc * zc) return;
+  double *S = S_folds + (size_t)blockIdx.y * zc * zc;
+  const int i = (int)(idx % zc), j = (int)(idx / zc);
+  if (i < j) { S[idx] = 0.0; return; }
+  const int ti = i / BT, tj = j / BT;
+  const int tile = ti * (ti + 1) / 2 + tj;
+  const size_t off = (size_t)(j % BT) * BT + (i % BT);
+  double s = 0.0;
+  for (int ch = chunk0[blockIdx.y]; ch < chunk0[blockIdx.y + 1]; ++ch) s += part[((size_t)ch * n_tiles + tile) * (BT * BT) + off];
+  S[idx] = s;
+}
+
+// The raw sums a finalise reads: S[k] of one system ...
+struct SumsOne {
+  const double *__restrict__ S;
+  __device__ __forceinline__ double operator()(size_t k) const { return S[k]; }
+};
+// ... or the training sums of held-out fold f: sum over the other folds g, ascending, of S_g[k] (no subtraction from a
+// total, so nothing cancels)
+struct SumsExcept {
+  const double *__restrict__ S;
+  size_t stride;
+  int F, f;
+  __device__ __forceinline__ double operator()(size_t k) const {
+    const int g0 = f == 0 ? 1 : 0;
+    double s = S[(size_t)g0 * stride + k];
+    for (int g = g0 + 1; g < F; ++g)
+      if (g != f) s += S[(size_t)g * stride + k];
+    return s;
+  }
+};
+
 // G = S (mirrored) + eta * |groups(i) & groups(j)|;  c = S[y row] (when c is not null);
 // scal = {yy, max|c|, max diag, non-finite flag} (scal[1..3] zeroed before launch; max via
 // atomicMax on the bit pattern, valid for non-negative doubles)
-__device__ __forceinline__ void finalize_entry(long long idx, const double *__restrict__ S, int zc, int Mp, double eta,
+template <class Sums>
+__device__ __forceinline__ void finalize_entry(long long idx, const Sums S, int zc, int Mp, double eta,
                                                const uint64_t *__restrict__ gmask, double *__restrict__ G, int ldg,
                                                double *__restrict__ c, double *__restrict__ scal) {
   double mc = 0.0, md = 0.0;
@@ -354,20 +392,20 @@ __device__ __forceinline__ void finalize_entry(long long idx, const double *__re
     if (i >= Mp) G[idx] = 0.0;
     else {
       const int hi = i > j ? i : j, lo = i > j ? j : i;
-      double g = S[(size_t)lo * zc + hi];
+      double g = S((size_t)lo * zc + hi);
       if (eta != 0.0) g += eta * (double)__popcll(gmask[i] & gmask[j]);
       G[idx] = g;
       if (!isfinite(g)) bad = 1;
       if (i == j) md = fabs(g);
       if (j == 0) {
-        const double ci = S[(size_t)i * zc + Mp];     // row index of y in Z'Z is Mp = M+1
+        const double ci = S((size_t)i * zc + Mp);     // row index of y in Z'Z is Mp = M+1
         if (c) c[i] = ci;
         mc = fabs(ci);
         if (!isfinite(ci)) bad = 1;
       }
     }
     if (idx == 0) {
-      const double yy = S[(size_t)Mp * zc + Mp];
+      const double yy = S((size_t)Mp * zc + Mp);
       scal[0] = yy;
       if (!isfinite(yy)) bad = 1;
     }
@@ -388,7 +426,7 @@ __device__ __forceinline__ void finalize_entry(long long idx, const double *__re
 __global__ void k1_finalize(const double *__restrict__ S, int zc, int Mp, double eta,
                             const uint64_t *__restrict__ gmask, double *__restrict__ G, int ldg,
                             double *__restrict__ c, double *__restrict__ scal) {
-  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, S, zc, Mp, eta, gmask, G, ldg, c, scal);
+  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, SumsOne{S}, zc, Mp, eta, gmask, G, ldg, c, scal);
 }
 
 // The eta path: blockIdx.y = l builds G_l and scal_l with etas[l]; c (shared by all l) is written by l = 0.
@@ -396,29 +434,46 @@ __global__ void k1_finalize_path(const double *__restrict__ S, int zc, int Mp, c
                                  const uint64_t *__restrict__ gmask, double *__restrict__ G, size_t gstride, int ldg,
                                  double *__restrict__ c, double *__restrict__ scal) {
   const int l = blockIdx.y;
-  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, S, zc, Mp, etas[l], gmask, G + (size_t)l * gstride,
+  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, SumsOne{S}, zc, Mp, etas[l], gmask, G + (size_t)l * gstride,
                  ldg, l == 0 ? c : nullptr, scal + 4 * l);
+}
+
+// Cross-validation: k1_finalize_path on the training sums of held-out fold f (the other folds' S_g, S_folds + g * zc^2)
+__global__ void k1_finalize_folds(const double *__restrict__ S_folds, int F, int f, int zc, int Mp,
+                                  const double *__restrict__ etas, const uint64_t *__restrict__ gmask, double *__restrict__ G,
+                                  size_t gstride, int ldg, double *__restrict__ c, double *__restrict__ scal) {
+  const int l = blockIdx.y;
+  finalize_entry((long long)blockIdx.x * blockDim.x + threadIdx.x, SumsExcept{S_folds, (size_t)zc * zc, F, f}, zc, Mp,
+                 etas[l], gmask, G + (size_t)l * gstride, ldg, l == 0 ? c : nullptr, scal + 4 * l);
 }
 
 }  // namespace
 
-int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
-  NvtxRange nvtx("pls:K1 gram build (TMA + DMMA)");
-  const int nt = pb.zcols_pad / BT;
-  const int n_tiles = nt * (nt + 1) / 2;
-  const long long n_rows_pad = round_up(pb.N, KB);      // <= ldz (ldz % 32 == 0)
+K1Plan k1_plan(int64_t N, int zcols_pad) {
+  K1Plan p;
+  const int nt = zcols_pad / BT;
+  p.n_tiles = nt * (nt + 1) / 2;
+  p.n_rows_pad = round_up(N, KB);      // <= ldz (ldz % 32 == 0)
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // ~4 waves of CTAs at 3 CTAs per SM (measured: 1 / 2 / 4 waves = 19.2 / 22.5 / 24.5 TFLOP/s at the configs[2] shape), chunks of whole stages
   const int waves = 4;
-  long long want_chunks = ((long long)waves * 3 * sms + n_tiles - 1) / n_tiles;
-  long long max_chunks = n_rows_pad / (KB * 8);
+  long long want_chunks = ((long long)waves * 3 * sms + p.n_tiles - 1) / p.n_tiles;
+  long long max_chunks = p.n_rows_pad / (KB * 8);
   if (max_chunks < 1) max_chunks = 1;
   if (want_chunks > max_chunks) want_chunks = max_chunks;
   if (want_chunks < 1) want_chunks = 1;
-  long long rows_per_chunk = round_up((n_rows_pad + want_chunks - 1) / want_chunks, KB);
-  const int n_chunks = (int)((n_rows_pad + rows_per_chunk - 1) / rows_per_chunk);
+  p.rows_per_chunk = round_up((p.n_rows_pad + want_chunks - 1) / want_chunks, KB);
+  p.n_chunks = (int)((p.n_rows_pad + p.rows_per_chunk - 1) / p.rows_per_chunk);
+  return p;
+}
+
+namespace {
+
+// The partial tiles of n_chunks chunks of rows_per_chunk rows of Z (ldz rows per column, zero padded) into pb.part
+int k1_tiles(Problem &pb, const double *Z, int64_t ldz, long long rows_per_chunk, long long n_rows_pad, int n_chunks,
+             int n_tiles, cudaStream_t st, int *launches) {
   const size_t need = (size_t)n_chunks * n_tiles * BT * BT * sizeof(double);
   if (need > pb.part_bytes) {
     if (pb.part) cudaFree(pb.part);
@@ -429,7 +484,7 @@ int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
   dim3 grid(n_tiles, n_chunks);
   const char *impl = getenv("PLS_K1_IMPL");
   CUtensorMap zmap;
-  if (!(impl && strcmp(impl, "v1") == 0) && make_zmap(pb, &zmap)) {
+  if (!(impl && strcmp(impl, "v1") == 0) && make_zmap(Z, ldz, pb.zcols_pad, &zmap)) {
     // pipeline shape.  Measured (profiles/r02_k1_pipe_sweep.txt): deeper rings do not help -- 2 stages of two 16-row
     // boxes per side (64 KB, 3 CTAs per SM) beat 4 x 1, 6 x 1, 8 x 1 and 3 x 2 at every shape: the kernel is bound by
     // DMMA issue, not by load latency.  More, shorter row chunks do help (4 waves).
@@ -438,13 +493,37 @@ int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
     PLS_CUDA_TRY(cudaFuncSetAttribute(k1_gram_tiles_tma<stages, boxes>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k1_gram_tiles_tma<stages, boxes><<<grid, T1B, smem, st>>>(zmap, rows_per_chunk, n_rows_pad, n_tiles, pb.zcols, pb.part);
   } else {
-    k1_gram_tiles<<<grid, T1, 0, st>>>(pb.Z, pb.ldz, rows_per_chunk, n_rows_pad, n_tiles, pb.part);
+    k1_gram_tiles<<<grid, T1, 0, st>>>(Z, ldz, rows_per_chunk, n_rows_pad, n_tiles, pb.part);
   }
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
+  return PLS_OK;
+}
+
+}  // namespace
+
+int k1_gram_build(Problem &pb, cudaStream_t st, int *launches) {
+  NvtxRange nvtx("pls:K1 gram build (TMA + DMMA)");
+  const K1Plan kp = k1_plan(pb.N, pb.zcols_pad);
+  int rc = k1_tiles(pb, pb.Z, pb.ldz, kp.rows_per_chunk, kp.n_rows_pad, kp.n_chunks, kp.n_tiles, st, launches);
+  if (rc) return rc;
   const int zc = pb.zcols;
   const long long tot = (long long)zc * zc;
-  k1_reduce<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(pb.part, n_tiles, n_chunks, zc, pb.S);
+  k1_reduce<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(pb.part, kp.n_tiles, kp.n_chunks, zc, pb.S);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  return PLS_OK;
+}
+
+int k1_gram_build_folds(Problem &pb, const double *Zf, int64_t ldf, long long R, const int *d_chunk0, int F,
+                        double *S_folds, cudaStream_t st, int *launches) {
+  NvtxRange nvtx("pls:K1 gram build (per fold)");
+  const K1Plan kp = k1_plan(pb.N, pb.zcols_pad);
+  int rc = k1_tiles(pb, Zf, ldf, R, ldf, (int)(ldf / R), kp.n_tiles, st, launches);
+  if (rc) return rc;
+  const int zc = pb.zcols;
+  const long long tot = (long long)zc * zc;
+  k1_reduce_folds<<<dim3((unsigned)((tot + 255) / 256), (unsigned)F), 256, 0, st>>>(pb.part, kp.n_tiles, d_chunk0, zc, S_folds);
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   return PLS_OK;
@@ -469,6 +548,18 @@ int k1_gram_finalize_path(const Problem &pb, const double *etas, int L, double *
   PLS_CUDA_TRY(cudaMemsetAsync(scal, 0, sizeof(double) * 4 * L, st));
   k1_finalize_path<<<dim3((unsigned)((tot + 255) / 256), (unsigned)L), 256, 0, st>>>(pb.S, pb.zcols, pb.Mp, etas, pb.gmask,
                                                                                     G, gstride, pb.ldg, c, scal);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  return PLS_OK;
+}
+
+int k1_gram_finalize_folds(const Problem &pb, const double *S_folds, int F, int f, const double *etas, int L, double *G,
+                           size_t gstride, double *c, double *scal, cudaStream_t st, int *launches) {
+  NvtxRange nvtx("pls:K1 gram finalize (training folds)");
+  const long long tot = (long long)pb.ldg * pb.Mp;
+  PLS_CUDA_TRY(cudaMemsetAsync(scal, 0, sizeof(double) * 4 * L, st));
+  k1_finalize_folds<<<dim3((unsigned)((tot + 255) / 256), (unsigned)L), 256, 0, st>>>(S_folds, F, f, pb.zcols, pb.Mp, etas,
+                                                                                     pb.gmask, G, gstride, pb.ldg, c, scal);
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   return PLS_OK;

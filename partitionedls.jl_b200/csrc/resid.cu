@@ -170,6 +170,80 @@ __global__ void __launch_bounds__(T4) k4_rows_multi(const double *__restrict__ Z
   }
 }
 
+// Held-out K4 of cross-validation: k4_rows_multi with blockIdx.y = f on segment f of the fold-contiguous copy Zf (rows
+// [row0[f], row0[f] + rows[f])) against fold f's L vectors Wf + f * L * Mp, partials at outf + f * gridDim.x * 64.  The
+// same tiling and order of sums; a separate copy of the body, so that the eta path's kernel compiles as it did.
+template <int LJ>
+__global__ void __launch_bounds__(T4) k4_rows_folds(const double *__restrict__ Zf, long long ldz,
+                                                    const long long *__restrict__ row0, const long long *__restrict__ rows,
+                                                    int ycol, const double *__restrict__ Wf, int Mp, int L,
+                                                    double *__restrict__ outf) {
+  __shared__ double zs[KM_COLS][KM_ROWS + 1];
+  __shared__ double wsm[KM_COLS][16 * LJ];
+  __shared__ double red[16][16 * LJ];
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;        // vectors tx + 16 j, rows ty + 16 i
+  const int f = blockIdx.y;
+  const double *Z = Zf + row0[f], *W = Wf + (size_t)f * L * Mp;
+  const long long n_rows = rows[f];
+  double *out = outf + (size_t)f * gridDim.x * KM_VEC;
+  double ssq[LJ];
+#pragma unroll
+  for (int j = 0; j < LJ; ++j) ssq[j] = 0.0;
+  const long long n_tiles = (n_rows + KM_ROWS - 1) / KM_ROWS;
+  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const long long r0 = tile * KM_ROWS;
+    double acc[4][LJ];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < LJ; ++j) acc[i][j] = 0.0;
+    for (int c0 = 0; c0 < Mp; c0 += KM_COLS) {
+      for (int e = tid; e < KM_COLS * KM_ROWS; e += T4) {
+        const int cc = e / KM_ROWS, rr = e - cc * KM_ROWS;
+        const long long row = r0 + rr;
+        zs[cc][rr] = (c0 + cc < Mp && row < n_rows) ? Z[(long long)(c0 + cc) * ldz + row] : 0.0;
+      }
+      for (int e = tid; e < KM_COLS * 16 * LJ; e += T4) {
+        const int l = e / KM_COLS, cc = e - l * KM_COLS;
+        wsm[cc][l] = (c0 + cc < Mp && l < L) ? W[(size_t)l * Mp + c0 + cc] : 0.0;
+      }
+      __syncthreads();
+#pragma unroll 8
+      for (int k = 0; k < KM_COLS; ++k) {
+        double a[4], b[LJ];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) a[i] = zs[k][ty + 16 * i];
+#pragma unroll
+        for (int j = 0; j < LJ; ++j) b[j] = wsm[k][tx + 16 * j];
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int j = 0; j < LJ; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const long long row = r0 + ty + 16 * i;
+      if (row < n_rows) {
+        const double yv = Z[(long long)ycol * ldz + row];
+#pragma unroll
+        for (int j = 0; j < LJ; ++j) { const double e = acc[i][j] - yv; ssq[j] = fma(e, e, ssq[j]); }
+      }
+    }
+  }
+  // fixed-order sum of the 16 row groups of each vector
+#pragma unroll
+  for (int j = 0; j < LJ; ++j) red[ty][tx + 16 * j] = ssq[j];
+  __syncthreads();
+  for (int l = tid; l < KM_VEC; l += T4) {
+    double s = 0.0;
+    if (l < 16 * LJ)
+      for (int q = 0; q < 16; ++q) s += red[q][l];
+    out[(size_t)blockIdx.x * KM_VEC + l] = s;
+  }
+}
+
 // out[l] = sum over blocks of part[block * 64 + l], one block per vector, fixed order
 __global__ void k4_sum_parts_multi(const double *__restrict__ part, int n, double *__restrict__ out) {
   __shared__ double sm[256];
@@ -183,6 +257,22 @@ __global__ void k4_sum_parts_multi(const double *__restrict__ part, int n, doubl
     __syncthreads();
   }
   if (threadIdx.x == 0) out[l] = sm[0];
+}
+
+// k4_sum_parts_multi for the F folds of k4_rows_folds: out[f * gridDim.x + l], blockIdx.y = f
+__global__ void k4_sum_parts_folds(const double *__restrict__ part, int n, double *__restrict__ out) {
+  __shared__ double sm[256];
+  const int l = blockIdx.x;
+  part += (size_t)blockIdx.y * n * KM_VEC;
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n; i += 256) s += part[(size_t)i * KM_VEC + l];
+  sm[threadIdx.x] = s;
+  __syncthreads();
+  for (int st = 128; st; st >>= 1) {
+    if (threadIdx.x < st) sm[threadIdx.x] += sm[threadIdx.x + st];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[(size_t)blockIdx.y * gridDim.x + l] = sm[0];
 }
 
 }  // namespace
@@ -241,6 +331,31 @@ int k4_residual_multi(const Problem &pb, SolveWs &ws, const double *d_W, int L, 
   PLS_CUDA_TRY(cudaGetLastError());
   ++*launches;
   return PLS_OK;
+}
+
+int k4_residual_folds(const Problem &pb, const double *Zf, int64_t ldf, const long long *d_row0, const long long *d_nrows,
+                      int F, const double *d_W, int L, int blocks, double *d_part, double *d_ssq, cudaStream_t st,
+                      int *launches) {
+  NvtxRange nvtx("pls:K4 held-out folds");
+  if (L < 1 || L > KM_VEC) { set_error("k4: %d weight vectors (1..%d)", L, KM_VEC); return PLS_EINVAL; }
+  const dim3 grid((unsigned)blocks, (unsigned)F);
+  if (L <= 16) k4_rows_folds<1><<<grid, T4, 0, st>>>(Zf, ldf, d_row0, d_nrows, pb.M + 1, d_W, pb.Mp, L, d_part);
+  else if (L <= 32) k4_rows_folds<2><<<grid, T4, 0, st>>>(Zf, ldf, d_row0, d_nrows, pb.M + 1, d_W, pb.Mp, L, d_part);
+  else k4_rows_folds<4><<<grid, T4, 0, st>>>(Zf, ldf, d_row0, d_nrows, pb.M + 1, d_W, pb.Mp, L, d_part);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  k4_sum_parts_folds<<<dim3((unsigned)L, (unsigned)F), 256, 0, st>>>(d_part, blocks, d_ssq);
+  PLS_CUDA_TRY(cudaGetLastError());
+  ++*launches;
+  return PLS_OK;
+}
+
+// k4_residual_folds' blocks per fold for folds of at most max_rows rows: about four CTAs per SM over all folds
+int k4_folds_blocks(int64_t max_rows, int F, int sm_count) {
+  const long long n_tiles = (max_rows + KM_ROWS - 1) / KM_ROWS;
+  long long cap = (long long)sm_count * 4 / F;
+  if (cap < 1) cap = 1;
+  return (int)(n_tiles < cap ? (n_tiles < 1 ? 1 : n_tiles) : cap);
 }
 
 // d_w: device vector of signed weights (length Mp, intercept last); d_yhat: device vector of round_up(N, 2) doubles.

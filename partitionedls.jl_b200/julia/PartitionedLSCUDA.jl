@@ -26,7 +26,7 @@ using PartitionedLS: PartLSFitResult, Opt, Alt, BnB, cleanupResult, homogeneousC
 using Random
 import PartitionedLS: fit
 
-export OptCUDA, AltCUDA, BnBCUDA, predict_resident, fit_path
+export OptCUDA, AltCUDA, BnBCUDA, predict_resident, fit_path, fit_cv
 
 """Marker types of the GPU solvers: `fit(OptCUDA, X, y, P; η)` is `fit(Opt, X, y, P; η)` on libpls_cuda.so."""
 struct OptCUDA end
@@ -130,6 +130,37 @@ function fit_path(::Type{OptCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray
         push!(out, (model, nothing, (; opt = opt, b = b[l], stats = stats[])))
     end
     return out
+end
+
+"""
+    fit_cv(OptCUDA, X, y, P; η::AbstractVector, folds=5, fold_ids=nothing, rng=Random.default_rng())
+
+K-fold cross-validation of `fit(OptCUDA, X, y, P; η=η[l])` over `η` (1 to 64 values) on one upload of the data
+(`pls_load` + `pls_opt_cv_path`): one K1 pass gives the Gram sums of every fold, each fold's training fits run as
+`fit_path` runs them, one pass over X scores every winner on its held-out fold.  `fold_ids` (N integers in 1:F,
+2 <= F <= 32, no fold empty) defaults to balanced random folds, `randperm(rng, N) .% folds .+ 1`.  Returns
+`(; cv_err, best, η, fold_ids, stats)`: `cv_err[l]` the pooled held-out mean squared error of `η[l]`, `best` the index
+of the lowest (first on ties) and `η` its value.  Refit with `fit(OptCUDA, X, y, P; η=η[best])`.
+"""
+function fit_cv(::Type{OptCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:AbstractFloat,1}, P::Array{Int,2};
+                η::AbstractVector, folds::Integer=5, fold_ids=nothing, rng=Random.default_rng())
+    Xd = convert(Matrix{Float64}, X); yd = convert(Vector{Float64}, y); Pd = convert(Matrix{Int64}, P)
+    N, M = size(Xd); K = size(Pd, 2); L = length(η); etas = convert(Vector{Float64}, η)
+    fid = fold_ids === nothing ? Int32.(randperm(rng, N) .% folds) : Int32.(fold_ids .- 1)   # 0-based for the ABI
+    F = Int64(maximum(fid) + 1)
+    alpha = zeros(Float64, M + 1, F * L); b = zeros(Int64, F * L); obj = zeros(Float64, F * L)
+    ssq = zeros(Float64, F * L); cv = zeros(Float64, L); best = Ref{Int64}(0); stats = Ref{PlsStats}()
+    ctx = context()
+    GC.@preserve Xd yd Pd etas fid alpha b obj ssq cv begin
+        _check(ccall((:pls_load, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, Int64, Int64, Ptr{Cdouble}, Ptr{Int64}, Int64, Cdouble),
+            ctx, Xd, N, N, M, yd, Pd, K, 0.0))
+        _check(ccall((:pls_opt_cv_path, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Int32}, Int64, Ptr{Cdouble}, Int64, UInt32, Ptr{Cdouble}, Ptr{Int64}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ref{Int64}, Ref{PlsStats}),
+            ctx, fid, F, etas, L, UInt32(0), alpha, b, obj, ssq, cv, best, stats))
+    end
+    return (; cv_err = cv, best = best[] + 1, η = etas[best[] + 1], fold_ids = fid .+ 1, stats = stats[])
 end
 
 """
