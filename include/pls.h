@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PLS_VERSION 120 /* 0.1.2: pls_opt_cv_path */
+#define PLS_VERSION 130 /* 0.1.3: pls_bnb_fit_path */
 
 enum {
   PLS_OK = 0,
@@ -171,6 +171,27 @@ int pls_opt_fit_resident(pls_ctx *ctx, uint32_t flags, double *alpha_raw, int64_
  * The context's own eta, G and c are not changed.  M + 1 > 1024: PLS_EUNSUPPORTED (fit each eta on its own). */
 int pls_opt_fit_path(pls_ctx *ctx, const double *etas, int64_t L, uint32_t flags, double *alpha_raw, int64_t *b_best,
                      double *obj_best, pls_stats *stats);
+
+/* ---- regularisation path of fit(BnB) on the resident data set (one-GPU context) ------------------------------------
+ * Result l is what pls_load(..., eta = etas[l]) followed by pls_bnb_fit_resident(ctx, flags, ...) returns: the same
+ * optimum and signed weights (within rounding: nopen and the last bits of the weights depend on the traversal, as they
+ * do for one fit).  S = Z'Z is built once (not at all when the context's Gram matrix is already finalised) and G_l =
+ * S + eta_l Po Po' is formed for every eta in one launch; the L searches then share every frontier wave (one K5 launch
+ * per wave carries the nodes of all unfinished searches), each with its own incumbent, open list and an equal share of
+ * the state pool.  One K4 pass over X evaluates all L winners.
+ *   etas[L]                 1 <= L <= 64, each finite and >= 0, any order, duplicates allowed
+ *   alpha_signed[(M+1) x L] column l = signed weights of eta_l's best feasible leaf, intercept last
+ *   obj[L], nopen[L]        as in pls_bnb_fit, per eta
+ *   flags                   PLS_FLAG_NO_RECOMPUTE as for pls_bnb_fit_resident
+ *   stats                   of the whole call (ms_gram: K1 + the batched finalise, ms_nnls: the waves and the leaf
+ *                           selection, ms_recompute: the K4 pass; orthants = sum of nopen, waves: waves of the call,
+ *                           max_open: the largest total number of open nodes)
+ * PLS_BNB_MAX_NODES bounds every search on its own; PLS_BNB_SLOTS sets the total pool.  The context's own eta, G, c and
+ * gram_ready are not changed.  Refused: PLS_EINVAL for a null pointer, no data loaded, L out of range or a bad eta;
+ * PLS_EUNSUPPORTED for M' > 1024 or a multi-GPU context; PLS_ENOMEM when the pool cannot give every eta the K' + 3
+ * slots a root needs; PLS_ENUMERIC (naming the eta) for a relaxation that did not converge or a non-finite Gram matrix. */
+int pls_bnb_fit_path(pls_ctx *ctx, const double *etas, int64_t L, uint32_t flags, double *alpha_signed, double *obj,
+                     int64_t *nopen, pls_stats *stats);
 
 /* ---- K-fold cross-validation of fit(Opt) over a grid of eta on the resident data set (one-GPU context) -------------
  * One K1 pass over a fold-contiguous copy of the loaded rows gives the raw Gram sums S_f of every fold; the training

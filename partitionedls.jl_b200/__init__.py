@@ -174,22 +174,32 @@ def fit(alg, X, y, P, *, η=0.0, eta=None, nnlsalg="nnls", returnAllSolutions=Fa
 
 
 def fit_path(alg, X, y, P, etas, *, ctx=None, **flags):
-    """fit(Opt, X, y, P; η=η_l) for every η_l in `etas` (1..64 values, any order, duplicates allowed) on one resident
-    copy of the data: one Gram build, the orthant solves of all η in as few launches as the kernel choice allows, and
-    one pass over X for all winners (pls_opt_fit_path).  Returns a list with one entry per η, each what
-    fit(Opt, X, y, P; η=η_l) returns: (PartLSFitResult, None, report) with report.opt, report.b and the call's shared
-    stats.  Keyword flags: enumerate_intercept, no_recompute (as PLS_FLAG_*)."""
-    if not (alg is Opt or isinstance(alg, Opt)):
-        raise TypeError(f"fit_path supports Opt only, not {alg!r}")
-    unknown = set(flags) - {"enumerate_intercept", "no_recompute"}
+    """fit(alg, X, y, P; η=η_l) for every η_l in `etas` (1..64 values, any order, duplicates allowed) on one resident
+    copy of the data.  Returns a list with one entry per η, each what fit(alg, X, y, P; η=η_l) returns.
+
+    Opt (pls_opt_fit_path): one Gram build, the orthant solves of all η in as few launches as the kernel choice allows,
+    and one pass over X for all winners; report.opt, report.b and the call's shared stats.  Keyword flags:
+    enumerate_intercept, no_recompute (as PLS_FLAG_*).
+    BnB (pls_bnb_fit_path): one Gram build, the searches of all η in the same frontier waves, and one pass over X for all
+    winners; each model is cleaned as fit(BnB) cleans it, report.opt, report.nopen and the call's shared stats.  Keyword
+    flag: no_recompute."""
+    is_opt, is_bnb = alg is Opt or isinstance(alg, Opt), alg is BnB or isinstance(alg, BnB)
+    if not (is_opt or is_bnb):
+        raise TypeError(f"fit_path supports Opt and BnB only, not {alg!r}")
+    unknown = set(flags) - ({"enumerate_intercept", "no_recompute"} if is_opt else {"no_recompute"})
     if unknown:
-        raise TypeError(f"unknown keyword(s) {sorted(unknown)}")
+        raise TypeError(f"unknown keyword(s) {sorted(unknown)}" + ("" if is_opt else " for BnB"))
     fl = (_abi.PLS_FLAG_ENUMERATE_INTERCEPT if flags.get("enumerate_intercept") else 0) | \
          (_abi.PLS_FLAG_NO_RECOMPUTE if flags.get("no_recompute") else 0)
     c = ctx or default_context()
     c.load(X, y, P)
-    res, stats = c.opt_fit_path(etas, flags=fl)
     out = []
+    if is_bnb:
+        res, stats = c.bnb_fit_path(etas, flags=fl)
+        for r in res:
+            out.append((_bnb_postprocess(r["alpha_signed"], P), None, SimpleNamespace(opt=r["opt"], nopen=r["nopen"], stats=stats)))
+        return out
+    res, stats = c.opt_fit_path(etas, flags=fl)
     for r in res:
         opt, model = _cleanup_result(r["opt"], r["alpha_raw"], r["b_best"], P)
         out.append((model, None, SimpleNamespace(opt=opt, b=r["b_best"], stats=stats)))

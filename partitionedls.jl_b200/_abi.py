@@ -81,6 +81,7 @@ lib.pls_bnb_lower_bounds.argtypes = [_vp, C.POINTER(C.c_uint64), C.POINTER(C.c_u
 lib.pls_gram.argtypes = [_vp, _dp, C.c_int64, C.c_int64, _dp, _ip, C.c_int64, C.c_double, _dp, _dp, _dp]
 lib.pls_opt_fit_path.argtypes = [_vp, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, C.POINTER(PlsStats)]
 lib.pls_residual_partial_multi.argtypes = [_vp, _dp, C.c_int64, _dp]
+lib.pls_bnb_fit_path.argtypes = [_vp, _dp, C.c_int64, C.c_uint32, _dp, _dp, _ip, C.POINTER(PlsStats)]
 _i32p = C.POINTER(C.c_int32)
 lib.pls_opt_cv_path.argtypes = [_vp, _i32p, C.c_int64, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, _dp, _dp, _ip,
                                 C.POINTER(PlsStats)]
@@ -90,7 +91,7 @@ lib.pls_nnls_batch.argtypes = [_vp, _dp, _dp, C.c_double, C.c_int64, C.POINTER(C
 for _n in ("pls_create", "pls_opt_fit", "pls_bnb_fit", "pls_bnb_fit_resident", "pls_alt_fit", "pls_alt_fit_resident", "pls_residual_partial_w", "pls_predict_resident", "pls_objective_finish_w", "pls_load", "pls_opt_fit_resident", "pls_gram_build", "pls_gram_raw",
            "pls_gram_finalize", "pls_opt_solve_range", "pls_opt_solve_pairs", "pls_opt_residual_partial", "pls_opt_objective_finish",
            "pls_get_stats", "pls_gram_scalars", "pls_bnb_lower_bounds", "pls_gram", "pls_nnls_batch", "pls_opt_fit_path",
-           "pls_residual_partial_multi", "pls_opt_cv_path", "pls_cv_fold_sums"):
+           "pls_residual_partial_multi", "pls_opt_cv_path", "pls_cv_fold_sums", "pls_bnb_fit_path"):
     getattr(lib, _n).restype = C.c_int
 
 
@@ -229,6 +230,16 @@ class Context:
         alpha = np.zeros((L, M + 1)); b = np.zeros(L, dtype=np.int64); obj = np.zeros(L); st = PlsStats()
         _check(lib.pls_opt_fit_path(self._h, _d(e), L, flags, _d(alpha), b.ctypes.data_as(_ip), _d(obj), C.byref(st)))
         return [dict(alpha_raw=alpha[l], b_best=int(b[l]), opt=float(obj[l])) for l in range(L)], st.as_dict()
+
+    def bnb_fit_path(self, etas, flags=0):
+        """pls_bnb_fit_path: fit(BnB) for every eta in `etas` (1..64 values) on the resident data set, all searches in the
+        same frontier waves.  Returns one dict per eta (alpha_signed, opt, nopen) and the call's shared stats."""
+        N, M, K = self._shape
+        e = np.ascontiguousarray(np.asarray(etas, dtype=np.float64).reshape(-1))
+        L = len(e)
+        a = np.zeros((L, M + 1)); obj = np.zeros(L); nopen = np.zeros(L, dtype=np.int64); st = PlsStats()
+        _check(lib.pls_bnb_fit_path(self._h, _d(e), L, flags, _d(a), _d(obj), nopen.ctypes.data_as(_ip), C.byref(st)))
+        return [dict(alpha_signed=a[l], opt=float(obj[l]), nopen=int(nopen[l])) for l in range(L)], st.as_dict()
 
     def _fold_ids(self, fold_id):
         f = np.ascontiguousarray(np.asarray(fold_id).reshape(-1), dtype=np.int32)

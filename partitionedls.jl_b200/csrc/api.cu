@@ -314,9 +314,9 @@ double eta_term(const pls_ctx *c, double eta, const double *alpha_raw, int64_t b
 }
 
 // the eta rows for signed weights w (BnB / Alt): eta * sum_k (sum_{m in k} w_m)^2
-double eta_term_w(const pls_ctx *c, const double *w) {
+double eta_term_w(const pls_ctx *c, double eta, const double *w) {
   const Problem &pb = c->pb;
-  if (pb.eta == 0.0) return 0.0;
+  if (eta == 0.0) return 0.0;
   double tot = 0.0;
   for (int k = 0; k < pb.Kp; ++k) {
     double s = 0.0;
@@ -324,7 +324,7 @@ double eta_term_w(const pls_ctx *c, const double *w) {
       if (c->h_gmask[m] >> k & 1ull) s += w[m];
     tot += s * s;
   }
-  return pb.eta * tot;
+  return eta * tot;
 }
 
 // K4 on the loaded rows for explicit signed weights w
@@ -865,7 +865,7 @@ int pls_predict_resident(pls_ctx *c, const double *w, double *yhat) {
 
 int pls_objective_finish_w(pls_ctx *c, const double *w, double ssq_total, double *obj_out) {
   if (!c || !w || !obj_out) { set_error("null pointer"); return PLS_EINVAL; }
-  *obj_out = std::sqrt(ssq_total + eta_term_w(c, w));
+  *obj_out = std::sqrt(ssq_total + eta_term_w(c, c->pb.eta, w));
   return PLS_OK;
 }
 
@@ -1020,7 +1020,7 @@ int pls_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, doubl
   if (c->pin_b() < 0) { set_error("bnb: no feasible leaf found"); return PLS_ENUMERIC; }
   memcpy(alpha_signed, c->h_pin, sizeof(double) * Mp);
   double obj = c->pin_obj();
-  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term_w(c, alpha_signed));
+  if (recompute && obj == obj) obj = std::sqrt(*c->pin_ssq() + eta_term_w(c, pb.eta, alpha_signed));
   *obj_out = obj;
   *nopen = rep.visited;
   float ms = 0.f;
@@ -1046,6 +1046,77 @@ int pls_bnb_fit(pls_ctx *c, const double *X, int64_t N, int64_t M, const double 
   rc = pls_bnb_fit_resident(c, flags, alpha_signed, obj, nopen, stats);
   c->stats.ms_upload = 0.0;
   return rc;
+}
+
+int pls_bnb_fit_path(pls_ctx *c, const double *etas, int64_t L, uint32_t flags, double *alpha_signed, double *obj,
+                     int64_t *nopen, pls_stats *stats) {
+  if (!c) { set_error("null context"); return PLS_EINVAL; }
+  if (!c->pb.loaded) { set_error("no data set loaded"); return PLS_EINVAL; }
+  if (!etas || !alpha_signed || !obj || !nopen) { set_error("null pointer"); return PLS_EINVAL; }
+  if (L < 1 || L > 64) { set_error("L = %lld eta values (1..64)", (long long)L); return PLS_EINVAL; }
+  for (int64_t l = 0; l < L; ++l)
+    if (!(etas[l] >= 0.0) || !std::isfinite(etas[l])) { set_error("eta[%lld] must be finite and >= 0", (long long)l); return PLS_EINVAL; }
+  if (!c->subs.empty()) { set_error("bnb path: a multi-GPU context is not supported (fit each eta on its own)"); return PLS_EUNSUPPORTED; }
+  int rc = check_ctx(c);
+  if (rc) return rc;
+  Problem &pb = c->pb;
+  const int Mp = pb.Mp, rl = record_len(Mp), n = (int)L;
+  if (Mp > 1024) { set_error("bnb: M' = %d exceeds this build's limit (1024)", Mp); return PLS_EUNSUPPORTED; }
+  const FitMark fm = fit_start(c);
+  cudaStream_t st = c->stream;
+  // the L systems G_l = S + eta_l Po Po' (S built first unless the context's Gram matrix is already finalised)
+  PathWs p;
+  rc = path_ws(c, n, &p);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaMemcpyAsync(p.etas, etas, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  if (!pb.gram_ready) { rc = k1_gram_build(pb, st, &c->launches); if (rc) return rc; }
+  rc = k1_gram_finalize_path(pb, p.etas, n, p.G, p.gstride, p.c, p.scal, st, &c->launches);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[1], st));
+  rc = path_check_formed(c, p, etas, n);
+  if (rc) return rc;
+  // every search in the same waves, the winners in records 0..L-1 of ws.win
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[2], st));
+  BnbSystems sys;
+  sys.G = p.G; sys.gstride = p.gstride; sys.c = p.c; sys.scal = p.scal; sys.L = n; sys.etas = etas;
+  BnbReport rep;
+  rc = k5_bnb_run(pb, c->ws, c->sm_count, st, &c->launches, &rep, nullptr, &sys);
+  if (rc) return rc;
+  PLS_CUDA_TRY(cudaEventRecord(c->ev[3], st));
+  std::vector<double> rec((size_t)n * rl), ssq((size_t)n, 0.0), W((size_t)n * Mp);
+  std::vector<unsigned long long> cnt(CNT_BLOCK_LEN);
+  PLS_CUDA_TRY(cudaMemcpyAsync(rec.data(), c->ws.win, sizeof(double) * rec.size(), cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaMemcpyAsync(cnt.data(), c->ws.counters, sizeof(unsigned long long) * CNT_BLOCK_LEN, cudaMemcpyDeviceToHost, st));
+  PLS_CUDA_TRY(cudaStreamSynchronize(st));
+  float ms_gram = 0.f, ms_nnls = 0.f;
+  cudaEventElapsedTime(&ms_gram, c->ev[0], c->ev[1]);
+  cudaEventElapsedTime(&ms_nnls, c->ev[2], c->ev[3]);
+  for (int l = 0; l < n; ++l) {
+    if (record_b(rec.data() + (size_t)l * rl, Mp) < 0) { set_error("bnb: no feasible leaf found (eta = %g)", etas[l]); return PLS_ENUMERIC; }
+    memcpy(W.data() + (size_t)l * Mp, rec.data() + (size_t)l * rl, sizeof(double) * Mp);
+  }
+  // the data-space sums of all winners in one pass over X (timed into c->stats.ms_recompute)
+  const bool recompute = !(flags & PLS_FLAG_NO_RECOMPUTE);
+  if (recompute) { rc = residual_partial_multi(c, W.data(), n, ssq.data()); if (rc) return rc; }
+  bool nan = false;
+  for (int l = 0; l < n; ++l) {
+    const double *w = W.data() + (size_t)l * Mp;
+    memcpy(alpha_signed + (size_t)l * Mp, w, sizeof(double) * Mp);
+    double o = rec[(size_t)l * rl + Mp];
+    if (recompute && o == o) o = std::sqrt(ssq[l] + eta_term_w(c, etas[l], w));
+    obj[l] = o;
+    nopen[l] = rep.nopen[l];
+    nan |= o != o;
+  }
+  pls_stats &s = c->stats;
+  read_counters(c, cnt.data());
+  s.spills = 0;
+  s.ms_gram = ms_gram; s.ms_nnls = ms_nnls;
+  s.orthants = rep.visited; s.waves = rep.waves; s.max_open = rep.max_open;
+  fit_finish(c, fm, stats);
+  if (nan) { set_error("NaN objective (non-finite input?)"); return PLS_ENUMERIC; }
+  return PLS_OK;
 }
 
 int pls_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps, int64_t T, uint32_t flags,
@@ -1092,7 +1163,7 @@ int pls_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double eps,
   memcpy(alpha, h.data(), sizeof(double) * Mp);
   memcpy(beta, h.data() + Mp, sizeof(double) * Kp);
   double obj = h[len];
-  if (recompute) obj = std::sqrt(h[len + 2 + Mp] + eta_term_w(c, h.data() + len + 2));
+  if (recompute) obj = std::sqrt(h[len + 2 + Mp] + eta_term_w(c, pb.eta, h.data() + len + 2));
   *obj_out = obj;
   if (best_restart) *best_restart = rbest;
   if (iters) *iters = (int64_t)h[Mp + Kp];

@@ -18,6 +18,11 @@
 // wave.  The incumbent mu is a device double updated with atomicMin by every leaf, so a positive
 // child's leaf already prunes its sibling.  The optimum does not depend on the traversal order;
 // the number of visited nodes (`nopen`) does, and is reported for this traversal.
+//
+// Several searches per run (an eta path): L <= 64 searches on L Gram systems of one shape share every wave.  An item
+// names its search l; node l solves G + l * gstride with the scalars at scal + 4 l (c is shared), prunes against its own
+// incumbent mu[l] and keeps its best leaf in its own per-CTA slot.  The host keeps one open list, pool quota and node
+// budget per search and concatenates the items every search would take into one launch.  A fit is the case L = 1.
 #include <string.h>
 #include <algorithm>
 #include <cmath>
@@ -34,7 +39,7 @@ struct BnbItem {
   int parent_slot;          // state to expand (-1: root, start from the empty state)
   int spare_slot;           // free slot for the positive child's state
   int k;                    // branching group (-1: root)
-  int pad;
+  int l;                    // search (system) index
   unsigned long long pos_mask, neg_mask;   // groups already fixed to + / -
 };
 struct BnbChild {
@@ -46,16 +51,17 @@ struct BnbChild {
 };
 
 struct BnbArgs {
-  const double *G; int ldg;
-  const double *c;
-  const double *scal;
+  const double *G; int ldg; size_t gstride;    // system l: G + l * gstride
+  const double *c;                             // shared by every system
+  const double *scal;                          // system l: scal + 4 l
   const uint64_t *gmask;
   int Mp, Kp, cap;
   double *pool; size_t slot_stride; size_t htile_doubles;
   const BnbItem *items; int n_items;
   unsigned long long *item_counter;
-  double *mu;                                  // incumbent (device, atomicMin on the bit pattern)
-  double *cta_obj; long long *cta_b; double *cta_w;   // per-CTA best leaf (persist across waves)
+  double *mu;                                  // [L] incumbents (device, atomicMin on the bit pattern)
+  int max_grid;                                // per-CTA best leaf of search l at slot l * max_grid + CTA:
+  double *cta_obj; long long *cta_b; double *cta_w;   // (persist across waves)
   unsigned long long *leaf_seq;                // global leaf counter: lower = found earlier
   BnbChild *out;                               // [n_items][2]
   unsigned long long *counters;
@@ -126,14 +132,10 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
   if (tid == 0)
     for (int i = 0; i < ST_NUM; ++i) s.stat[i] = 0;
-  const double yy = A.scal[0], cmax = A.scal[1];
-  double best_obj = A.cta_obj[blockIdx.x];
-  long long best_seq = A.cta_b[blockIdx.x];
   long long n_solved = 0;
   __shared__ unsigned long long s_item;
-  __shared__ int s_nextk, s_feas;
+  __shared__ int s_nextk, s_feas, s_better;
   __shared__ double s_mu;
-  __shared__ unsigned long long s_seq;
   double *nu = s.Spart;                        // [Kp <= 64] scratch between solves
   __syncthreads();
 
@@ -145,6 +147,9 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
     if (it >= (unsigned long long)A.n_items) break;
     const BnbItem item = A.items[it];
     const bool root = item.k < 0;
+    const double *G = A.G + (size_t)item.l * A.gstride;
+    const double yy = A.scal[4 * item.l], cmax = A.scal[4 * item.l + 1];
+    double *mu = A.mu + item.l;
     double *home = A.pool + (size_t)(root ? item.spare_slot : item.parent_slot) * A.slot_stride;
     cf.hg = home;
     s = make_sh3(cf);
@@ -168,7 +173,7 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
         s.vflag[m] = 0;
       }
       __syncthreads();
-      bool ok = bpp_solve3<T, 1>(cf, s, A.G, A.ldg, Mp, cmax, st);
+      bool ok = bpp_solve3<T, 1>(cf, s, G, A.ldg, Mp, cmax, st);
       if (!ok) {
         // block pivoting stalled on a nearly singular intermediate passive set (lower_bound, BnB.jl:69-92, always
         // returns): solve this node again from the empty passive set, one variable per step behind the pivot test
@@ -176,7 +181,7 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
         st.nt_dirty = 0; st.hwm = 0; st.nt_cur = 0; st.r_valid = true;
         for (int m = tid; m < cap; m += T) { s.w[m] = 0.0; s.r[m] = s.cs[m]; s.pos[m] = -1; s.vflag[m] = 0; }
         __syncthreads();
-        ok = bpp_solve3<T, 1>(cf, s, A.G, A.ldg, Mp, cmax, st, true);
+        ok = bpp_solve3<T, 1>(cf, s, G, A.ldg, Mp, cmax, st, true);
         STAT_ADD3(ST_REBUILD, 1);
         if (!ok) STAT_ADD3(ST_NOCONV, 1);
       }
@@ -200,7 +205,7 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
         int bk = 0; double bv = nu[0]; bool feas = nu[0] == 0.0;
         for (int k = 1; k < Kp; ++k) { if (nu[k] > bv) { bv = nu[k]; bk = k; } feas = feas && nu[k] == 0.0; }
         s_nextk = bk; s_feas = feas ? 1 : 0;
-        s_mu = *reinterpret_cast<volatile double *>(A.mu);   // one read, broadcast: the status must be uniform
+        s_mu = *reinterpret_cast<volatile double *>(mu);     // one read, broadcast: the status must be uniform
       }
       __syncthreads();
       const double mu_now = s_mu;
@@ -211,13 +216,18 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
       else status = 2;
       int child_slot = -1;
       if (status == 1) {
-        if (tid == 0) { atomic_min_nonneg(A.mu, lb); s_seq = atomicAdd(A.leaf_seq, 1ull); }
-        __syncthreads();
-        const long long seq = (long long)s_seq;
-        if (best_seq < 0 || lb < best_obj) {
-          best_obj = lb; best_seq = seq;
-          for (int m = tid; m < Mp; m += T) A.cta_w[(size_t)blockIdx.x * Mp + m] = s.pos[m] >= 0 ? s.w[m] : 0.0;
+        // this CTA's best leaf of search l so far: only this CTA writes the slot, so it reads back what it wrote
+        const size_t bslot = (size_t)item.l * A.max_grid + blockIdx.x;
+        if (tid == 0) {
+          atomic_min_nonneg(mu, lb);
+          const long long seq = (long long)atomicAdd(A.leaf_seq, 1ull);
+          const long long bseq = A.cta_b[bslot];
+          s_better = bseq < 0 || lb < A.cta_obj[bslot];
+          if (s_better) { A.cta_obj[bslot] = lb; A.cta_b[bslot] = seq; }
         }
+        __syncthreads();
+        if (s_better)
+          for (int m = tid; m < Mp; m += T) A.cta_w[bslot * Mp + m] = s.pos[m] >= 0 ? s.w[m] : 0.0;
       } else if (status == 2) {
         if (root || ch == 1) {                          // the state stays where it is
           child_slot = root ? item.spare_slot : item.parent_slot;
@@ -237,8 +247,6 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
     }
   }
   if (tid == 0) {
-    A.cta_obj[blockIdx.x] = best_obj;
-    A.cta_b[blockIdx.x] = best_seq;
     atomicAdd(&A.counters[CNT_PIVOTS], (unsigned long long)s.stat[ST_PIV]);
     atomicAdd(&A.counters[CNT_GRAD], (unsigned long long)s.stat[ST_GRAD]);
     atomicAdd(&A.counters[CNT_SUMP], (unsigned long long)s.stat[ST_SUMP]);
@@ -251,13 +259,16 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
   }
 }
 
-// lexicographic (objective, leaf sequence) minimum over the per-CTA best leaves
+// lexicographic (objective, leaf sequence) minimum over the per-CTA best leaves; block l: search l's n slots into
+// record l of win
 __global__ void __launch_bounds__(256) k5_select_leaf(const double *cta_obj, const long long *cta_b, const double *cta_w,
                                                       int n, int Mp, double *win) {
   __shared__ double so[256];
   __shared__ long long sb[256];
   __shared__ int si[256];
   const int tid = threadIdx.x;
+  cta_obj += (size_t)blockIdx.x * n; cta_b += (size_t)blockIdx.x * n; cta_w += (size_t)blockIdx.x * n * Mp;
+  win += (size_t)blockIdx.x * (Mp + 2);
   double o = 0.0; long long b = -1; int idx = -1;
   for (int i = tid; i < n; i += 256)
     if (lex_better(cta_obj[i], cta_b[i], o, b)) { o = cta_obj[i]; b = cta_b[i]; idx = i; }
@@ -282,12 +293,23 @@ struct OpenNode {
 
 }  // namespace
 
-// Host driver.  Leaves the winner (signed weights, objective, leaf sequence) in ws.win.
+// Host driver.  Leaves the winner of search l (signed weights, objective, leaf sequence) in record l of ws.win
+// (record_len(M') doubles each).  sys: the systems to search (null: the context's own, one search).
 int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, int *launches, BnbReport *rep,
-               BnbShard *shard) {
+               BnbShard *shard, const BnbSystems *sys) {
   NvtxRange nvtx("pls:K5 BnB frontier waves");
   std::atomic<unsigned long long> *shared_mu = shard ? shard->shared_mu : nullptr;
   const int Mp = pb.Mp, Kp = pb.Kp;
+  const int L = sys ? sys->L : 1;
+  if (L < 1 || L > 64) { set_error("bnb: %d searches (1..64)", L); return PLS_EINVAL; }
+  if (shard && L > 1) { set_error("bnb: a sharded search runs on one system"); return PLS_EINVAL; }
+  // names the system of search l in error messages, when there are several
+  char who_buf[64];
+  auto who = [&](int l) -> const char * {
+    who_buf[0] = 0;
+    if (sys && sys->etas) snprintf(who_buf, sizeof(who_buf), " (eta = %g)", sys->etas[l]);
+    return who_buf;
+  };
   if (Mp > CAP3MAX) { set_error("bnb: M' = %d exceeds this build's limit (%d)", Mp, CAP3MAX); return PLS_EUNSUPPORTED; }
   if (Kp > 64) { set_error("bnb: more than 63 groups"); return PLS_EUNSUPPORTED; }
   const int cap = (Mp + 7) & ~7;
@@ -309,86 +331,103 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
   int launch_grid = max_grid;                  // per-CTA bests (cta_*) stay sized and scanned by max_grid
   if (const char *eg = getenv("PLS_BNB_GRID")) { const int g = atoi(eg); if (g >= 1 && g < max_grid) launch_grid = g; }   // tests: several nodes per CTA
 
-  // state pool: a bounded share of the free memory
+  // state pool: a bounded share of the free memory, split into L equal quotas (search l owns slots [l q, (l + 1) q))
   size_t free_b = 0, total_b = 0;
   PLS_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
   const size_t slot_bytes = slot_doubles * sizeof(double);
   size_t n_slots = (size_t)(0.5 * (double)free_b) / slot_bytes;
-  if (n_slots > 65536) n_slots = 65536;
+  if (n_slots > 65536 * (size_t)L) n_slots = 65536 * (size_t)L;
   if (shard && shard->stop_open > 0) n_slots = std::min<size_t>(n_slots, std::max<size_t>(2048, 16 * (size_t)shard->stop_open));   // frontier seeding pass: small pool
   if (const char *e = getenv("PLS_BNB_SLOTS")) n_slots = (size_t)atoll(e);
+  const size_t quota = n_slots / (size_t)L;
   // the first wave takes a root only while more than K' + 2 slots are free: a smaller pool would launch an empty wave
-  if (n_slots < (size_t)Kp + 3) { set_error("bnb: state pool of %zu slots is too small (a root needs K + 4 = %d)", n_slots, Kp + 3); return PLS_ENOMEM; }
-  const int wave_max = (int)std::min<size_t>((size_t)max_grid * 2, n_slots / 2);
+  if (quota < (size_t)Kp + 3) {
+    if (L == 1) set_error("bnb: state pool of %zu slots is too small (a root needs K + 4 = %d)", n_slots, Kp + 3);
+    else set_error("bnb: state pool of %zu slots is too small for %d searches (a root needs K + 4 = %d each)", n_slots, L, Kp + 3);
+    return PLS_ENOMEM;
+  }
+  n_slots = quota * (size_t)L;
+  const int wave_max = (int)std::min<size_t>((size_t)max_grid * 2, quota / 2);    // items per search and wave
 
+  struct Search {
+    std::vector<OpenNode> open;
+    std::vector<int> free_slots;
+    std::vector<BnbItem> pending;              // roots not started yet
+    long long visited = 0;
+    bool done = false;
+  };
   double *pool = nullptr, *mu = nullptr, *d_probe = nullptr;
   BnbItem *d_items = nullptr; BnbChild *d_out = nullptr;
   unsigned long long *d_ctr = nullptr;
   int rc = PLS_OK;
   std::vector<BnbItem> items; std::vector<BnbChild> out;
-  std::vector<OpenNode> open; std::vector<int> free_slots;
-  std::vector<BnbItem> pending;
-  long long visited = 0, waves = 0, max_open = 0;
+  std::vector<Search> srch(L);
+  long long waves = 0, max_open = 0;
   bool complete = true;
   const long long max_nodes = getenv("PLS_BNB_MAX_NODES") ? atoll(getenv("PLS_BNB_MAX_NODES")) : 0;
-  double h_mu = INFINITY;
+  std::vector<double> h_mu(L, INFINITY);
   const unsigned long long inf_bits = 0x7ff0000000000000ull;
+  const size_t n_win = (size_t)L * max_grid;   // per-CTA best leaves, [L][max_grid]
 #define BNB_TRY(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); rc = e_ == cudaErrorMemoryAllocation ? PLS_ENOMEM : PLS_ECUDA; goto done; } } while (0)
   BNB_TRY(cudaMalloc(&pool, n_slots * slot_bytes));
-  BNB_TRY(cudaMalloc(&mu, sizeof(double)));
-  BNB_TRY(cudaMalloc(&d_items, sizeof(BnbItem) * wave_max));
-  BNB_TRY(cudaMalloc(&d_out, sizeof(BnbChild) * 2 * wave_max));
+  BNB_TRY(cudaMalloc(&mu, sizeof(double) * L));
+  BNB_TRY(cudaMalloc(&d_items, sizeof(BnbItem) * (size_t)L * wave_max));
+  BNB_TRY(cudaMalloc(&d_out, sizeof(BnbChild) * 2 * (size_t)L * wave_max));
   BNB_TRY(cudaMalloc(&d_ctr, sizeof(unsigned long long) * 2));
   {
     // start from the incumbent other devices / an earlier pass already hold
     const unsigned long long start_bits = shared_mu ? std::min(shared_mu->load(), inf_bits) : inf_bits;
-    memcpy(&h_mu, &start_bits, sizeof(double));
-    BNB_TRY(cudaMemcpyAsync(mu, &h_mu, sizeof(double), cudaMemcpyHostToDevice, st));
+    memcpy(&h_mu[0], &start_bits, sizeof(double));
+    BNB_TRY(cudaMemcpyAsync(mu, h_mu.data(), sizeof(double) * L, cudaMemcpyHostToDevice, st));
     BNB_TRY(cudaStreamSynchronize(st));
   }
-  if (max_grid > ws.max_ctas || Mp != ws.Mp) {
+  if (n_win > (size_t)ws.max_ctas || Mp != ws.Mp) {
     cudaFree(ws.cta_obj); cudaFree(ws.cta_b); cudaFree(ws.cta_w);
     ws.cta_obj = nullptr; ws.cta_b = nullptr; ws.cta_w = nullptr; ws.max_ctas = 0;
-    BNB_TRY(cudaMalloc(&ws.cta_obj, sizeof(double) * max_grid));
-    BNB_TRY(cudaMalloc(&ws.cta_b, sizeof(long long) * max_grid));
-    BNB_TRY(cudaMalloc(&ws.cta_w, sizeof(double) * (size_t)max_grid * Mp));
-    ws.max_ctas = max_grid; ws.Mp = Mp;
+    BNB_TRY(cudaMalloc(&ws.cta_obj, sizeof(double) * n_win));
+    BNB_TRY(cudaMalloc(&ws.cta_b, sizeof(long long) * n_win));
+    BNB_TRY(cudaMalloc(&ws.cta_w, sizeof(double) * n_win * Mp));
+    ws.max_ctas = (int)n_win; ws.Mp = Mp;
   }
   BNB_TRY(ensure_counters(ws, true, st));
-  BNB_TRY(ensure_win(ws, Mp + 2));
-  BNB_TRY(cudaMemsetAsync(ws.cta_obj, 0, sizeof(double) * max_grid, st));
-  BNB_TRY(cudaMemsetAsync(ws.cta_b, 0xff, sizeof(long long) * max_grid, st));     // -1: no leaf yet
+  BNB_TRY(ensure_win(ws, L * (Mp + 2)));
+  BNB_TRY(cudaMemsetAsync(ws.cta_obj, 0, sizeof(double) * n_win, st));
+  BNB_TRY(cudaMemsetAsync(ws.cta_b, 0xff, sizeof(long long) * n_win, st));     // -1: no leaf yet
   BNB_TRY(cudaMemsetAsync(d_ctr, 0, sizeof(unsigned long long) * 2, st));
 
-  items.reserve(wave_max); out.resize((size_t)2 * wave_max);
-  free_slots.reserve(n_slots);
-  for (size_t i = n_slots; i-- > 1;) free_slots.push_back((int)i);
-  {
+  items.reserve((size_t)L * wave_max); out.resize((size_t)2 * L * wave_max);
+  for (int l = 0; l < L; ++l) {
     // first wave: the root(s), solved cold.  More roots than one wave holds wait in `pending`.
+    Search &S = srch[l];
+    const int base = (int)(l * quota);
+    S.free_slots.reserve(quota);
+    for (size_t i = quota; i-- > 1;) S.free_slots.push_back(base + (int)i);
     const size_t n_roots = shard && !shard->root_pos.empty() ? shard->root_pos.size() : 1;
     for (size_t i = 0; i < n_roots; ++i) {
-      BnbItem r; r.parent_slot = -1; r.spare_slot = -1; r.k = -1; r.pad = 0;
+      BnbItem r; r.parent_slot = -1; r.spare_slot = -1; r.k = -1; r.l = l;
       r.pos_mask = shard && !shard->root_pos.empty() ? shard->root_pos[i] : 0ull;
       r.neg_mask = shard && !shard->root_pos.empty() ? shard->root_neg[i] : 0ull;
-      pending.push_back(r);
+      S.pending.push_back(r);
     }
-    free_slots.push_back(0);
-    while (!pending.empty() && (int)items.size() < wave_max && free_slots.size() > (size_t)(Kp + 2)) {
-      BnbItem r = pending.back(); pending.pop_back();
-      r.spare_slot = free_slots.back(); free_slots.pop_back();
-      items.push_back(r);
+    S.free_slots.push_back(base);
+    int taken = 0;
+    while (!S.pending.empty() && taken < wave_max && S.free_slots.size() > (size_t)(Kp + 2)) {
+      BnbItem r = S.pending.back(); S.pending.pop_back();
+      r.spare_slot = S.free_slots.back(); S.free_slots.pop_back();
+      items.push_back(r); ++taken;
     }
   }
   for (;;) {
     const int n = (int)items.size();
     BnbArgs A;
-    A.G = pb.G; A.ldg = pb.ldg; A.c = pb.c; A.scal = pb.scal; A.gmask = pb.gmask; A.Mp = Mp; A.Kp = Kp; A.cap = cap;
+    A.G = sys ? sys->G : pb.G; A.ldg = pb.ldg; A.gstride = sys ? sys->gstride : 0;
+    A.c = sys ? sys->c : pb.c; A.scal = sys ? sys->scal : pb.scal; A.gmask = pb.gmask; A.Mp = Mp; A.Kp = Kp; A.cap = cap;
     A.pool = pool; A.slot_stride = slot_doubles; A.htile_doubles = ht;
     A.items = d_items; A.n_items = n; A.item_counter = d_ctr; A.mu = mu;
-    A.cta_obj = ws.cta_obj; A.cta_b = ws.cta_b; A.cta_w = ws.cta_w; A.leaf_seq = d_ctr + 1;
+    A.max_grid = max_grid; A.cta_obj = ws.cta_obj; A.cta_b = ws.cta_b; A.cta_w = ws.cta_w; A.leaf_seq = d_ctr + 1;
     A.out = d_out; A.counters = ws.counters;
     if (shard && shard->probe) {                 // test hook: the relaxations of the given roots, nothing else
-      if (!pending.empty()) { set_error("bnb probe: too many nodes for one wave (%d)", wave_max); rc = PLS_EINVAL; goto done; }
+      if (!srch[0].pending.empty()) { set_error("bnb probe: too many nodes for one wave (%d)", wave_max); rc = PLS_EINVAL; goto done; }
       BNB_TRY(cudaMalloc(&d_probe, sizeof(double) * (size_t)n * Mp));
       A.probe_w = d_probe;
     }
@@ -398,16 +437,16 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
     BNB_TRY(cudaGetLastError());
     ++*launches; ++waves;
     BNB_TRY(cudaMemcpyAsync(out.data(), d_out, sizeof(BnbChild) * 2 * n, cudaMemcpyDeviceToHost, st));
-    BNB_TRY(cudaMemcpyAsync(&h_mu, mu, sizeof(double), cudaMemcpyDeviceToHost, st));
+    BNB_TRY(cudaMemcpyAsync(h_mu.data(), mu, sizeof(double) * L, cudaMemcpyDeviceToHost, st));
     BNB_TRY(cudaStreamSynchronize(st));
     if (shared_mu) {                 // exchange the incumbent with the other devices (bit patterns of doubles >= 0 order like integers)
       unsigned long long mine, cur = shared_mu->load();
-      memcpy(&mine, &h_mu, sizeof(mine));
+      memcpy(&mine, &h_mu[0], sizeof(mine));
       while (mine < cur && !shared_mu->compare_exchange_weak(cur, mine)) {}
       cur = shared_mu->load();
       if (cur < mine) {
-        memcpy(&h_mu, &cur, sizeof(double));
-        BNB_TRY(cudaMemcpyAsync(mu, &h_mu, sizeof(double), cudaMemcpyHostToDevice, st));   // leaves only ever lower it further
+        memcpy(&h_mu[0], &cur, sizeof(double));
+        BNB_TRY(cudaMemcpyAsync(mu, &h_mu[0], sizeof(double), cudaMemcpyHostToDevice, st));   // leaves only ever lower it further
         BNB_TRY(cudaStreamSynchronize(st));
       }
     }
@@ -419,75 +458,97 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
         if (out[(size_t)2 * i].status == 3) { set_error("bnb: a node relaxation did not converge"); rc = PLS_ENUMERIC; goto done; }
         shard->probe_lb[i] = out[(size_t)2 * i].lb;
       }
-      visited = n; complete = false;
+      srch[0].visited = n; complete = false;
       goto done;
     }
     for (int i = 0; i < n; ++i) {
       const BnbItem &itx = items[i];
+      Search &S = srch[itx.l];
       const bool root = itx.k < 0;
       bool parent_slot_kept = false, spare_kept = false;
       for (int ch = 0; ch < (root ? 1 : 2); ++ch) {
         const BnbChild &c = out[(size_t)2 * i + ch];
-        ++visited;
-        if (c.status == 3) { set_error("bnb: a node relaxation did not converge"); rc = PLS_ENUMERIC; goto done; }
+        ++S.visited;
+        if (c.status == 3) { set_error("bnb: a node relaxation did not converge%s", who(itx.l)); rc = PLS_ENUMERIC; goto done; }
         if (c.status != 2) continue;
         OpenNode nd; nd.lb = c.lb; nd.slot = c.slot; nd.k = c.next_k;
         nd.pos = itx.pos_mask; nd.neg = itx.neg_mask;
         if (!root) { if (ch == 0) nd.pos |= 1ull << itx.k; else nd.neg |= 1ull << itx.k; }
         nd.depth = __builtin_popcountll(nd.pos | nd.neg);
-        open.push_back(nd);
+        S.open.push_back(nd);
         if (c.slot == itx.spare_slot) spare_kept = true; else parent_slot_kept = true;
       }
-      if (!spare_kept) free_slots.push_back(itx.spare_slot);
-      if (!root && !parent_slot_kept) free_slots.push_back(itx.parent_slot);
+      if (!spare_kept) S.free_slots.push_back(itx.spare_slot);
+      if (!root && !parent_slot_kept) S.free_slots.push_back(itx.parent_slot);
     }
     // next wave: drop nodes the incumbent now prunes; best-first by lower bound while the pool has
     // room, deepest-first when it runs low (depth-first keeps the number of live states bounded)
-    {
+    long long n_open = 0;
+    bool all_done = true;
+    for (int l = 0; l < L; ++l) {
+      Search &S = srch[l];
+      if (S.done) continue;
       size_t keep = 0;
-      for (size_t i = 0; i < open.size(); ++i) {
-        if (open[i].lb < h_mu) open[keep++] = open[i]; else free_slots.push_back(open[i].slot);
+      for (size_t i = 0; i < S.open.size(); ++i) {
+        if (S.open[i].lb < h_mu[l]) S.open[keep++] = S.open[i]; else S.free_slots.push_back(S.open[i].slot);
       }
-      open.resize(keep);
+      S.open.resize(keep);
+      n_open += (long long)keep;
+      S.done = S.open.empty() && S.pending.empty();
+      all_done = all_done && S.done;
     }
-    max_open = std::max<long long>(max_open, (long long)open.size());
-    if (open.empty() && pending.empty()) break;
-    if (shard && pending.empty() && ((shard->stop_waves > 0 && waves >= shard->stop_waves) ||
-                                     (shard->stop_open > 0 && (long long)open.size() >= shard->stop_open))) {
+    max_open = std::max<long long>(max_open, n_open);
+    if (all_done) break;
+    if (shard && srch[0].pending.empty() && ((shard->stop_waves > 0 && waves >= shard->stop_waves) ||
+                                             (shard->stop_open > 0 && (long long)srch[0].open.size() >= shard->stop_open))) {
       complete = false;                        // hand the frontier back (best lower bound first)
+      std::vector<OpenNode> &open = srch[0].open;
       std::sort(open.begin(), open.end(), [](const OpenNode &a, const OpenNode &b) { return a.lb < b.lb; });
       for (const OpenNode &nd : open) { shard->open_pos.push_back(nd.pos); shard->open_neg.push_back(nd.neg); }
       break;
     }
-    if (max_nodes > 0 && visited >= max_nodes) {
-      set_error("bnb: node budget PLS_BNB_MAX_NODES=%lld exhausted (%lld visited, %zu open, incumbent %.9g)", max_nodes, visited, open.size(), h_mu);
-      rc = PLS_EUNSUPPORTED; goto done;
-    }
-    const bool low = free_slots.size() < (size_t)2 * wave_max;
-    if (low) std::sort(open.begin(), open.end(), [](const OpenNode &a, const OpenNode &b) { return a.depth != b.depth ? a.depth < b.depth : a.lb > b.lb; });
-    else std::sort(open.begin(), open.end(), [](const OpenNode &a, const OpenNode &b) { return a.lb > b.lb; });
     items.clear();
-    // depth-first needs at most Kp + 1 slots per node in flight before a leaf frees one
-    const int limit = low ? (int)std::max<size_t>(1, free_slots.size() / (size_t)(Kp + 1)) : wave_max;
-    while (!pending.empty() && (int)items.size() < std::min(limit, wave_max) && !free_slots.empty()) {   // roots not started yet
-      BnbItem r = pending.back(); pending.pop_back();
-      r.spare_slot = free_slots.back(); free_slots.pop_back();
-      items.push_back(r);
+    for (int l = 0; l < L; ++l) {
+      Search &S = srch[l];
+      if (S.done) continue;
+      if (max_nodes > 0 && S.visited >= max_nodes) {
+        set_error("bnb: node budget PLS_BNB_MAX_NODES=%lld exhausted (%lld visited, %zu open, incumbent %.9g)%s", max_nodes, S.visited,
+                  S.open.size(), h_mu[l], who(l));
+        rc = PLS_EUNSUPPORTED; goto done;
+      }
+      std::vector<OpenNode> &open = S.open;
+      std::vector<int> &free_slots = S.free_slots;
+      const bool low = free_slots.size() < (size_t)2 * wave_max;
+      if (low) std::sort(open.begin(), open.end(), [](const OpenNode &a, const OpenNode &b) { return a.depth != b.depth ? a.depth < b.depth : a.lb > b.lb; });
+      else std::sort(open.begin(), open.end(), [](const OpenNode &a, const OpenNode &b) { return a.lb > b.lb; });
+      // depth-first needs at most Kp + 1 slots per node in flight before a leaf frees one
+      const int limit = std::min(wave_max, low ? (int)std::max<size_t>(1, free_slots.size() / (size_t)(Kp + 1)) : wave_max);
+      int taken = 0;
+      while (!S.pending.empty() && taken < limit && !free_slots.empty()) {
+        BnbItem r = S.pending.back(); S.pending.pop_back();
+        r.spare_slot = free_slots.back(); free_slots.pop_back();
+        items.push_back(r); ++taken;
+      }
+      while (!open.empty() && taken < limit && !free_slots.empty()) {
+        const OpenNode nd = open.back(); open.pop_back();
+        BnbItem it; it.parent_slot = nd.slot; it.spare_slot = free_slots.back(); free_slots.pop_back();
+        it.k = nd.k; it.l = l; it.pos_mask = nd.pos; it.neg_mask = nd.neg;
+        items.push_back(it); ++taken;
+      }
+      if (taken == 0) {
+        set_error("bnb: state pool exhausted (%zu slots; depth-first needs K + 3 = %d)%s", quota, Kp + 2, who(l));
+        rc = PLS_ENOMEM; goto done;
+      }
     }
-    while (!open.empty() && (int)items.size() < std::min(limit, wave_max) && !free_slots.empty()) {
-      const OpenNode nd = open.back(); open.pop_back();
-      BnbItem it; it.parent_slot = nd.slot; it.spare_slot = free_slots.back(); free_slots.pop_back();
-      it.k = nd.k; it.pad = 0; it.pos_mask = nd.pos; it.neg_mask = nd.neg;
-      items.push_back(it);
-    }
-    if (items.empty()) { set_error("bnb: state pool exhausted (%zu slots; depth-first needs K + 3 = %d)", n_slots, Kp + 2); rc = PLS_ENOMEM; goto done; }
   }
-  k5_select_leaf<<<1, 256, 0, st>>>(ws.cta_obj, ws.cta_b, ws.cta_w, max_grid, Mp, ws.win);
+  k5_select_leaf<<<L, 256, 0, st>>>(ws.cta_obj, ws.cta_b, ws.cta_w, max_grid, Mp, ws.win);
   BNB_TRY(cudaGetLastError());
   ++*launches;
   BNB_TRY(cudaStreamSynchronize(st));
   if (rep) {
-    rep->visited = visited; rep->waves = waves; rep->max_open = max_open; rep->pool_slots = (long long)n_slots; rep->mu = h_mu;
+    rep->visited = 0; rep->nopen.assign(L, 0);
+    for (int l = 0; l < L; ++l) { rep->nopen[l] = srch[l].visited; rep->visited += srch[l].visited; }
+    rep->waves = waves; rep->max_open = max_open; rep->pool_slots = (long long)n_slots; rep->mu = h_mu[0];
     rep->complete = complete; rep->has_leaf = false;
   }
 done:

@@ -235,7 +235,8 @@ struct K2Choice { int variant = 0, cap = 0, occ = 1; size_t smem = 0; K3Plan p3;
 int k2_choose(int Mp, int Kp, int64_t b_begin, int64_t b_count, bool outputs, int sm_count, bool free_top,
               int force_variant, const uint64_t *h_gmask, K2Choice *ch);
 // K5: branch and bound with batched frontier expansion (bnb.cu); winner left in ws.win
-struct BnbReport { long long visited, waves, max_open, pool_slots; double mu; bool complete, has_leaf; };
+// visited: nodes solved by all searches, nopen[l]: by search l
+struct BnbReport { long long visited, waves, max_open, pool_slots; double mu; bool complete, has_leaf; std::vector<long long> nopen; };
 // Multi-GPU sharding of the search (multi.cu).  roots: the subtrees this call searches, each given by the
 // groups fixed to + / - at its root (empty = the whole tree); shared_mu: bit pattern of an incumbent shared
 // with the other devices, read and lowered after every wave; stop_waves / stop_open: hand the frontier
@@ -250,8 +251,12 @@ struct BnbShard {
   bool probe = false;
   std::vector<double> probe_lb, probe_w;
 };
+// Several searches in one run (an eta path): L <= 64 Gram systems of one shape, system l at G + l * gstride with its
+// scalars at scal + 4 l, c shared.  Each has its own incumbent, open list, pool quota and winner record; their nodes
+// share the waves.  etas (host, nullable) name a system in error messages.  A fit searches the context's own system.
+struct BnbSystems { const double *G = nullptr; size_t gstride = 0; const double *c = nullptr, *scal = nullptr; int L = 1; const double *etas = nullptr; };
 int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, int *launches, BnbReport *rep,
-               BnbShard *shard = nullptr);
+               BnbShard *shard = nullptr, const BnbSystems *sys = nullptr);
 // K6: alternating optimisation, batched restarts (alt.cu)
 int k6_alt_run(const Problem &pb, SolveWs &ws, const std::vector<uint64_t> &h_gmask, const double *h_beta0, long long R,
                double eps, int Tmax, double *d_w, double *h_all_obj, int sm_count, cudaStream_t st, int *launches,

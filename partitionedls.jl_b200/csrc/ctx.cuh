@@ -85,7 +85,7 @@ FitMark fit_start(pls_ctx *c);
 void fit_finish(pls_ctx *c, const FitMark &m, pls_stats *out);
 bool use_pairs(const pls_ctx *c, uint32_t flags, bool per_orthant_outputs);
 double eta_term(const pls_ctx *c, double eta, const double *alpha_raw, int64_t b);
-double eta_term_w(const pls_ctx *c, const double *w);
+double eta_term_w(const pls_ctx *c, double eta, const double *w);
 int residual_partial_w(pls_ctx *c, const double *w, double *ssq_out);
 double now_ms();
 // The eta path's workspace in ws.path for L <= 64 problems: etas [64] | failure counts [64] | c [ldg] | scal_l [4 L] |

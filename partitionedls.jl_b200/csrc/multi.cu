@@ -411,7 +411,7 @@ int multi_bnb_fit_resident(pls_ctx *c, uint32_t flags, double *alpha_signed, dou
     if (rc) return rc;
     double tot = 0.0;
     for (int g = 0; g < G; ++g) tot += ssq[g];
-    obj = std::sqrt(tot + eta_term_w(c, alpha_signed));
+    obj = std::sqrt(tot + eta_term_w(c, c->pb.eta, alpha_signed));
   }
   *obj_out = obj;
   long long vis = 0;
@@ -474,7 +474,7 @@ int multi_alt_fit_resident(pls_ctx *c, const double *beta0, int64_t R, double ep
     if (rc) return rc;
     double tot = 0.0;
     for (int g = 0; g < G; ++g) tot += ssq[g];
-    obj = std::sqrt(tot + eta_term_w(c, w.data()));
+    obj = std::sqrt(tot + eta_term_w(c, c->pb.eta, w.data()));
   }
   *obj_out = obj;
   pls_stats &s = c->stats;

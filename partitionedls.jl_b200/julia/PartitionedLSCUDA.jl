@@ -189,6 +189,40 @@ function fit(::Type{BnBCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:Ab
 end
 
 """
+    fit_path(BnBCUDA, X, y, P; η::AbstractVector)
+
+`fit(BnBCUDA, X, y, P; η=η[l])` for every value of `η` (1 to 64 values, any order, duplicates allowed) on one upload
+of the data (`pls_load` + `pls_bnb_fit_path`): one Gram build, the searches of all η in the same frontier waves, one
+pass over X for all winners.  Returns a vector with one `(model, nothing, (; opt, nopen, stats))` per η; entry l has the
+optimum and model of `fit(BnBCUDA, X, y, P; η=η[l])` (within rounding: nopen is traversal dependent, as for one fit).
+`stats` is the call's, shared by all.
+"""
+function fit_path(::Type{BnBCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:AbstractFloat,1}, P::Array{Int,2};
+                  η::AbstractVector)
+    Xd = convert(Matrix{Float64}, X); yd = convert(Vector{Float64}, y); Pd = convert(Matrix{Int64}, P)
+    N, M = size(Xd); K = size(Pd, 2); L = length(η); etas = convert(Vector{Float64}, η)
+    alpha = zeros(Float64, M + 1, L); obj = zeros(Float64, L); nopen = zeros(Int64, L); stats = Ref{PlsStats}()
+    ctx = context()
+    GC.@preserve Xd yd Pd etas alpha obj nopen begin
+        _check(ccall((:pls_load, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, Int64, Int64, Ptr{Cdouble}, Ptr{Int64}, Int64, Cdouble),
+            ctx, Xd, N, N, M, yd, Pd, K, 0.0))
+        _check(ccall((:pls_bnb_fit_path, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, UInt32, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Ref{PlsStats}),
+            ctx, etas, L, UInt32(0), alpha, obj, nopen, stats))
+    end
+    _, Po = homogeneousCoords(Xd[1:1, :], Pd)            # only Po is needed (PartitionedLS.jl:76-81)
+    out = []
+    for l in 1:L
+        β = sum(Po .* alpha[:, l], dims = 1)             # BnB.jl:36
+        α = sum(Po .* alpha[:, l] ./ β, dims = 2)        # BnB.jl:37 (no zero guard upstream)
+        push!(out, (PartLSFitResult(α[1:end-1], β[1:end-1], β[end], P), nothing,
+                    (; opt = obj[l], nopen = Int(nopen[l]), stats = stats[])))
+    end
+    return out
+end
+
+"""
     fit(AltCUDA, X, y, P; η=0.0, ϵ=1e-6, T=100, nnlsalg=:nnls, rng=nothing, restarts=1)
 
 Same signature and return tuple as the reference (Alt.jl:50-51, :119) plus `restarts`: the
