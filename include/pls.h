@@ -215,6 +215,32 @@ int pls_opt_cv_path(pls_ctx *ctx, const int32_t *fold_id, int64_t F, const doubl
                     double *alpha_raw, int64_t *b_best, double *obj_train, double *ssq_heldout, double *cv_err,
                     int64_t *best, pls_stats *stats);
 
+/* ---- K-fold cross-validation of fit(BnB) over a grid of eta on the resident data set (one-GPU context) -------------
+ * The folds' raw Gram sums come from one K1 pass as for pls_opt_cv_path.  The F*L searches run in batches of whole
+ * folds (floor(64 / L) folds per batch, at least one): every search of a batch shares the same K5 waves, as the
+ * searches of pls_bnb_fit_path do, each fold with its own training c.  One K4 pass over the copy of the rows scores
+ * every leaf on its held-out fold.  X is not uploaded again.
+ *   fold_id[N], F, etas[L]  as for pls_opt_cv_path
+ *   alpha_signed[(M+1) x F*L], obj_train[F*L], nopen[F*L]
+ *                           column f*L + l = the best feasible leaf of fit(BnB) on the rows with fold_id != f at eta_l:
+ *                           its signed weights (intercept last), its Gram-space objective (what PLS_FLAG_NO_RECOMPUTE
+ *                           returns, eta rows included) and the nodes its search visited
+ *   ssq_heldout[F*L]        sum over the rows of fold f of (Xo * w - y)^2 for that leaf (no eta term)
+ *   cv_err[L], best         as for pls_opt_cv_path
+ *   flags                   PLS_FLAG_DEFAULT
+ *   stats                   of the whole call (ms_gram: the copy and the per-fold K1, ms_nnls: the finalises, the waves
+ *                           and the leaf selections, ms_recompute: the held-out K4 pass; orthants = sum of nopen, waves:
+ *                           the waves of all batches, max_open: the largest total number of open nodes)
+ * PLS_BNB_MAX_NODES bounds every search on its own; PLS_BNB_SLOTS sets the total pool of each batch.  The context's own
+ * eta, S, G, c and gram_ready are not changed.  Refused: PLS_EINVAL for a null pointer, no data loaded, F or L out of
+ * range, a fold id out of range, an empty fold, a bad eta or flags other than PLS_FLAG_DEFAULT; PLS_EUNSUPPORTED for
+ * M' > 1024, a multi-GPU context or an exhausted node budget; PLS_ENOMEM when the pool cannot give every search the
+ * K' + 3 slots a root needs; PLS_ENUMERIC for a relaxation that did not converge or a non-finite Gram matrix.  The
+ * messages of an exhausted budget and of PLS_ENUMERIC name the fold and the eta. */
+int pls_bnb_cv_path(pls_ctx *ctx, const int32_t *fold_id, int64_t F, const double *etas, int64_t L, uint32_t flags,
+                    double *alpha_signed, double *obj_train, int64_t *nopen, double *ssq_heldout, double *cv_err,
+                    int64_t *best, pls_stats *stats);
+
 /* ---- stage-wise entry points (one process per GPU; the caller owns the collectives) ----------
  * K1 on the loaded rows.  pls_gram_raw exposes the device buffer of raw sums S = Z'Z
  * ((M+2) x (M+2) doubles, column-major, lower triangle valid) so the caller can all-reduce it in

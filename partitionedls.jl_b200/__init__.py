@@ -254,7 +254,11 @@ def fit_cv(alg, X, y, P, etas, *, folds=5, seed=0, fold_ids=None, refit=True, ct
                    report.opt is its Gram-space training objective, report.b its orthant, report.ssq_heldout its
                    squared error on fold f
       fold_ids, stats
-      model, report  with refit: fit(Opt, X, y, P; η=best η) on all rows, from the same upload (None without)."""
+      model, report  with refit: fit(Opt, X, y, P; η=best η) on all rows, from the same upload (None without).
+
+    For fit(BnB), the exact method for K beyond what Opt can enumerate, load the data on a Context and call
+    Context.bnb_cv_path(fold_ids, etas) (pls_bnb_cv_path): the same folds and cv_err / best, with the signed weights of
+    every fold's best feasible leaf."""
     if not (alg is Opt or isinstance(alg, Opt)):
         raise TypeError(f"fit_cv supports Opt only, not {alg!r}")
     Xd, yd, Pd = _abi._as_inputs(X, y, P)

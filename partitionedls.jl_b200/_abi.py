@@ -85,13 +85,15 @@ lib.pls_bnb_fit_path.argtypes = [_vp, _dp, C.c_int64, C.c_uint32, _dp, _dp, _ip,
 _i32p = C.POINTER(C.c_int32)
 lib.pls_opt_cv_path.argtypes = [_vp, _i32p, C.c_int64, _dp, C.c_int64, C.c_uint32, _dp, _ip, _dp, _dp, _dp, _ip,
                                 C.POINTER(PlsStats)]
+lib.pls_bnb_cv_path.argtypes = [_vp, _i32p, C.c_int64, _dp, C.c_int64, C.c_uint32, _dp, _dp, _ip, _dp, _dp, _ip,
+                                C.POINTER(PlsStats)]
 lib.pls_cv_fold_sums.argtypes = [_vp, _i32p, C.c_int64, _dp]
 lib.pls_nnls_batch.argtypes = [_vp, _dp, _dp, C.c_double, C.c_int64, C.POINTER(C.c_uint64), C.c_int64,
                                C.c_int64, C.c_int64, _dp, _dp]
 for _n in ("pls_create", "pls_opt_fit", "pls_bnb_fit", "pls_bnb_fit_resident", "pls_alt_fit", "pls_alt_fit_resident", "pls_residual_partial_w", "pls_predict_resident", "pls_objective_finish_w", "pls_load", "pls_opt_fit_resident", "pls_gram_build", "pls_gram_raw",
            "pls_gram_finalize", "pls_opt_solve_range", "pls_opt_solve_pairs", "pls_opt_residual_partial", "pls_opt_objective_finish",
            "pls_get_stats", "pls_gram_scalars", "pls_bnb_lower_bounds", "pls_gram", "pls_nnls_batch", "pls_opt_fit_path",
-           "pls_residual_partial_multi", "pls_opt_cv_path", "pls_cv_fold_sums", "pls_bnb_fit_path"):
+           "pls_residual_partial_multi", "pls_opt_cv_path", "pls_cv_fold_sums", "pls_bnb_fit_path", "pls_bnb_cv_path"):
     getattr(lib, _n).restype = C.c_int
 
 
@@ -263,6 +265,25 @@ class Context:
         _check(lib.pls_opt_cv_path(self._h, f.ctypes.data_as(_i32p), F, _d(e), L, flags, _d(alpha), b.ctypes.data_as(_ip),
                                    _d(obj), _d(ssq), _d(cv), C.byref(best), C.byref(st)))
         return dict(alpha_raw=alpha.reshape(F, L, M + 1), b_best=b.reshape(F, L), obj_train=obj.reshape(F, L),
+                    ssq_heldout=ssq.reshape(F, L), cv_err=cv, best=best.value, stats=st.as_dict())
+
+    def bnb_cv_path(self, fold_id, etas, F=None, flags=0):
+        """pls_bnb_cv_path: K-fold cross-validation of fit(BnB) over `etas` on the resident data set, with fold_id and F
+        as for opt_cv_path.  Per (fold f, eta l): the best feasible leaf on the other folds' rows (alpha_signed[f, l], its
+        signed weights with the intercept last; obj_train[f, l], its Gram-space objective; nopen[f, l], the nodes its
+        search visited) and its sum of squared errors on fold f (ssq_heldout[f, l]); cv_err and best as for
+        opt_cv_path."""
+        N, M, K = self._shape
+        f = self._fold_ids(fold_id)
+        F = int(f.max()) + 1 if F is None else int(F)
+        e = np.ascontiguousarray(np.asarray(etas, dtype=np.float64).reshape(-1))
+        L = len(e)
+        FL = max(F, 0) * L
+        a = np.zeros((FL, M + 1)); obj = np.zeros(FL); nopen = np.zeros(FL, dtype=np.int64); ssq = np.zeros(FL)
+        cv = np.zeros(L); best = C.c_int64(); st = PlsStats()
+        _check(lib.pls_bnb_cv_path(self._h, f.ctypes.data_as(_i32p), F, _d(e), L, flags, _d(a), _d(obj),
+                                   nopen.ctypes.data_as(_ip), _d(ssq), _d(cv), C.byref(best), C.byref(st)))
+        return dict(alpha_signed=a.reshape(F, L, M + 1), obj_train=obj.reshape(F, L), nopen=nopen.reshape(F, L),
                     ssq_heldout=ssq.reshape(F, L), cv_err=cv, best=best.value, stats=st.as_dict())
 
     def cv_fold_sums(self, fold_id, F):

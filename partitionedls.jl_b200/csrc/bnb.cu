@@ -20,9 +20,14 @@
 // the number of visited nodes (`nopen`) does, and is reported for this traversal.
 //
 // Several searches per run (an eta path): L <= 64 searches on L Gram systems of one shape share every wave.  An item
-// names its search l; node l solves G + l * gstride with the scalars at scal + 4 l (c is shared), prunes against its own
-// incumbent mu[l] and keeps its best leaf in its own per-CTA slot.  The host keeps one open list, pool quota and node
-// budget per search and concatenates the items every search would take into one launch.  A fit is the case L = 1.
+// names its search l; node l solves G + l * gstride with the scalars at scal + 4 l, prunes against its own incumbent
+// mu[l] and keeps its best leaf in its own per-CTA slot.  The host keeps one open list, pool quota and node budget per
+// search and concatenates the items every search would take into one launch.  A fit is the case L = 1.
+//
+// c: a fit and an eta path share one c (eta only changes G), which a CTA copies to shared memory once.  The training
+// systems of cross-validation have one c per fold (c_f = sum over g != f of Xo_g' y_g): search l reads c + (l /
+// searches_per_c) * ldg, and the PER_C instantiation reloads its shared copy before an item of another fold.  Items
+// are concatenated search by search, so a CTA reloads only where a wave crosses a fold boundary.
 #include <string.h>
 #include <algorithm>
 #include <cmath>
@@ -52,7 +57,7 @@ struct BnbChild {
 
 struct BnbArgs {
   const double *G; int ldg; size_t gstride;    // system l: G + l * gstride
-  const double *c;                             // shared by every system
+  const double *c;                             // system l: c + (l / searches_per_c) * ldg (PER_C kernels only)
   const double *scal;                          // system l: scal + 4 l
   const uint64_t *gmask;
   int Mp, Kp, cap;
@@ -66,6 +71,7 @@ struct BnbArgs {
   BnbChild *out;                               // [n_items][2]
   unsigned long long *counters;
   double *probe_w = nullptr;                   // test hook: [n_items][Mp] signed weights of every ROOT item's relaxation
+  int searches_per_c = 0;                      // PER_C kernels: consecutive searches that share one c
 };
 
 // ---- pooled state: [H tiles | w (cap) | r (cap) | F (cap ints) | meta (8 ints)] -------------------
@@ -118,7 +124,7 @@ __device__ __forceinline__ void atomic_min_nonneg(double *addr, double v) {
   atomicMin(reinterpret_cast<unsigned long long *>(addr), (unsigned long long)__double_as_longlong(v));
 }
 
-template <int T, int MINB>
+template <int T, int MINB, bool PER_C = false>
 __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
   constexpr int NW = T / 32;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -127,7 +133,11 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
   const size_t ht = A.htile_doubles;
   Cfg3 cf; cf.cap = cap; cf.qs = 0; cf.hg = A.pool;
   Sh3 s = make_sh3(cf);
-  for (int m = tid; m < cap; m += T) { s.cs[m] = m < Mp ? A.c[m] : 0.0; s.gms[m] = m < Mp ? A.gmask[m] : 0ull; }
+  if constexpr (PER_C)
+    for (int m = tid; m < cap; m += T) s.gms[m] = m < Mp ? A.gmask[m] : 0ull;
+  else
+    for (int m = tid; m < cap; m += T) { s.cs[m] = m < Mp ? A.c[m] : 0.0; s.gms[m] = m < Mp ? A.gmask[m] : 0ull; }
+  int c_held = -1;                             // PER_C: the c (fold) s.cs holds; the same in every thread
   for (int ti = tid; ti < ntc; ti += T)
     for (int tj = 0; tj <= ti; ++tj) s.tmap[tile_q(ti, tj)] = (unsigned short)((ti << 8) | tj);
   if (tid == 0)
@@ -147,6 +157,16 @@ __global__ void __launch_bounds__(T, MINB) k5_bnb_expand(const BnbArgs A) {
     if (it >= (unsigned long long)A.n_items) break;
     const BnbItem item = A.items[it];
     const bool root = item.k < 0;
+    if constexpr (PER_C) {
+      // the barriers above ended every read of s.cs for the previous item; the one below orders the copy before use
+      const int ci = item.l / A.searches_per_c;
+      if (ci != c_held) {
+        const double *cc = A.c + (size_t)ci * A.ldg;
+        for (int m = tid; m < cap; m += T) s.cs[m] = m < Mp ? cc[m] : 0.0;
+        c_held = ci;
+        __syncthreads();
+      }
+    }
     const double *G = A.G + (size_t)item.l * A.gstride;
     const double yy = A.scal[4 * item.l], cmax = A.scal[4 * item.l + 1];
     double *mu = A.mu + item.l;
@@ -302,12 +322,15 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
   const int Mp = pb.Mp, Kp = pb.Kp;
   const int L = sys ? sys->L : 1;
   if (L < 1 || L > 64) { set_error("bnb: %d searches (1..64)", L); return PLS_EINVAL; }
+  const int per_c = sys && sys->searches_per_c > 0 ? sys->searches_per_c : L;    // searches that share one c
   if (shard && L > 1) { set_error("bnb: a sharded search runs on one system"); return PLS_EINVAL; }
   // names the system of search l in error messages, when there are several
   char who_buf[64];
   auto who = [&](int l) -> const char * {
     who_buf[0] = 0;
-    if (sys && sys->etas) snprintf(who_buf, sizeof(who_buf), " (eta = %g)", sys->etas[l]);
+    if (sys && sys->etas && sys->fold0 >= 0)
+      snprintf(who_buf, sizeof(who_buf), " (fold %d, eta = %g)", sys->fold0 + l / per_c, sys->etas[l % per_c]);
+    else if (sys && sys->etas) snprintf(who_buf, sizeof(who_buf), " (eta = %g)", sys->etas[l]);
     return who_buf;
   };
   if (Mp > CAP3MAX) { set_error("bnb: M' = %d exceeds this build's limit (%d)", Mp, CAP3MAX); return PLS_EUNSUPPORTED; }
@@ -318,7 +341,8 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
   const size_t slot_doubles = (bnb_slot_doubles(cap) + 1) & ~(size_t)1;     // keep slots 16-byte aligned
   const size_t smem = sh3_doubles(cap) * sizeof(double) + sh3_ints(cap) * sizeof(int) + 5 * (size_t)cap + 16;
   const bool wide = Mp > 256;
-  auto kern = wide ? k5_bnb_expand<TB, 2> : k5_bnb_expand<TB, 3>;
+  auto kern = per_c < L ? (wide ? k5_bnb_expand<TB, 2, true> : k5_bnb_expand<TB, 3, true>)
+                        : (wide ? k5_bnb_expand<TB, 2> : k5_bnb_expand<TB, 3>);
   int dev = 0, max_smem = 0;
   PLS_CUDA_TRY(cudaGetDevice(&dev));
   PLS_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
@@ -425,7 +449,7 @@ int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, in
     A.pool = pool; A.slot_stride = slot_doubles; A.htile_doubles = ht;
     A.items = d_items; A.n_items = n; A.item_counter = d_ctr; A.mu = mu;
     A.max_grid = max_grid; A.cta_obj = ws.cta_obj; A.cta_b = ws.cta_b; A.cta_w = ws.cta_w; A.leaf_seq = d_ctr + 1;
-    A.out = d_out; A.counters = ws.counters;
+    A.out = d_out; A.counters = ws.counters; A.searches_per_c = per_c;
     if (shard && shard->probe) {                 // test hook: the relaxations of the given roots, nothing else
       if (!srch[0].pending.empty()) { set_error("bnb probe: too many nodes for one wave (%d)", wave_max); rc = PLS_EINVAL; goto done; }
       BNB_TRY(cudaMalloc(&d_probe, sizeof(double) * (size_t)n * Mp));

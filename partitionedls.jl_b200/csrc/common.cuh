@@ -252,9 +252,14 @@ struct BnbShard {
   std::vector<double> probe_lb, probe_w;
 };
 // Several searches in one run (an eta path): L <= 64 Gram systems of one shape, system l at G + l * gstride with its
-// scalars at scal + 4 l, c shared.  Each has its own incumbent, open list, pool quota and winner record; their nodes
-// share the waves.  etas (host, nullable) name a system in error messages.  A fit searches the context's own system.
-struct BnbSystems { const double *G = nullptr; size_t gstride = 0; const double *c = nullptr, *scal = nullptr; int L = 1; const double *etas = nullptr; };
+// scalars at scal + 4 l and its c at c + (l / searches_per_c) * ldg (0: every system shares c).  Each has its own
+// incumbent, open list, pool quota and winner record; their nodes share the waves.  etas (host, nullable) name a system
+// in error messages: etas[l] or, for cross-validation (fold0 >= 0), fold fold0 + l / searches_per_c at
+// etas[l % searches_per_c].  A fit searches the context's own system.
+struct BnbSystems {
+  const double *G = nullptr; size_t gstride = 0; const double *c = nullptr, *scal = nullptr; int L = 1;
+  const double *etas = nullptr; int searches_per_c = 0, fold0 = -1;
+};
 int k5_bnb_run(const Problem &pb, SolveWs &ws, int sm_count, cudaStream_t st, int *launches, BnbReport *rep,
                BnbShard *shard = nullptr, const BnbSystems *sys = nullptr);
 // K6: alternating optimisation, batched restarts (alt.cu)

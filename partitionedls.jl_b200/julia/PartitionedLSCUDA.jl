@@ -223,6 +223,53 @@ function fit_path(::Type{BnBCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray
 end
 
 """
+    fit_cv(BnBCUDA, X, y, P; η::AbstractVector, folds=5, fold_ids=nothing, rng=Random.default_rng(), refit=true)
+
+K-fold cross-validation of `fit(BnBCUDA, X, y, P; η=η[l])` over `η` (1 to 64 values) on one upload of the data
+(`pls_load` + `pls_bnb_cv_path`): one K1 pass gives the Gram sums of every fold, the searches of whole folds share the
+same frontier waves, one pass over X scores every best leaf on its held-out fold.  `folds`, `fold_ids` and `rng` as for
+`fit_cv(OptCUDA, ...)`.  Returns `(; cv_err, best, η, fold_ids, model, report, stats)`: `cv_err`, `best` and `η` as for
+`fit_cv(OptCUDA, ...)`; with `refit`, `model` and `report` (`(; opt, nopen, stats)`) are `fit(BnBCUDA, X, y, P;
+η=η[best])` on all rows, from the same upload (`pls_bnb_fit_path` at that η), and `nothing` without.
+"""
+function fit_cv(::Type{BnBCUDA}, X::Array{<:AbstractFloat,2}, y::AbstractArray{<:AbstractFloat,1}, P::Array{Int,2};
+                η::AbstractVector, folds::Integer=5, fold_ids=nothing, rng=Random.default_rng(), refit::Bool=true)
+    Xd = convert(Matrix{Float64}, X); yd = convert(Vector{Float64}, y); Pd = convert(Matrix{Int64}, P)
+    N, M = size(Xd); K = size(Pd, 2); L = length(η); etas = convert(Vector{Float64}, η)
+    fid = fold_ids === nothing ? Int32.(randperm(rng, N) .% folds) : Int32.(fold_ids .- 1)   # 0-based for the ABI
+    F = Int64(maximum(fid) + 1)
+    alpha = zeros(Float64, M + 1, F * L); obj = zeros(Float64, F * L); nopen = zeros(Int64, F * L)
+    ssq = zeros(Float64, F * L); cv = zeros(Float64, L); best = Ref{Int64}(0); stats = Ref{PlsStats}()
+    ctx = context()
+    GC.@preserve Xd yd Pd etas fid alpha obj nopen ssq cv begin
+        _check(ccall((:pls_load, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Cdouble}, Int64, Int64, Int64, Ptr{Cdouble}, Ptr{Int64}, Int64, Cdouble),
+            ctx, Xd, N, N, M, yd, Pd, K, 0.0))
+        _check(ccall((:pls_bnb_cv_path, libpls), Cint,
+            (Ptr{Cvoid}, Ptr{Int32}, Int64, Ptr{Cdouble}, Int64, UInt32, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ref{Int64}, Ref{PlsStats}),
+            ctx, fid, F, etas, L, UInt32(0), alpha, obj, nopen, ssq, cv, best, stats))
+    end
+    ηbest = etas[best[] + 1]
+    model = report = nothing
+    if refit
+        a = zeros(Float64, M + 1); o = Ref{Cdouble}(0.0); n = Ref{Int64}(0); st = Ref{PlsStats}(); e = [ηbest]
+        GC.@preserve a e begin
+            _check(ccall((:pls_bnb_fit_path, libpls), Cint,
+                (Ptr{Cvoid}, Ptr{Cdouble}, Int64, UInt32, Ptr{Cdouble}, Ref{Cdouble}, Ref{Int64}, Ref{PlsStats}),
+                ctx, e, 1, UInt32(0), a, o, n, st))
+        end
+        _, Po = homogeneousCoords(Xd[1:1, :], Pd)        # only Po is needed (PartitionedLS.jl:76-81)
+        β = sum(Po .* a, dims = 1)                       # BnB.jl:36
+        α = sum(Po .* a ./ β, dims = 2)                  # BnB.jl:37 (no zero guard upstream)
+        model = PartLSFitResult(α[1:end-1], β[1:end-1], β[end], P)
+        report = (; opt = o[], nopen = Int(n[]), stats = st[])
+    end
+    return (; cv_err = cv, best = best[] + 1, η = ηbest, fold_ids = fid .+ 1, model = model, report = report,
+            stats = stats[])
+end
+
+"""
     fit(AltCUDA, X, y, P; η=0.0, ϵ=1e-6, T=100, nnlsalg=:nnls, rng=nothing, restarts=1)
 
 Same signature and return tuple as the reference (Alt.jl:50-51, :119) plus `restarts`: the
